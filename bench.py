@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the x-vector extraction hot path (BASELINE.json metric: x-vectors/sec & frames/sec).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--dtype bf16|tf32] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dtype bf16|tf32] [--impl b200|reference] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...        (one rank per GPU)
 
 A step = one pass of the hot path (TDNN1-5 -> statistics pooling -> segment6) over the workload of BASELINE.json configs[1]:
@@ -305,16 +305,20 @@ class Arm:
             return self.model.extract_x_vec_flat(self.x_dev[i % self.n_res], self.lengths, slot=i % self.n_inflight)
 
     def device_leg(self, n_batches, barrier):
-        """n_batches batches, two in flight, one CUDA-event bracket; returns device milliseconds."""
+        """n_batches batches, two in flight, one CUDA-event bracket; returns device milliseconds.  The x-vectors of the last
+        step's batches stay in self.last_step."""
         torch = self.torch
         e_beg, e_end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         cur = torch.cuda.current_stream()
+        self.last_step = []
         barrier()
         e_beg.record(cur)
         for st in self.streams:
             st.wait_event(e_beg)
         for i in range(n_batches):
-            self.batch(i)
+            y = self.batch(i)
+            if i >= n_batches - BATCHES_PER_STEP:
+                self.last_step.append(y)
         for st in self.streams:
             cur.wait_stream(st)
         e_end.record(cur)
@@ -464,6 +468,7 @@ def run_b200(args, rank, world, local_rank):
         sampler.start()
         dev_ms = arm.device_leg(steps_b, barrier)
         clocks_value = sampler.stop()
+        xvectors = torch.cat(arm.last_step).cpu().numpy() if args.dump_outputs else None
         sampler = ClockSampler(local_rank)
         sampler.start()
         e2e_ms, checksum, enq_us = arm.e2e_leg(steps_b, barrier)
@@ -478,7 +483,7 @@ def run_b200(args, rank, world, local_rank):
         dev_ms, e2e_ms, long_dev_ms, long_e2e_ms = max_over_ranks([dev_ms, e2e_ms, long_dev_ms, long_e2e_ms])
         return arm, {"dev_ms": dev_ms, "e2e_ms": e2e_ms, "checksum": checksum, "enq_us": enq_us, "h2d": h2d, "d2h": d2h, "clocks_value": clocks_value,
                      "clocks_e2e": clocks_e2e, "long_dev_ms": long_dev_ms, "long_e2e_ms": long_e2e_ms, "long_enq_us": long_enq_us,
-                     "clocks_long": clocks_long}
+                     "clocks_long": clocks_long, "xvectors": xvectors}
 
     def arm_numbers(r):
         utts = N_UTTS * args.steps * world
@@ -580,6 +585,10 @@ def run_b200(args, rank, world, local_rank):
             line["roofline_pool"] = pooling_roofline(arm.model, dev, peaks)
         if world == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline_leg()
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {f"xvectors_{primary}": res["xvectors"]})
+            if not args.no_second_dtype:
+                dump_outputs(args.dump_outputs, {f"xvectors_{other}": res2["xvectors"]})
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()
@@ -732,6 +741,8 @@ def run_c5(args, torch, dist, xvec_b200, model, dev, rank, world, barrier, max_o
     decisions = (s >= thr)
     wall = sorted(walls)[len(walls) // 2]
     total_frames = int(lengths.sum())
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"c5_embeddings": emb_host.numpy(), "c5_scores": scores_host.numpy()})
     return {"workload": "c5: 4874 utterances of 4-20 s (5.86 M frames, 563 MB of fp32 MFCC) LPT-sharded by utterance over the GPUs, "
                         "x-vectors gathered on the devices, 37,720 centred-cosine trials scored on GPU 0, scores + embeddings to the host",
             "scaling": "strong", "dtype": model.precision, "n_gpus": world, "n_utts": C5_N, "frames": total_frames, "trials": C5_TRIALS,
@@ -756,6 +767,15 @@ def run_c5(args, torch, dist, xvec_b200, model, dev, rank, world, barrier, max_o
             "scores_sum": float(s.sum()), "embeddings_abs_sum": float(np.abs(emb_host.numpy().astype(np.float64)).sum()),
             "identity_note": "the three sha1 are over the raw float32 bytes of all 4874 x 512 embeddings, of the 37,720 scores and over the "
                              "decision bits: identical for N = 1, 2, 4, 8 because batches, not utterances, are the unit of sharding"}
+
+
+def dump_outputs(dirname, arrays):
+    """<dirname>/<name>.npy in float32 for every array: the inputs are seeded, so two builds run with the same arguments can be
+    compared output for output."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), np.asarray(a, dtype=np.float32))
 
 
 def tdnn_flops_ragged(lengths):
@@ -836,7 +856,14 @@ def main():
     ap.add_argument("--no-c5", action="store_true")
     ap.add_argument("--c5-batch-frames", type=int, default=49152)
     ap.add_argument("--no-second-dtype", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write rank 0's x-vectors of the last timed step (xvectors_<dtype>.npy, one row per utterance, for each precision run) and the c5 "
+                         "embeddings and trial scores (c5_embeddings.npy, c5_scores.npy) to DIR as float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
