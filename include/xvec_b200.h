@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define XVEC_ABI_VERSION 5
+#define XVEC_ABI_VERSION 6
 
 #if defined(__GNUC__)
 #define XVEC_API __attribute__((visibility("default")))
@@ -203,30 +203,10 @@ XVEC_API int xvec_tdnn_stack(const struct XvecLayerDesc* tdnn_host, int n_tdnn, 
 XVEC_API int xvec_linear_small(const void* x_dev, int dtype, int64_t rows, int k, int64_t x_ld, const void* w_dev, int n, int64_t w_ld,
                       const float* bias_dev, int relu, void* y_dev, int y_dtype, int64_t y_ld, void* stream);
 
-/* Statistics-pooling finalize FUSED with the first segment layer: out = act([mean || std] W' + bias) per utterance, straight from
- * the pooling partials (the (n_utts, 2p) pooled matrix is never written) — one launch for the tail of a batch.  The K dimension
- * (2p) is split over the grid; the last CTA of an output tile to arrive adds the float32 partial tiles in slice order
- * (deterministic) and applies bias / ReLU.  Same small footprint as xvec_linear_small (128 threads, < 14 KiB of shared memory, no
- * tensor memory), so it runs next to the resident CTAs of the next batch's xvec_tdnn_stack kernel.  Measured (B200, 256 utterances,
- * p = 1500, n = 512, warm L2): 37.9 us against 7.9 + 23.3 us for xvec_pool_finalize + xvec_linear_small: it saves a launch and the
- * 3 MB pooled matrix but re-reads its slice of W once per 16 utterances; an alternative entry point, not what
- * xvec_extract_forward uses.
- * replaces: torch.mean / torch.std / torch.cat of stat_pool (main.py:59-63) + segment_layer6 (main.py:45, 87-90).
- *   part / slot_start / n_rows / bn_scale / bn_shift as for xvec_pool_finalize;  w_dev (n, 2p) row-major of `dtype` with row stride
- *   w_ld elements (the nn.Linear weight, NOT packed);  out_dev (n_utts, n) float32 or bfloat16, row stride out_ld;
- *   ws_dev: 16-byte aligned scratch of xvec_pool_fc_workspace_bytes(...) bytes, ZERO-FILLED before its first use (the kernel
- *   keeps its arrival counters at zero between launches), private to the call until it completes.  p a multiple of 4, n even. */
-XVEC_API int64_t xvec_pool_fc_workspace_bytes(int n_utts, int p, int n, int dtype);
-XVEC_API int xvec_pool_fc_fused(const float* part_dev, const int32_t* slot_start_dev, const int32_t* n_rows_dev, int n_utts, int p,
-                       const float* bn_scale_dev, const float* bn_shift_dev, const void* w_dev, int dtype, int64_t w_ld,
-                       const float* bias_dev, int n, int relu, void* out_dev, int out_dtype, int64_t out_ld, void* ws_dev,
-                       int64_t ws_bytes, void* stream);
-
 /* The whole extraction path for one flat batch in ONE call (3 kernel launches + one small memset enqueued on `stream`; the tensor
  * maps of recurring argument sets are cached): xvec_tdnn_stack, xvec_pool_finalize, then the n_fc segment layers (ReLU between
  * them, none after the last; xvec_linear_small when the layer carries w_plain_dev, else xvec_tdnn_layer with split-K).
- * (xvec_pool_fc_fused can run finalize + first segment layer as one launch; measured slower than the pair — 37.9 vs 31.2 us per
- * 256 utterances — so this call only uses it in -DXVEC_DEBUG builds with XVEC_TAIL_FUSED=1, for A/B runs.)  Without ctrl_dev (NULL) or for a stack xvec_tdnn_stack does not take, the TDNN layers run as one launch each
+ * Without ctrl_dev (NULL) or for a stack xvec_tdnn_stack does not take, the TDNN layers run as one launch each
  * (xvec_tdnn_layer / xvec_tdnn_pool_fused) — same results.
  * replaces: XVectorModel.extract_x_vec (main.py:81-94) = time_context_layers (main.py:38-44) + stat_pool (:59-63) +
  * segment_layer6 [+ relu + segment_layer7]; eval-mode BatchNorm of layers 0..n-2 must already be folded into the next
@@ -236,16 +216,14 @@ XVEC_API int xvec_pool_fc_fused(const float* part_dev, const int32_t* slot_start
  *   pooled_dev float32 (n_utts, 2 n_last);  pooled_lp_dev same in fc[0].dtype when that is XVEC_BF16, else NULL;
  *   fc_tmp_dev (n_utts, fc[0].n) of fc[1].dtype when n_fc == 2;  out_dev float32 (n_utts, fc[n_fc-1].n), row stride out_ld;
  *   splitk_ws_dev: scratch for the segment layers (see xvec_splitk_workspace_bytes) or NULL;
- *   tail_ws_dev / tail_ws_bytes: zero-initialised scratch of xvec_pool_fc_fused (xvec_pool_fc_workspace_bytes) or NULL / 0
- *   (only read by the debug-build A/B path);
  *   ctrl_dev / ctrl_bytes: scratch of xvec_tdnn_stack or NULL / 0. */
 XVEC_API int xvec_extract_forward(const XvecLayerDesc* tdnn_host, int n_tdnn, const void* x_dev, int64_t rows, int64_t x_ld,
                          void* act0_dev, void* act1_dev, int64_t act_ld, const int32_t* row_utt_dev,
                          const int32_t* blk_slot_base_dev, const int32_t* utt_slot_start_dev, const int32_t* n_pool_dev,
                          int n_utts, float* part_dev, const float* bn_last_scale_dev, const float* bn_last_shift_dev,
                          float* pooled_dev, void* pooled_lp_dev, const XvecLayerDesc* fc_host, int n_fc, void* fc_tmp_dev,
-                         void* splitk_ws_dev, int64_t splitk_ws_bytes, float* out_dev, int64_t out_ld, void* tail_ws_dev,
-                         int64_t tail_ws_bytes, void* ctrl_dev, int64_t ctrl_bytes, void* stream);
+                         void* splitk_ws_dev, int64_t splitk_ws_bytes, float* out_dev, int64_t out_ld, void* ctrl_dev,
+                         int64_t ctrl_bytes, void* stream);
 
 /* MFCC front end (the step BEFORE the path; SURVEY §8 row f4): waveform -> (frames, 24) float32 rows of the flat frame
  * matrix, with the reference's fixed parameters: 16 kHz, pre-emphasis 0.97, 400-sample frames every 160 samples (zero padded,

@@ -16,7 +16,7 @@ LIB_PATH = os.environ.get("XVEC_LIB") or os.path.join(HERE, "libxvec_b200.so")  
 F32, BF16 = 0, 1
 E_ARG, E_CUDA, E_DEVICE = -1, -2, -3
 TILE_N, POOL_BLOCK, POOL_CHUNK, MAX_TAPS = 256, 128, 128, 8
-ABI_VERSION = 5
+ABI_VERSION = 6
 MAX_STACK = 6
 STACK_MAX_TAP_OFFSET = 8  # XVEC_STACK_MAX_TAP_OFFSET
 
@@ -48,10 +48,7 @@ _SIGNATURES = {
                                    c_int, c_int64, c_void_p]),
     "xvec_extract_forward": (c_int, [POINTER(LayerDesc), c_int, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_void_p, c_void_p,
                                      c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, POINTER(LayerDesc), c_int,
-                                     c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p]),
-    "xvec_pool_fc_workspace_bytes": (c_int64, [c_int, c_int, c_int, c_int]),
-    "xvec_pool_fc_fused": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int, c_int64, c_void_p, c_int, c_int,
-                                   c_void_p, c_int, c_int64, c_void_p, c_int64, c_void_p]),
+                                     c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p]),
     "xvec_stack_ctrl_bytes": (c_int64, [c_int64, c_int]),
     "xvec_stack_plan": (c_int64, [c_int64, c_int, POINTER(c_int32), c_int, c_void_p, c_int64]),
     "xvec_linear_small": (c_int, [c_void_p, c_int, c_int64, c_int, c_int64, c_void_p, c_int, c_int64, c_void_p, c_int, c_void_p, c_int, c_int64,

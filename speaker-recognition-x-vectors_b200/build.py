@@ -11,7 +11,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libxvec_b200.so")
-SOURCES = ["capi.cu", "tdnn_gemm.cu", "tdnn_stack.cu", "fc_small.cu", "seg_fused.cu", "pool.cu", "mfcc.cu"]
+SOURCES = ["capi.cu", "tdnn_gemm.cu", "tdnn_stack.cu", "fc_small.cu", "pool.cu", "mfcc.cu"]
 HEADERS = ["ptx.cuh", "gemm_tile.cuh", "xvec_internal.h", os.path.join("..", "..", "include", "xvec_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC",
               "-Xcompiler", "-fvisibility=hidden", "--expt-relaxed-constexpr"]
@@ -33,11 +33,6 @@ def needs_build(lib: str = LIB) -> bool:
     t = os.path.getmtime(lib)
     deps = [os.path.join(CSRC, s) for s in SOURCES + HEADERS] + [os.path.abspath(__file__)]
     return any(os.path.getmtime(d) > t for d in deps)
-
-
-def build_variant(name: str, defines) -> str:
-    """Developer A/B builds: libxvec_b200_<name>.so with extra -D flags (select it with XVEC_LIB=...)."""
-    return _build_to(os.path.join(HERE, f"libxvec_b200_{name}.so"), list(NVCC_FLAGS) + [f"-D{d}" for d in defines], False, "_" + name)
 
 
 def build(force: bool = False, verbose: bool = False, debug: bool = False) -> str:

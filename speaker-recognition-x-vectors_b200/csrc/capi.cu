@@ -1,7 +1,6 @@
 // extern "C" surface of libxvec_b200.so (declared in include/xvec_b200.h) + small host utilities.
 #include <stdarg.h>
 #include <stdio.h>
-#include <stdlib.h>
 
 #include "xvec_internal.h"
 
@@ -84,36 +83,6 @@ int read_watchdog() {
   return w ? static_cast<int>(*reinterpret_cast<volatile unsigned int*>(w)) : 0;
 }
 
-// Developer A/B switches exist in -DXVEC_DEBUG builds only (libxvec_b200_debug.so); the product library reads no environment.
-//   XVEC_STACK=0     xvec_extract_forward runs one launch per TDNN layer
-//   XVEC_FC_SMALL=0  the segment layers stay on the tcgen05 kernel
-#ifdef XVEC_DEBUG
-static bool env_switch_on(const char* name) {
-  const char* e = getenv(name);
-  return !(e && e[0] == '0');
-}
-static bool use_stack_kernel() {
-  static const bool v = env_switch_on("XVEC_STACK");
-  return v;
-}
-static bool use_fc_small() {
-  static const bool v = env_switch_on("XVEC_FC_SMALL");
-  return v;
-}
-// XVEC_TAIL_FUSED=1  the tail of xvec_extract_forward runs as ONE launch (xvec_pool_fc_fused) instead of xvec_pool_finalize +
-//                     xvec_linear_small.  Measured on B200 (256 utterances, warm L2, ncu --cache-control none): 7.9 + 23.3 us
-//                     unfused vs 37.9 us fused in bf16 (41.8 + 7.9 vs 54.8 in TF32) — one launch less, but every 16-utterance CTA
-//                     re-reads its slice of W (89 MB of L2 traffic against 55 MB), so the two-launch tail stays the default.
-static bool use_fused_tail() {
-  static const bool v = getenv("XVEC_TAIL_FUSED") && getenv("XVEC_TAIL_FUSED")[0] == '1';
-  return v;
-}
-#else
-static constexpr bool use_stack_kernel() { return true; }
-static constexpr bool use_fc_small() { return true; }
-static constexpr bool use_fused_tail() { return false; }
-#endif
-
 }  // namespace xvec
 
 using namespace xvec;
@@ -167,15 +136,6 @@ int64_t xvec_stack_plan(int64_t rows, int n_layers, const int32_t* n_tiles_per_l
   return stack_plan(rows, n_layers, n_tiles_per_layer_host, band, items_out_host, capacity);
 }
 
-int64_t xvec_pool_fc_workspace_bytes(int n_utts, int p, int n, int dtype) { return pool_fc_workspace_bytes(n_utts, p, n, dtype); }
-int xvec_pool_fc_fused(const float* part_dev, const int32_t* slot_start_dev, const int32_t* n_rows_dev, int n_utts, int p,
-                       const float* bn_scale_dev, const float* bn_shift_dev, const void* w_dev, int dtype, int64_t w_ld,
-                       const float* bias_dev, int n, int relu, void* out_dev, int out_dtype, int64_t out_ld, void* ws_dev, int64_t ws_bytes,
-                       void* stream) {
-  return pool_fc_dispatch(part_dev, slot_start_dev, n_rows_dev, n_utts, p, bn_scale_dev, bn_shift_dev, w_dev, dtype, w_ld, bias_dev, n, relu,
-                          out_dev, out_dtype, out_ld, ws_dev, ws_bytes, stream);
-}
-
 int xvec_linear_small(const void* x_dev, int dtype, int64_t rows, int k, int64_t x_ld, const void* w_dev, int n, int64_t w_ld,
                       const float* bias_dev, int relu, void* y_dev, int y_dtype, int64_t y_ld, void* stream) {
   return fc_small_dispatch(x_dev, dtype, rows, k, x_ld, w_dev, n, w_ld, bias_dev, relu, y_dev, y_dtype, y_ld, stream);
@@ -194,14 +154,13 @@ int xvec_extract_forward(const XvecLayerDesc* tdnn, int n_tdnn, const void* x_de
                          const int32_t* utt_slot_start_dev, const int32_t* n_pool_dev, int n_utts, float* part_dev,
                          const float* bn_last_scale_dev, const float* bn_last_shift_dev, float* pooled_dev, void* pooled_lp_dev,
                          const XvecLayerDesc* fc, int n_fc, void* fc_tmp_dev, void* splitk_ws_dev, int64_t splitk_ws_bytes,
-                         float* out_dev, int64_t out_ld, void* tail_ws_dev, int64_t tail_ws_bytes, void* ctrl_dev, int64_t ctrl_bytes,
-                         void* stream) {
+                         float* out_dev, int64_t out_ld, void* ctrl_dev, int64_t ctrl_bytes, void* stream) {
   if (!tdnn || n_tdnn < 2 || !fc || n_fc < 1 || n_fc > 2) return set_error(XVEC_E_ARG, "need >= 2 TDNN layers and 1 or 2 segment layers");
   if (!x_dev || !act0_dev || !act1_dev || !pooled_dev || !out_dev) return set_error(XVEC_E_ARG, "null pointer argument");
   if (n_fc == 2 && !fc_tmp_dev) return set_error(XVEC_E_ARG, "fc_tmp_dev is NULL");
   const XvecLayerDesc& last = tdnn[n_tdnn - 1];
   int rc;
-  if (ctrl_dev && use_stack_kernel() && stack_supported(tdnn, n_tdnn, rows)) {
+  if (ctrl_dev && stack_supported(tdnn, n_tdnn, rows)) {
     rc = stack_dispatch(tdnn, n_tdnn, x_dev, rows, x_ld, act0_dev, act1_dev, act_ld, row_utt_dev, blk_slot_base_dev, part_dev, ctrl_dev,
                         ctrl_bytes, 0, stream);
     if (rc) return rc;
@@ -222,47 +181,19 @@ int xvec_extract_forward(const XvecLayerDesc* tdnn, int n_tdnn, const void* x_de
                        nullptr, 1, nullptr, XVEC_F32, 0, row_utt_dev, blk_slot_base_dev, part_dev, rows, true, nullptr, 0, stream);
     if (rc) return rc;
   }
-#ifdef XVEC_DEBUG
-  static const int skip_tail = getenv("XVEC_SKIP_TAIL") ? atoi(getenv("XVEC_SKIP_TAIL")) : 0;  // experiment: 1 = no segment layers, 2 = no finalize either
-  if (skip_tail >= 2) return XVEC_OK;
-#endif
   const int fc_in_dtype = fc[0].dtype;
-  int first_fc = 0;
-  const void* a = nullptr;
-  int64_t a_ld = 0;
-  if (use_fused_tail() && fc[0].w_plain_dev && tail_ws_dev && use_fc_small() && fc[0].cin == 2 * last.n &&
-      pool_fc_supported(n_utts, last.n, fc[0].n, fc_in_dtype, fc[0].cin, fc[0].w_plain_dev) &&
-      tail_ws_bytes >= pool_fc_workspace_bytes(n_utts, last.n, fc[0].n, fc_in_dtype)) {
-    // the tail in ONE launch: pooling finalize + first segment layer (seg_fused.cu); the pooled matrix is never materialised
-    // (debug-build A/B switch only: measured slower than the two launches, see use_fused_tail)
-    const bool final_layer = n_fc == 1;
-    void* y = final_layer ? static_cast<void*>(out_dev) : fc_tmp_dev;
-    const int y_dtype = final_layer ? XVEC_F32 : fc[1].dtype;
-    const int64_t y_ld = final_layer ? out_ld : fc[0].n;
-    rc = pool_fc_dispatch(part_dev, utt_slot_start_dev, n_pool_dev, n_utts, last.n, bn_last_scale_dev, bn_last_shift_dev, fc[0].w_plain_dev,
-                          fc_in_dtype, fc[0].cin, fc[0].bias_dev, fc[0].n, final_layer ? 0 : 1, y, y_dtype, y_ld, tail_ws_dev, tail_ws_bytes, stream);
-    if (rc) return rc;
-    first_fc = 1;
-    a = y;
-    a_ld = y_ld;
-  } else {
   if (fc_in_dtype == XVEC_BF16 && !pooled_lp_dev) return set_error(XVEC_E_ARG, "pooled_lp_dev is required for bf16 segment layers");
   rc = xvec_pool_finalize(part_dev, utt_slot_start_dev, n_pool_dev, n_utts, last.n, bn_last_scale_dev, bn_last_shift_dev, nullptr, pooled_dev,
                           fc_in_dtype == XVEC_BF16 ? pooled_lp_dev : nullptr, XVEC_BF16, 2 * static_cast<int64_t>(last.n), stream);
   if (rc) return rc;
-#ifdef XVEC_DEBUG
-  if (skip_tail >= 1) return XVEC_OK;
-#endif
-  a = fc_in_dtype == XVEC_BF16 ? pooled_lp_dev : static_cast<const void*>(pooled_dev);
-  a_ld = 2 * static_cast<int64_t>(last.n);
-  }
-  for (int i = first_fc; i < n_fc; ++i) {
+  const void* a = fc_in_dtype == XVEC_BF16 ? pooled_lp_dev : static_cast<const void*>(pooled_dev);
+  int64_t a_ld = 2 * static_cast<int64_t>(last.n);
+  for (int i = 0; i < n_fc; ++i) {
     const bool final_layer = i == n_fc - 1;
     void* y = final_layer ? static_cast<void*>(out_dev) : fc_tmp_dev;
     const int y_dtype = final_layer ? XVEC_F32 : fc[i + 1].dtype;
     const int64_t y_ld = final_layer ? out_ld : fc[i].n;
-    if (fc[i].w_plain_dev && use_fc_small() &&
-        fc_small_supported(n_utts, fc[i].cin, fc[i].n, a_ld, fc[i].cin, a, fc[i].w_plain_dev, fc[i].dtype)) {
+    if (fc[i].w_plain_dev && fc_small_supported(n_utts, fc[i].cin, fc[i].n, a_ld, fc[i].cin, a, fc[i].w_plain_dev, fc[i].dtype)) {
       // small-footprint kernel: runs next to the resident stack CTAs of the next batch instead of waiting for free SMs
       rc = fc_small_dispatch(a, fc[i].dtype, n_utts, fc[i].cin, a_ld, fc[i].w_plain_dev, fc[i].n, fc[i].cin, fc[i].bias_dev,
                              final_layer ? 0 : 1, y, y_dtype, y_ld, stream);

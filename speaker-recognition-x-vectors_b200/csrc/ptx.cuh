@@ -127,44 +127,18 @@ __device__ __forceinline__ void cluster_sync_all() {
 }
 
 // ----------------------------------------------------------------------------- cluster-scope hand-off of a 32-bit word
-// Writer: st.shared::cluster into the peer CTA, then a release.cluster arrive on the peer's barrier; reader: acquire.cluster
-// wait on its own barrier, then a plain shared load.
-__device__ __forceinline__ void st_shared_cluster_u32(uint32_t cluster_addr, uint32_t v) {
-  asm volatile("st.shared::cluster.u32 [%0], %1;" ::"r"(cluster_addr), "r"(v) : "memory");
-}
-// The same hand-off without a cluster-scope release / acquire pair: the word travels as an ASYNC store that completes 4 bytes of
-// transaction on the peer's barrier (st.async ... mbarrier::complete_tx::bytes), which the writer has armed with a remote
-// arrive.expect_tx.  Observing the phase completion makes the word visible (the mbarrier's transaction mechanism, as for TMA
-// loads), so the reader waits with an ordinary try_wait.  ptxas implements `mbarrier.arrive.release.cluster` as MEMBAR.ALL.GPU and
-// every `try_wait.acquire.cluster` as CCTL.IVALL (an L1 invalidation): one GPU-scope barrier per work item in the scheduler warp
-// and twelve L1 invalidations per work item in the peer CTA went away with this.
+// The word travels as an ASYNC store that completes 4 bytes of transaction on the peer's barrier (st.async ...
+// mbarrier::complete_tx::bytes), which the writer has armed with a remote arrive.expect_tx.  Observing the phase completion makes
+// the word visible (the mbarrier's transaction mechanism, as for TMA loads), so the reader waits with an ordinary try_wait.  The
+// plain form — st.shared::cluster, a release.cluster arrive, acquire.cluster waits — costs more: ptxas implements
+// `mbarrier.arrive.release.cluster` as MEMBAR.ALL.GPU and every `try_wait.acquire.cluster` as CCTL.IVALL (an L1 invalidation),
+// i.e. one GPU-scope barrier per work item in the scheduler warp and twelve L1 invalidations per work item in the peer CTA
+// (tdnn_stack.cu on a B200: 267.0 vs 268.8 us per launch at 256 x 300 frames in bf16, 1 314 vs 1 338 us at 64 x 6000).
 __device__ __forceinline__ void mbar_arrive_expect_tx_cluster(uint32_t cluster_addr, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cluster.b64 _, [%0], %1;" ::"r"(cluster_addr), "r"(bytes) : "memory");
 }
 __device__ __forceinline__ void st_async_cluster_u32(uint32_t cluster_addr, uint32_t v, uint32_t cluster_mbar) {
   asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.u32 [%0], %1, [%2];" ::"r"(cluster_addr), "r"(v), "r"(cluster_mbar) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_release_cluster(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait_cluster(uint64_t* bar, uint32_t parity) {
-  uint32_t done;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(done)
-      : "r"(smem_u32(bar)), "r"(parity)
-      : "memory");
-  return done != 0;
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity, uint32_t code) {
-  uint32_t spins = 0;
-  while (!mbar_try_wait_cluster(bar, parity)) {
-    if (++spins > (1u << 26)) {
-      watchdog_trip(code);
-    }
-  }
 }
 
 // ----------------------------------------------------------------------------- inter-CTA flags in global memory
@@ -183,30 +157,13 @@ __device__ __forceinline__ uint32_t atom_add_acq_rel_cta_shared_u32(uint32_t sme
   asm volatile("atom.acq_rel.cta.shared::cta.add.u32 %0, [%1], %2;" : "=r"(old) : "r"(smem_addr), "r"(v) : "memory");
   return old;
 }
-// The 128-byte line at `p` (128-byte aligned) holds dead data: L2 may drop it instead of writing it back to HBM.  Semantically a
-// weak write of an indeterminate value — only ever issued on lines whose last reader has finished and whose next access is a write.
-__device__ __forceinline__ void discard_l2_line(const void* p) { asm volatile("discard.global.L2 [%0], 128;" ::"l"(p) : "memory"); }
-__device__ __forceinline__ uint32_t atom_add_relaxed_gpu_u32(uint32_t* p, uint32_t v) {
-  uint32_t old;
-  asm volatile("atom.relaxed.gpu.global.add.u32 %0, [%1], %2;" : "=r"(old) : "l"(p), "r"(v) : "memory");
-  return old;
-}
 // Orders generic-proxy accesses (the flag acquire / release) against async-proxy accesses (TMA loads / stores) of this thread.
 // The data behind the flags (activation tiles) lives in GLOBAL memory, so the fence is restricted to that state space: ptxas
 // emits FENCE.VIEW.ASYNC.G for it, while the unrestricted `fence.proxy.async` is MEMBAR.ALL.GPU + FENCE.VIEW.ASYNC.S — a
 // GPU-scope memory barrier of ~1 000 cycles that sat in the dependency warp's per-tile chain (scheduler -> flags -> fence ->
 // producer may start) and in every publication of a stored tile (measured: 287 -> 281 us per launch in the debug build with
-// the fences switched off; profiles/r02_experiments.txt).  XVEC_PROXY_FENCE_ALL = 1 restores the unrestricted form.
-#ifndef XVEC_PROXY_FENCE_ALL
-#define XVEC_PROXY_FENCE_ALL 0
-#endif
-__device__ __forceinline__ void fence_proxy_async_global() {
-#if XVEC_PROXY_FENCE_ALL
-  asm volatile("fence.proxy.async;" ::: "memory");
-#else
-  asm volatile("fence.proxy.async.global;" ::: "memory");
-#endif
-}
+// the fences switched off; profiles/r02_experiments.txt).
+__device__ __forceinline__ void fence_proxy_async_global() { asm volatile("fence.proxy.async.global;" ::: "memory"); }
 
 // ----------------------------------------------------------------------------- proxies / fences
 __device__ __forceinline__ void fence_proxy_async_smem() {

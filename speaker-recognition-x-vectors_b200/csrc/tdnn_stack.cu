@@ -55,42 +55,21 @@ namespace xvec {
 // Measured: MMA-warp cycles per TDNN2/3 tile 9 / 10 / 11 / 12 slots: 16 480 / 14 050 / 13 540 / 13 090; whole launch 326.8 /
 // 299.2 / 295.8 / 297.1 us (debug builds) — the launch as a whole gains 1-2 % over the separate rings, within box-to-box spread.
 // Shared memory per CTA: 1 KiB alignment slack + the ring + the TMA-store staging of the 8 epilogue warps.  bf16 activations:
-// 10 slots + two 2 KiB boxes (32 rows x 64 bytes) per warp = 203 KiB (until the last sessions: 11 slots + one box = 204 KiB); float32 activations: 10 slots + one 4 KiB box (32 rows x
+// 10 slots + two 2 KiB boxes (32 rows x 64 bytes) per warp = 203 KiB; float32 activations: 10 slots + one 4 KiB box (32 rows x
 // 128 bytes) = 203 KiB.  NOT the 227 KiB a CTA could have: the kernels of a batch's tail (pooling finalize + segment layers)
 // must fit on the SM NEXT TO a resident CTA of the next batch's stack kernel (about 20 KiB of shared memory and 20 K registers
 // stay free), otherwise they wait for a whole stack kernel to drain — measured in round 1: ~24 us of a 325 us step.  Measured
 // here (256 x 300, bf16, us per launch on one box): 12 slots / 1 box 290.5, 11 / 2 boxes 291.9, 11 / 1 box 292.2 — the last
 // slot buys less than the co-residency it would cost.
-// Last sessions of round 2 (after the fences / publication were made cheap, so that the store epilogue weighs more): 10 slots + TWO
-// boxes per warp (staging chunk k+1 while the store of chunk k still reads its box) 262.8 us against 11 slots + one box 263.7
-// (64 x 6000: 1 297 vs 1 303) — 203 KiB, the default now; the wait for the box's previous store sits after the chunk's math.
-// XVEC_MMA_FIXED = 1: the MMA warp runs the K loop specialised at compile time for the tap counts the x-vector stack has
-// (mma_tile_fixed); 0: the generic loop for every layer (mma_tile).  Same MMAs in the same order either way.
-#ifndef XVEC_MMA_FIXED
-#define XVEC_MMA_FIXED 1
-#endif
-// XVEC_ITEM_ST_ASYNC = 1: the scheduler hands a work item to the peer CTA with st.async + the barrier's transaction count instead
-// of st.shared::cluster + a release.cluster arrive / acquire.cluster waits (ptx.cuh: st_async_cluster_u32).
-#ifndef XVEC_ITEM_ST_ASYNC
-#define XVEC_ITEM_ST_ASYNC 1
-#endif
-#ifndef XVEC_PUBLISH_PER_CTA
-#define XVEC_PUBLISH_PER_CTA 1  // one gpu-scope release per stored tile and CTA (the last of its 8 epilogue warps) instead of one per warp
-#endif
-#ifndef XVEC_LATE_WAIT_READ
-#define XVEC_LATE_WAIT_READ 1
-#endif
-#ifndef XVEC_RING_SLOTS_BF16
-#define XVEC_RING_SLOTS_BF16 10
-#define XVEC_RING_SLOTS_F32 10
-#define XVEC_STAGE_BOXES_BF16 2
-#endif
+// Once the fences / publication were made cheap (round 2), the store epilogue weighs more: 10 slots + TWO boxes per bf16 warp
+// (staging chunk k+1 while the store of chunk k still reads its box) 262.8 us against 11 slots + one box 263.7 (64 x 6000:
+// 1 297 vs 1 303).
 template <bool kAllTf32>
 struct StackCfg {
-  static constexpr int SLOTS = kAllTf32 ? XVEC_RING_SLOTS_F32 : XVEC_RING_SLOTS_BF16;
+  static constexpr int SLOTS = 10;
   static constexpr int BOX_W = kAllTf32 ? 128 : 64;                     // bytes per row of a store box (32 rows x 32 columns)
   static constexpr int BOX_BYTES = 32 * BOX_W;
-  static constexpr int NBUF = kAllTf32 ? 1 : XVEC_STAGE_BOXES_BF16;      // store boxes in flight per epilogue warp
+  static constexpr int NBUF = kAllTf32 ? 1 : 2;                          // store boxes in flight per epilogue warp
   static constexpr int STAGE_BYTES = NBUF * BOX_BYTES;                   // staging per epilogue warp
 };
 constexpr int SLAB_ROWS_MAX = BM_CTA + XVEC_STACK_MAX_TAP_OFFSET;  // frame rows per slab (128 + the largest tap offset, <= 8)
@@ -131,10 +110,6 @@ struct StackParams {
   StackLayer L[XVEC_MAX_STACK];
   unsigned* counter;          // next work item (zeroed before the launch)
   unsigned* ready;            // [(n_layers-1)][m_tiles] completed epilogue-warp stores per tile (zeroed before the launch)
-  unsigned* consumed;         // [n_layers][m_tiles] epilogue warps that have seen the tile's MMAs complete (layers >= 1; zeroed)
-  char* act[2];               // the two ping-pong activation buffers (layer l >= 1 reads act[(l-1) & 1]) ...
-  long long act_ld_bytes;     // ... their row pitch; 0 = do not discard consumed activations 
-  int act_es;                 // bytes per activation element
   const int* row_utt;
   const int* blk_slot_base;
   float* part;
@@ -278,6 +253,7 @@ __device__ __forceinline__ void mma_tile(uint32_t ring_addr, uint32_t full_addr,
 // straight-line code with compile-time commit / probe sets (umma_step_fixed), the operand swap of the pooled layer is a template
 // argument, single-tap layers unroll two chunks, so the descriptor arithmetic of one step is scheduled under the issue of its
 // neighbour.  Same ring protocol and the same MMAs in the same order as mma_tile (which stays for every other tap count).
+// Measured against mma_tile for every layer (B200, 256 x 300, us per launch): 277.0 vs 277.9 in bf16, 509.4 vs 512.0 in TF32.
 template <bool kTf32, int kSlots, int kTaps, bool kSwap>
 __device__ __forceinline__ void mma_tile_fixed(uint32_t ring_addr, uint32_t full_addr, uint32_t empty_addr, uint32_t d, const TileK k,
                                                MmaRing<kSlots>& r, unsigned long long& c_wait, unsigned long long& c_step) {
@@ -333,7 +309,7 @@ template <bool kAllTf32>
 constexpr int stack_smem_bytes() { return 1024 + StackCfg<kAllTf32>::SLOTS * SLOT_BYTES + EPI_WARPS * StackCfg<kAllTf32>::STAGE_BYTES; }
 static_assert(stack_smem_bytes<false>() <= 227 * 1024 - 1024 && stack_smem_bytes<true>() <= 227 * 1024 - 1024,
               "operand ring + store staging (+ 1 KiB of static barriers) exceed the 227 KiB of shared memory a CTA can have");
-constexpr int STACK_SMEM_LEFT_FOR_TAIL = 20 * 1024;  // what a co-resident tail kernel may use (fc_small.cu, seg_fused.cu assert against it)
+constexpr int STACK_SMEM_LEFT_FOR_TAIL = 20 * 1024;  // what a co-resident tail kernel may use (fc_small.cu takes 5 KiB)
 static_assert(228 * 1024 - stack_smem_bytes<false>() - 2048 - 2 * 1024 >= STACK_SMEM_LEFT_FOR_TAIL &&
               228 * 1024 - stack_smem_bytes<true>() - 2048 - 2 * 1024 >= STACK_SMEM_LEFT_FOR_TAIL,
               "the stack kernel must leave room on the SM for the tail kernels of the previous batch");
@@ -394,12 +370,7 @@ tdnn_stack_kernel(const __grid_constant__ StackMaps maps, const __grid_constant_
   auto ring_read = [&](int it) -> uint32_t {
     const int slot = it % SCHED_SLOTS;
     const uint32_t sph = (it / SCHED_SLOTS) & 1u;
-#if XVEC_ITEM_ST_ASYNC
     mbar_wait(&sfull_bar[slot], sph, 6);  // leader: the scheduler's arrive; peer: the 4 bytes of the scheduler's st.async have landed
-#else
-    if (rank == 0) mbar_wait(&sfull_bar[slot], sph, 6);
-    else mbar_wait_cluster(&sfull_bar[slot], sph, 6);
-#endif
     const uint32_t item = *reinterpret_cast<volatile uint32_t*>(&sched_item[slot]);
     __syncwarp();
     if (lane == 0) mbar_arrive_cluster(mapa_u32(smem_u32(&sempty_bar[slot]), 0));
@@ -498,10 +469,10 @@ tdnn_stack_kernel(const __grid_constant__ StackMaps maps, const __grid_constant_
         const TileK tk_(L);
         auto run = [&](auto tf_c) {
           constexpr bool tf = decltype(tf_c)::value;
-          if (XVEC_MMA_FIXED && tk_.taps == 1) {
+          if (tk_.taps == 1) {
             if (pooled) mma_tile_fixed<tf, RING_SLOTS, 1, true>(ring_addr, full_addr, empty_addr, d, tk_, ring, c_full, c_step);
             else mma_tile_fixed<tf, RING_SLOTS, 1, false>(ring_addr, full_addr, empty_addr, d, tk_, ring, c_full, c_step);
-          } else if (XVEC_MMA_FIXED && tk_.taps == 3) {
+          } else if (tk_.taps == 3) {
             if (pooled) mma_tile_fixed<tf, RING_SLOTS, 3, true>(ring_addr, full_addr, empty_addr, d, tk_, ring, c_full, c_step);
             else mma_tile_fixed<tf, RING_SLOTS, 3, false>(ring_addr, full_addr, empty_addr, d, tk_, ring, c_full, c_step);
           } else {
@@ -564,14 +535,9 @@ tdnn_stack_kernel(const __grid_constant__ StackMaps maps, const __grid_constant_
         if (lane == 0) {
           sched_item[slot] = item;
           mbar_arrive(&sfull_bar[slot]);
-#if XVEC_ITEM_ST_ASYNC
           const uint32_t peer_bar = mapa_u32(smem_u32(&sfull_bar[slot]), 1);
           mbar_arrive_expect_tx_cluster(peer_bar, 4);
           st_async_cluster_u32(mapa_u32(smem_u32(&sched_item[slot]), 1), item, peer_bar);
-#else
-          st_shared_cluster_u32(mapa_u32(smem_u32(&sched_item[slot]), 1), item);
-          mbar_arrive_release_cluster(mapa_u32(smem_u32(&sfull_bar[slot]), 1));
-#endif
         }
         __syncwarp();
       } else {
@@ -620,7 +586,8 @@ tdnn_stack_kernel(const __grid_constant__ StackMaps maps, const __grid_constant_
     int pend_it = 0;           // ... and the work-item index it was processed at (all epilogue warps of a CTA see the same sequence)
     // Publish `pend`: lane 0 owns the warp's bulk groups; once they are complete the tile's rows are in global memory.  The eight
     // epilogue warps of a CTA count themselves in shared memory (acq_rel at CTA scope), and the LAST one to arrive publishes for
-    // all: one fence + one red.release.gpu (+ 8) per tile and CTA instead of eight — a gpu-scope release is a MEMBAR.ALL.GPU.
+    // all: one fence + one red.release.gpu (+ 8) per tile and CTA instead of eight — a gpu-scope release is a MEMBAR.ALL.GPU
+    // (measured on a B200: 262.3 vs 264.5 us per launch against one release per warp; 256 x 300, bf16).
     // A tile's counter is free-running (8 arrivals per use; at most three stored tiles of a CTA are unpublished at any time: a
     // warp publishes tile i before it leaves tile i + 1, and nobody enters tile i + 2 before every warp has released tile i).
     // kAll: wait for every bulk group of this thread; otherwise for all but the BOXES most recent (the current tile's).
@@ -628,15 +595,10 @@ tdnn_stack_kernel(const __grid_constant__ StackMaps maps, const __grid_constant_
       if (lane == 0 && !XVEC_SDBG(p, 2)) {
         if (all) tma_store_wait_all();
         else tma_store_wait_done<BOXES>();
-#if XVEC_PUBLISH_PER_CTA
         if ((atom_add_acq_rel_cta_shared_u32(smem_u32(&pub_cnt[pend_it & 3]), 1u) & (EPI_WARPS - 1)) == EPI_WARPS - 1) {
           if (!XVEC_SDBG(p, 4)) fence_proxy_async_global();
           red_release_gpu_add_u32(pend, static_cast<uint32_t>(EPI_WARPS));
         }
-#else
-        if (!XVEC_SDBG(p, 4)) fence_proxy_async_global();
-        red_release_gpu_add_u32(pend, 1u);
-#endif
       }
       pend = nullptr;
     };
@@ -674,31 +636,6 @@ tdnn_stack_kernel(const __grid_constant__ StackMaps maps, const __grid_constant_
       mbar_wait(&tfull_bar[buf], use, 4);
       tc_fence_after();
       XVEC_CNT(e_t1 = clock64(); e_wait[pooled_tile ? 0 : 1] += e_t1 - e_t0;)
-#ifdef XVEC_DEBUG
-      if (layer > 0 && p.act_ld_bytes) {
-        // EXPERIMENT (debug builds, XVEC_STACK_DISCARD=1; measured on B200: DRAM writes per launch 187 MB -> 17.5 MB, but CCTL.RML2
-        // retires one 128-byte line per ~75 cycles and SM, so the 2.4 M lines of a 256 x 300 batch make the launch 3x slower:
-        // 296 -> 934 us.  Kept as the record of that measurement, not compiled into the product library.)
-        // Dead activations: every MMA of this item is complete, so its share of the reads of layer-1's rows is over.  The warp
-        // that sees the LAST of the (n_tiles x 2 CTAs x EPI_WARPS) arrivals for (layer, mt) tells L2 to drop rows
-        // [256 mt + 8, 256 mt + 256) of the input buffer instead of writing them back to HBM: the first 8 rows are also read by
-        // tile mt-1 (tap offsets <= 8), everything else has no reader left, and the next access is the write of tile
-        // (layer+1, mt), which waits for ready[layer][mt] — published by this very warp only after the discards below.
-        unsigned old = 0;
-        if (lane == 0) old = atom_add_relaxed_gpu_u32(p.consumed + static_cast<size_t>(layer) * p.m_tiles + mt, 1u);
-        old = __shfl_sync(0xffffffffu, old, 0);
-        if (old + 1 == static_cast<unsigned>(L.n_tiles) * 2u * EPI_WARPS) {
-          const int r_lo = mt * BM + XVEC_STACK_MAX_TAP_OFFSET;
-          const int r_hi = min(mt * BM + BM, p.rows);
-          const int lines = (p.L[layer - 1].n * p.act_es) >> 7;  // 128-byte lines per row (stored layers are whole 256-channel tiles)
-          char* in = p.act[(layer - 1) & 1];
-          for (int r = r_lo; r < r_hi; ++r) {
-            char* row = in + static_cast<long long>(r) * p.act_ld_bytes;
-            for (int i = lane; i < lines; i += 32) discard_l2_line(row + (i << 7));
-          }
-        }
-      }
-#endif
       const uint32_t tbase = tmem_base + buf * BN + (static_cast<uint32_t>(q * 32) << 16);
       const int row0 = m0 + q * 32;
       bool released = false;
@@ -737,10 +674,6 @@ tdnn_stack_kernel(const __grid_constant__ StackMaps maps, const __grid_constant_
           uint32_t(&v)[32] = (k & 1) ? vb : va;
           if (k + 1 < BOXES) tmem_ld_32x32(tbase + cbeg + 32 * (k + 1), (k & 1) ? va : vb);
           uint8_t* ob = out_stage + (store_seq % NBUF) * BOX_BYTES;
-#if !XVEC_LATE_WAIT_READ
-          if (lane == 0) tma_store_wait_read<NBUF - 1>();  // the store that last used this box has read it
-          __syncwarp();
-#endif
           const int col0 = n0 + cbeg + k * 32;
           // r = relu(acc + bias') — every BatchNorm is folded forward into the next layer's weights (xvector.py)
           float o[32];
@@ -752,11 +685,10 @@ tdnn_stack_kernel(const __grid_constant__ StackMaps maps, const __grid_constant_
             const float2 d = __fadd2_rn(make_float2(__uint_as_float(v[j4 + 2]), __uint_as_float(v[j4 + 3])), make_float2(bb.z, bb.w));
             o[j4 + 0] = a.x; o[j4 + 1] = a.y; o[j4 + 2] = d.x; o[j4 + 3] = d.y;
           }
-#if XVEC_LATE_WAIT_READ
           // the store that last used this box must have read it — checked only now, after the bias / ReLU math of this chunk
+          // (measured on a B200: 263.7 vs 264.3 us per launch against the wait before the math; 256 x 300, bf16)
           if (lane == 0) tma_store_wait_read<NBUF - 1>();
           __syncwarp();
-#endif
           // row `lane` of the box, 16-byte pieces XOR-swizzled like the tensor map's swizzle mode expects
           uint8_t* orow = ob + lane * BOX_W;
           if constexpr (!kAllTf32) {  // SWIZZLE_64B: piece index ^ address bits [7,9) = (row / 2) % 4
@@ -889,7 +821,7 @@ int64_t stack_plan(int64_t rows, int n_layers, const int32_t* n_tiles_per_layer,
 int64_t stack_ctrl_bytes(int64_t rows, int n_layers) {
   if (rows <= 0 || n_layers < 2) return 0;
   const int64_t m_tiles = (rows + BM - 1) / BM;
-  return 256 + (n_layers - 1) * m_tiles * 4 + n_layers * m_tiles * 4;  // counters (64 words) | ready[layers - 1][m_tiles] | consumed[layers][m_tiles]
+  return 256 + (n_layers - 1) * m_tiles * 4;  // counters (64 words) | ready[layers - 1][m_tiles]
 }
 
 XVEC_DEFINE_WATCHDOG_BINDER(bind_watchdog_stack)
@@ -1032,19 +964,7 @@ static int build_plan(StackPlan& pl, const XvecLayerDesc* tdnn, int n_tdnn, cons
   if (rc) return rc;
   l2_policies(&p.pol_a, &p.pol_b, &p.pol_y);
   p.runahead = STACK_RUNAHEAD;
-#ifdef XVEC_DEBUG
-  if (const char* e = getenv("XVEC_STACK_RUNAHEAD")) {
-    const int v = atoi(e);
-    if (v >= 1 && v < CREDIT_BARS) p.runahead = v;
-  }
-#endif
-  int64_t pairs = static_cast<int64_t>(p.total_items) < max_pairs ? p.total_items : max_pairs;
-#ifdef XVEC_DEBUG
-  if (const char* e = getenv("XVEC_STACK_PAIRS")) {  // experiment: fewer CTA pairs (is the operand stream a per-SM or a global limit?)
-    const int v = atoi(e);
-    if (v > 0 && v < pairs) pairs = v;
-  }
-#endif
+  const int64_t pairs = static_cast<int64_t>(p.total_items) < max_pairs ? p.total_items : max_pairs;
   pl.grid = 2 * static_cast<int>(pairs);
   return XVEC_OK;
 }
@@ -1109,11 +1029,6 @@ int stack_dispatch(const XvecLayerDesc* tdnn, int n_tdnn, const void* x, int64_t
   }
   p.counter = static_cast<unsigned*>(ctrl);
   p.ready = reinterpret_cast<unsigned*>(static_cast<char*>(ctrl) + 256);
-  p.consumed = p.ready + static_cast<size_t>(n_tdnn - 1) * p.m_tiles;
-  p.act[0] = static_cast<char*>(act0);
-  p.act[1] = static_cast<char*>(act1);
-  p.act_es = tdnn[1].dtype == XVEC_BF16 ? 2 : 4;
-  p.act_ld_bytes = 0;
   p.row_utt = row_utt;
   p.blk_slot_base = blk_slot_base;
   p.part = part;
@@ -1121,11 +1036,6 @@ int stack_dispatch(const XvecLayerDesc* tdnn, int n_tdnn, const void* x, int64_t
   {
     const char* e = getenv("XVEC_STACK_DBG");
     p.dbg = e ? atoi(e) : 0;
-    if (getenv("XVEC_STACK_DISCARD")) {  // experiment: drop consumed activation rows from L2 (discard.global.L2) instead of writing them back
-      const long long ldb = act_ld * p.act_es;
-      const bool aligned = ((reinterpret_cast<uintptr_t>(act0) | reinterpret_cast<uintptr_t>(act1)) & 127u) == 0 && ldb % 128 == 0;
-      p.act_ld_bytes = aligned ? ldb : 0;
-    }
   }
 #endif
   cudaStream_t st = static_cast<cudaStream_t>(stream);

@@ -39,12 +39,6 @@ bool fc_small_supported(int64_t rows, int k, int n, int64_t x_ld, int64_t w_ld, 
 int fc_small_dispatch(const void* x, int dtype, int64_t rows, int k, int64_t x_ld, const void* w, int n, int64_t w_ld, const float* bias,
                       int relu, void* y, int y_dtype, int64_t y_ld, void* stream);
 int64_t splitk_workspace_bytes(int64_t rows, int cin, int taps, int n, int dtype);
-// seg_fused.cu: pooling finalize fused with the first segment layer (one launch for the tail of a batch).
-bool pool_fc_supported(int n_utts, int p, int n, int dtype, int64_t w_ld, const void* w);
-int64_t pool_fc_workspace_bytes(int n_utts, int p, int n, int dtype);
-int pool_fc_dispatch(const float* part, const int32_t* slot_start, const int32_t* n_rows, int n_utts, int p, const float* scale,
-                     const float* shift, const void* w, int dtype, int64_t w_ld, const float* bias, int n, int relu, void* out,
-                     int out_dtype, int64_t out_ld, void* ws, int64_t ws_bytes, void* stream);
 
 // Per-device one-time initialisation (cudaFuncSetAttribute, binding the watchdog word) that is safe when several host threads
 // — one per device or several per device — make their first call at the same time.

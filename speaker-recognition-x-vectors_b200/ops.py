@@ -315,27 +315,3 @@ def linear_small(x: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor | Non
         check(lib.xvec_linear_small(ptr(x), dtype_code(x.dtype), x.shape[0], x.shape[1], x_ld, ptr(weight), weight.shape[0], w_ld, ptr(b),
                                     int(bool(relu)), ptr(out), dtype_code(out_dtype), out.stride(0), stream_ptr()))
     return out
-
-
-def pool_fc_fused(part: torch.Tensor, slot_start: torch.Tensor, n_rows: torch.Tensor, p: int, weight: torch.Tensor,
-                  bias: torch.Tensor | None = None, bn_scale=None, bn_shift=None, relu: bool = False,
-                  out_dtype: torch.dtype = torch.float32, workspace: torch.Tensor | None = None) -> torch.Tensor:
-    """Pooling finalize fused with the first segment layer (xvec_pool_fc_fused): act([mean || std] W' + bias) per utterance from the
-    pooling partials `part` (n_slots, 2, p); weight (n, 2p) row-major, bfloat16 or float32 (TF32 math).  Returns (n_utts, n)."""
-    _require_cuda(part, slot_start, n_rows, weight, bias, bn_scale, bn_shift, workspace)
-    lib = _lib.load()
-    n_utts, n = n_rows.numel(), weight.shape[0]
-    w_ld = _rowmajor_2d(weight, "weight")
-    if weight.shape[1] != 2 * p:
-        raise ValueError("weight must be (n, 2p)")
-    code = dtype_code(weight.dtype)
-    need = lib.xvec_pool_fc_workspace_bytes(n_utts, p, n, code)
-    if workspace is None:
-        workspace = torch.zeros(need, dtype=torch.uint8, device=part.device)
-    out = torch.empty((n_utts, n), dtype=out_dtype, device=part.device)
-    b = None if bias is None else bias.detach().float().contiguous()
-    with _lib.on_device(part.device):
-        check(lib.xvec_pool_fc_fused(ptr(part), ptr(slot_start), ptr(n_rows), n_utts, p, ptr(bn_scale), ptr(bn_shift), ptr(weight), code, w_ld,
-                                     ptr(b), n, int(bool(relu)), ptr(out), dtype_code(out_dtype), out.stride(0), ptr(workspace),
-                                     workspace.numel(), stream_ptr()))
-    return out

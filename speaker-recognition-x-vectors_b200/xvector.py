@@ -98,8 +98,7 @@ class _Scratch:
         self.ld = (max(widths) + per16 - 1) // per16 * per16
         self.rows_cap = self.slots_cap = self.utts_cap = 0
         self.act = self.part = self.pooled = self.pooled_lp = self.ctrl = None
-        self.fc_tmp = self.ws = self.tail_ws = None
-        self.ws_for = self.tail_for = None
+        self.fc_tmp = self.ws = self.ws_for = None
 
     def ensure(self, rows, n_slots, n_utts):
         if rows > self.rows_cap:
@@ -131,14 +130,6 @@ class _Scratch:
             if need > 0 and (self.ws is None or self.ws.numel() < need):
                 self.ws = torch.empty(need, dtype=torch.uint8, device=self.device)
             self.ws_for = key
-        # scratch of the fused pooling-finalize + segment-layer kernel: arrival counters + float32 partial tiles; zero-filled once
-        # (the kernel leaves its counters at zero), sized for the slot's utterance capacity
-        cap = max(n_utts, self.utts_cap)
-        tkey = (cap, fc_shapes[0])
-        if self.tail_for != tkey:
-            need = _lib.load().xvec_pool_fc_workspace_bytes(cap, self.pool_dim, fc_shapes[0][1], _lib.dtype_code(self.act_dtype))
-            self.tail_ws = torch.zeros(need, dtype=torch.uint8, device=self.device) if need > 0 else None
-            self.tail_for = tkey
 
 
 class XVectorModel(nn.Module):
@@ -415,8 +406,7 @@ class XVectorModel(nn.Module):
                 pipe["tdnn"], pipe["n_tdnn"], p(x), lay.rows, x.stride(0), p(sc.act[0]), p(sc.act[1]), sc.ld, p(lay.row_utt),
                 p(lay.blk_slot_base), p(lay.utt_slot_start), p(lay.n_pool), lay.n_utts, p(sc.part), p(pipe["scale5"]), p(pipe["shift5"]),
                 p(sc.pooled), p(sc.pooled_lp), pipe["fc"], pipe["n_fc"], p(sc.fc_tmp), p(sc.ws),
-                0 if sc.ws is None else sc.ws.numel(), p(out), out.stride(0), p(sc.tail_ws), 0 if sc.tail_ws is None else sc.tail_ws.numel(),
-                p(sc.ctrl), sc.ctrl.numel(), _lib.stream_ptr()))
+                0 if sc.ws is None else sc.ws.numel(), p(out), out.stride(0), p(sc.ctrl), sc.ctrl.numel(), _lib.stream_ptr()))
         return out
 
     # ------------------------------------------------------------------ reference surface
