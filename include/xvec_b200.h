@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define XVEC_ABI_VERSION 6
+#define XVEC_ABI_VERSION 7
 
 #if defined(__GNUC__)
 #define XVEC_API __attribute__((visibility("default")))
@@ -213,10 +213,12 @@ XVEC_API int xvec_linear_small(const void* x_dev, int dtype, int64_t rows, int k
  * layer's packed weights, the last TDNN layer's BatchNorm is passed as bn_last_scale/shift (or NULL).
  *   x_dev (rows, tdnn[0].cin) of tdnn[0].dtype, row stride x_ld (window form: see xvec_tdnn_stack);  act0/act1: ping-pong activation buffers (rows, act_ld) of the
  *   dtype of tdnn[1];  layout arrays as for xvec_tdnn_pool_fused / xvec_pool_finalize;  part_dev (n_slots, 2, n_last);
- *   pooled_dev float32 (n_utts, 2 n_last);  pooled_lp_dev same in fc[0].dtype when that is XVEC_BF16, else NULL;
+ *   pooled_dev float32 (n_utts, 2 n_last);  pooled_lp_dev NULL or a bfloat16 copy of it (n_utts, 2 n_last), required when
+ *   fc[0].dtype is XVEC_BF16 (the first segment layer reads it);  fc: n_fc segment layers (taps == 1);
  *   fc_tmp_dev (n_utts, fc[0].n) of fc[1].dtype when n_fc == 2;  out_dev float32 (n_utts, fc[n_fc-1].n), row stride out_ld;
  *   splitk_ws_dev: scratch for the segment layers (see xvec_splitk_workspace_bytes) or NULL;
- *   ctrl_dev / ctrl_bytes: scratch of xvec_tdnn_stack or NULL / 0. */
+ *   ctrl_dev / ctrl_bytes: scratch of xvec_tdnn_stack or NULL / 0.
+ *   n_fc == 0 ends the call after xvec_pool_finalize; fc_host, fc_tmp_dev, splitk_ws_dev and out_dev may then be NULL. */
 XVEC_API int xvec_extract_forward(const XvecLayerDesc* tdnn_host, int n_tdnn, const void* x_dev, int64_t rows, int64_t x_ld,
                          void* act0_dev, void* act1_dev, int64_t act_ld, const int32_t* row_utt_dev,
                          const int32_t* blk_slot_base_dev, const int32_t* utt_slot_start_dev, const int32_t* n_pool_dev,

@@ -16,7 +16,7 @@ LIB_PATH = os.environ.get("XVEC_LIB") or os.path.join(HERE, "libxvec_b200.so")  
 F32, BF16 = 0, 1
 E_ARG, E_CUDA, E_DEVICE = -1, -2, -3
 TILE_N, POOL_BLOCK, POOL_CHUNK, MAX_TAPS = 256, 128, 128, 8
-ABI_VERSION = 6
+ABI_VERSION = 7
 MAX_STACK = 6
 STACK_MAX_TAP_OFFSET = 8  # XVEC_STACK_MAX_TAP_OFFSET
 

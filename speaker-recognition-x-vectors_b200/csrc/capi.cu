@@ -83,6 +83,20 @@ int read_watchdog() {
   return w ? static_cast<int>(*reinterpret_cast<volatile unsigned int*>(w)) : 0;
 }
 
+int layer_desc(XvecLayerDesc* l, const void* w_packed, const float* bias, int n, int cin, int taps, int dtype, const int32_t* tap_offsets) {
+  if (!tap_offsets) return set_error(XVEC_E_ARG, "tap_offsets_host is NULL");
+  if (taps < 1 || taps > XVEC_MAX_TAPS) return set_error(XVEC_E_ARG, "taps must be in [1,%d]", XVEC_MAX_TAPS);
+  *l = XvecLayerDesc{};
+  l->w_packed_dev = w_packed;
+  l->bias_dev = bias;
+  l->n = n;
+  l->cin = cin;
+  l->taps = taps;
+  l->dtype = dtype;
+  for (int j = 0; j < taps; ++j) l->tap_offsets[j] = tap_offsets[j];
+  return XVEC_OK;
+}
+
 }  // namespace xvec
 
 using namespace xvec;
@@ -103,7 +117,7 @@ void xvec_watchdog_reset(void) {
 int xvec_debug_trace(long long* out_host, int n) { return read_trace(out_host, n); }
 
 int64_t xvec_packed_k(int cin, int taps, int dtype) {
-  const int kc = dtype == XVEC_BF16 ? 64 : 32;
+  const int kc = chunk_elems(dtype);
   return static_cast<int64_t>(taps) * ((cin + kc - 1) / kc) * kc;
 }
 int64_t xvec_splitk_workspace_bytes(int64_t rows, int cin, int taps, int n, int dtype) {
@@ -116,18 +130,20 @@ int xvec_tdnn_layer(const void* x_dev, int x_dtype, int64_t x_rows, int cin, int
                     const int32_t* tap_offsets_host, int taps, const float* bias_dev, const float* bn_scale_dev,
                     const float* bn_shift_dev, int relu, void* y_dev, int y_dtype, int64_t y_ld, int64_t rows, void* splitk_ws_dev,
                     int64_t splitk_ws_bytes, void* stream) {
-  if (!tap_offsets_host) return set_error(XVEC_E_ARG, "tap_offsets_host is NULL");
-  return gemm_dispatch(x_dev, x_dtype, x_rows, cin, x_ld, w_packed_dev, n, tap_offsets_host, taps, bias_dev, bn_scale_dev,
-                       bn_shift_dev, relu, y_dev, y_dtype, y_ld, nullptr, nullptr, nullptr, rows, false, splitk_ws_dev, splitk_ws_bytes,
-                       stream);
+  XvecLayerDesc l;
+  const int rc = layer_desc(&l, w_packed_dev, bias_dev, n, cin, taps, x_dtype, tap_offsets_host);
+  if (rc) return rc;
+  return gemm_store(l, x_dev, x_rows, x_ld, rows, bn_scale_dev, bn_shift_dev, relu, y_dev, y_dtype, y_ld, splitk_ws_dev, splitk_ws_bytes,
+                    stream);
 }
 
 int xvec_tdnn_pool_fused(const void* x_dev, int x_dtype, int64_t x_rows, int cin, int64_t x_ld, const void* w_packed_dev, int n,
                          const int32_t* tap_offsets_host, int taps, const float* bias_dev, const int32_t* row_utt_dev,
                          const int32_t* blk_slot_base_dev, float* part_dev, int64_t rows, void* stream) {
-  if (!tap_offsets_host) return set_error(XVEC_E_ARG, "tap_offsets_host is NULL");
-  return gemm_dispatch(x_dev, x_dtype, x_rows, cin, x_ld, w_packed_dev, n, tap_offsets_host, taps, bias_dev, nullptr, nullptr, 1,
-                       nullptr, XVEC_F32, 0, row_utt_dev, blk_slot_base_dev, part_dev, rows, true, nullptr, 0, stream);
+  XvecLayerDesc l;
+  const int rc = layer_desc(&l, w_packed_dev, bias_dev, n, cin, taps, x_dtype, tap_offsets_host);
+  if (rc) return rc;
+  return gemm_pool(l, x_dev, x_rows, x_ld, rows, row_utt_dev, blk_slot_base_dev, part_dev, stream);
 }
 
 int64_t xvec_stack_ctrl_bytes(int64_t rows, int n_tdnn) { return stack_ctrl_bytes(rows, n_tdnn); }
@@ -149,67 +165,69 @@ int xvec_tdnn_stack(const XvecLayerDesc* tdnn, int n_tdnn, const void* x_dev, in
                         ctrl_bytes, band, stream);
 }
 
+// Frame-level stack of xvec_extract_forward: the persistent stack kernel when given its scratch and the stack fits it, else one
+// launch per layer.
+static int frame_stack(const XvecLayerDesc* tdnn, int n_tdnn, const void* x, int64_t rows, int64_t x_ld, void* act0, void* act1,
+                       int64_t act_ld, const int32_t* row_utt, const int32_t* blk_slot_base, float* part, void* ctrl, int64_t ctrl_bytes,
+                       void* stream) {
+  if (ctrl && stack_supported(tdnn, n_tdnn, rows))
+    return stack_dispatch(tdnn, n_tdnn, x, rows, x_ld, act0, act1, act_ld, row_utt, blk_slot_base, part, ctrl, ctrl_bytes, 0, stream);
+  void* act[2] = {act0, act1};
+  const void* h = x;
+  int64_t h_ld = x_ld;
+  for (int i = 0; i + 1 < n_tdnn; ++i) {
+    const int rc = gemm_store(tdnn[i], h, rows, h_ld, rows, nullptr, nullptr, 1, act[i & 1], tdnn[i + 1].dtype, act_ld, nullptr, 0, stream);
+    if (rc) return rc;
+    h = act[i & 1];
+    h_ld = act_ld;
+  }
+  return gemm_pool(tdnn[n_tdnn - 1], h, rows, h_ld, rows, row_utt, blk_slot_base, part, stream);
+}
+
+// Segment head of xvec_extract_forward: n_fc layers on the pooled statistics `a`, ReLU between them, none after the last.
+static int segment_head(const XvecLayerDesc* fc, int n_fc, const void* a, int64_t a_ld, int n_utts, void* fc_tmp, void* splitk_ws,
+                        int64_t splitk_ws_bytes, float* out, int64_t out_ld, void* stream) {
+  for (int i = 0; i < n_fc; ++i) {
+    const XvecLayerDesc& l = fc[i];
+    const bool final_layer = i == n_fc - 1;
+    void* y = final_layer ? static_cast<void*>(out) : fc_tmp;
+    const int y_dtype = final_layer ? XVEC_F32 : fc[i + 1].dtype;
+    const int64_t y_ld = final_layer ? out_ld : l.n;
+    const int relu = final_layer ? 0 : 1;
+    int rc;
+    if (l.w_plain_dev && fc_small_supported(n_utts, l.cin, l.n, a_ld, l.cin, a, l.w_plain_dev, l.dtype))
+      // small-footprint kernel: runs next to the resident stack CTAs of the next batch instead of waiting for free SMs
+      rc = fc_small_dispatch(a, l.dtype, n_utts, l.cin, a_ld, l.w_plain_dev, l.n, l.cin, l.bias_dev, relu, y, y_dtype, y_ld, stream);
+    else
+      rc = gemm_store(l, a, n_utts, a_ld, n_utts, nullptr, nullptr, relu, y, y_dtype, y_ld, splitk_ws, splitk_ws_bytes, stream);
+    if (rc) return rc;
+    a = y;
+    a_ld = y_ld;
+  }
+  return XVEC_OK;
+}
+
 int xvec_extract_forward(const XvecLayerDesc* tdnn, int n_tdnn, const void* x_dev, int64_t rows, int64_t x_ld, void* act0_dev,
                          void* act1_dev, int64_t act_ld, const int32_t* row_utt_dev, const int32_t* blk_slot_base_dev,
                          const int32_t* utt_slot_start_dev, const int32_t* n_pool_dev, int n_utts, float* part_dev,
                          const float* bn_last_scale_dev, const float* bn_last_shift_dev, float* pooled_dev, void* pooled_lp_dev,
                          const XvecLayerDesc* fc, int n_fc, void* fc_tmp_dev, void* splitk_ws_dev, int64_t splitk_ws_bytes,
                          float* out_dev, int64_t out_ld, void* ctrl_dev, int64_t ctrl_bytes, void* stream) {
-  if (!tdnn || n_tdnn < 2 || !fc || n_fc < 1 || n_fc > 2) return set_error(XVEC_E_ARG, "need >= 2 TDNN layers and 1 or 2 segment layers");
-  if (!x_dev || !act0_dev || !act1_dev || !pooled_dev || !out_dev) return set_error(XVEC_E_ARG, "null pointer argument");
+  if (!tdnn || n_tdnn < 2 || n_fc < 0 || n_fc > 2 || (n_fc > 0 && !fc))
+    return set_error(XVEC_E_ARG, "need >= 2 TDNN layers and 0 to 2 segment layers");
+  if (!x_dev || !act0_dev || !act1_dev || !pooled_dev || (n_fc > 0 && !out_dev)) return set_error(XVEC_E_ARG, "null pointer argument");
   if (n_fc == 2 && !fc_tmp_dev) return set_error(XVEC_E_ARG, "fc_tmp_dev is NULL");
-  const XvecLayerDesc& last = tdnn[n_tdnn - 1];
-  int rc;
-  if (ctrl_dev && stack_supported(tdnn, n_tdnn, rows)) {
-    rc = stack_dispatch(tdnn, n_tdnn, x_dev, rows, x_ld, act0_dev, act1_dev, act_ld, row_utt_dev, blk_slot_base_dev, part_dev, ctrl_dev,
-                        ctrl_bytes, 0, stream);
-    if (rc) return rc;
-  } else {
-    void* act[2] = {act0_dev, act1_dev};
-    const void* h = x_dev;
-    int64_t h_ld = x_ld;
-    for (int i = 0; i + 1 < n_tdnn; ++i) {
-      const XvecLayerDesc& l = tdnn[i];
-      const int out_dtype = tdnn[i + 1].dtype;
-      rc = gemm_dispatch(h, l.dtype, rows, l.cin, h_ld, l.w_packed_dev, l.n, l.tap_offsets, l.taps, l.bias_dev, nullptr, nullptr, 1,
-                         act[i & 1], out_dtype, act_ld, nullptr, nullptr, nullptr, rows, false, nullptr, 0, stream);
-      if (rc) return rc;
-      h = act[i & 1];
-      h_ld = act_ld;
-    }
-    rc = gemm_dispatch(h, last.dtype, rows, last.cin, h_ld, last.w_packed_dev, last.n, last.tap_offsets, last.taps, last.bias_dev, nullptr,
-                       nullptr, 1, nullptr, XVEC_F32, 0, row_utt_dev, blk_slot_base_dev, part_dev, rows, true, nullptr, 0, stream);
-    if (rc) return rc;
-  }
-  const int fc_in_dtype = fc[0].dtype;
-  if (fc_in_dtype == XVEC_BF16 && !pooled_lp_dev) return set_error(XVEC_E_ARG, "pooled_lp_dev is required for bf16 segment layers");
-  rc = xvec_pool_finalize(part_dev, utt_slot_start_dev, n_pool_dev, n_utts, last.n, bn_last_scale_dev, bn_last_shift_dev, nullptr, pooled_dev,
-                          fc_in_dtype == XVEC_BF16 ? pooled_lp_dev : nullptr, XVEC_BF16, 2 * static_cast<int64_t>(last.n), stream);
+  const bool lp_head = n_fc > 0 && fc[0].dtype == XVEC_BF16;
+  if (lp_head && !pooled_lp_dev) return set_error(XVEC_E_ARG, "pooled_lp_dev is required for bf16 segment layers");
+  int rc = frame_stack(tdnn, n_tdnn, x_dev, rows, x_ld, act0_dev, act1_dev, act_ld, row_utt_dev, blk_slot_base_dev, part_dev, ctrl_dev,
+                       ctrl_bytes, stream);
   if (rc) return rc;
-  const void* a = fc_in_dtype == XVEC_BF16 ? pooled_lp_dev : static_cast<const void*>(pooled_dev);
-  int64_t a_ld = 2 * static_cast<int64_t>(last.n);
-  for (int i = 0; i < n_fc; ++i) {
-    const bool final_layer = i == n_fc - 1;
-    void* y = final_layer ? static_cast<void*>(out_dev) : fc_tmp_dev;
-    const int y_dtype = final_layer ? XVEC_F32 : fc[i + 1].dtype;
-    const int64_t y_ld = final_layer ? out_ld : fc[i].n;
-    if (fc[i].w_plain_dev && fc_small_supported(n_utts, fc[i].cin, fc[i].n, a_ld, fc[i].cin, a, fc[i].w_plain_dev, fc[i].dtype)) {
-      // small-footprint kernel: runs next to the resident stack CTAs of the next batch instead of waiting for free SMs
-      rc = fc_small_dispatch(a, fc[i].dtype, n_utts, fc[i].cin, a_ld, fc[i].w_plain_dev, fc[i].n, fc[i].cin, fc[i].bias_dev,
-                             final_layer ? 0 : 1, y, y_dtype, y_ld, stream);
-      if (rc) return rc;
-      a = y;
-      a_ld = y_ld;
-      continue;
-    }
-    rc = gemm_dispatch(a, fc[i].dtype, n_utts, fc[i].cin, a_ld, fc[i].w_packed_dev, fc[i].n, fc[i].tap_offsets, 1, fc[i].bias_dev, nullptr,
-                       nullptr, final_layer ? 0 : 1, y, y_dtype, y_ld, nullptr, nullptr, nullptr, n_utts, false, splitk_ws_dev,
-                       splitk_ws_bytes, stream);
-    if (rc) return rc;
-    a = y;
-    a_ld = y_ld;
-  }
-  return XVEC_OK;
+  const int64_t pooled_ld = 2 * static_cast<int64_t>(tdnn[n_tdnn - 1].n);
+  rc = xvec_pool_finalize(part_dev, utt_slot_start_dev, n_pool_dev, n_utts, tdnn[n_tdnn - 1].n, bn_last_scale_dev, bn_last_shift_dev, nullptr,
+                          pooled_dev, pooled_lp_dev, XVEC_BF16, pooled_ld, stream);
+  if (rc) return rc;
+  return segment_head(fc, n_fc, lp_head ? pooled_lp_dev : static_cast<const void*>(pooled_dev), pooled_ld, n_utts, fc_tmp_dev, splitk_ws_dev,
+                      splitk_ws_bytes, out_dev, out_ld, stream);
 }
 
 }  // extern "C"

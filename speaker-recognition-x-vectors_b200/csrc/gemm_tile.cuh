@@ -181,6 +181,52 @@ inline int make_tmap_2d(CUtensorMap* map, const void* ptr, int dtype, uint64_t i
   return XVEC_OK;
 }
 
+// Rows of an input matrix its tensor map covers.  Window form (x_ld < cin: overlapping rows): only rows whose whole window lies
+// inside the matrix exist, the rest read as zero.  Returns XVEC_E_ARG (negative) when there is not even one window.
+inline int64_t window_rows(int64_t x_rows, int cin, int64_t x_ld) {
+  const int64_t rows = x_ld < cin ? x_rows - (cin + x_ld - 1) / x_ld + 1 : x_rows;
+  return rows > 0 ? rows : set_error(XVEC_E_ARG, "window form: fewer rows than one window");
+}
+
+// Packed weights of layer `l` are chunk-major (xvec_pack_weight): a (kblocks * n_pad) x chunk matrix, so the box a CTA loads per
+// K chunk (half of the 256-row weight tile x 128 bytes) is one contiguous 16 KiB run.
+inline int make_weight_tmap(CUtensorMap* map, const XvecLayerDesc& l) {
+  const int bke = chunk_elems(l.dtype);
+  const uint64_t kblocks = static_cast<uint64_t>(l.taps) * ((l.cin + bke - 1) / bke);
+  const uint64_t n_pad = static_cast<uint64_t>((l.n + BN - 1) / BN) * BN;
+  return make_tmap_2d(map, l.w_packed_dev, l.dtype, bke, kblocks * n_pad, bke, bke, BN_CTA);
+}
+
+// Launches kKernel as clusters of 2 CTAs (one tcgen05 CTA pair each).  The first launch on a device raises the kernel's dynamic
+// shared-memory limit (once per kernel) and binds the watchdog word of the kernel's translation unit (bind_watchdog).
+template <auto kKernel, class... Args>
+inline int launch_pair(const char* name, int threads, int smem, int grid, int (*bind_watchdog)(), cudaStream_t st, const Args&... args) {
+  static PerDeviceInit configured;  // per kernel
+  int rc = once_per_device(configured, [smem] {
+    cudaError_t e = cudaFuncSetAttribute(kKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    if (e != cudaSuccess) return set_error(XVEC_E_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+    return static_cast<int>(XVEC_OK);
+  });
+  if (rc) return rc;
+  rc = bind_watchdog();
+  if (rc) return rc;
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = dim3(grid);
+  cfg.blockDim = dim3(threads);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = st;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = 2;
+  attr[0].val.clusterDim.y = 1;
+  attr[0].val.clusterDim.z = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  cudaError_t e = cudaLaunchKernelEx(&cfg, kKernel, args...);
+  if (e != cudaSuccess) return set_error(XVEC_E_CUDA, "%s launch: %s", name, cudaGetErrorString(e));
+  return XVEC_OK;
+}
+
 // L2 eviction hints of the TMA traffic: activations in (evict-first), weights (evict-last), activations out (evict-last).
 // Debug builds: XVEC_L2HINT = three digits (0 normal, 1 evict-first, 2 evict-last) overrides the default.
 inline void l2_policies(unsigned long long* pol_a, unsigned long long* pol_b, unsigned long long* pol_y) {

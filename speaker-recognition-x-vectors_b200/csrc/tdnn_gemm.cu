@@ -415,33 +415,15 @@ splitk_reduce_kernel(const float* __restrict__ ws, int ksplit, int rows, int row
 // ------------------------------------------------------------------------------------------------ host side
 static long long* g_trace_buf = nullptr;
 
-template <bool kTf32, int kEpi>
-static int launch(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& ty, const GemmParams& p, int grid, cudaStream_t st) {
-  static PerDeviceInit configured;  // per instantiation
+// Persistent grid: one CTA pair per tile, at most one pair per two SMs.
+template <int kEpi>
+static int launch(bool tf32, const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& ty, const GemmParams& p, cudaStream_t st) {
+  const int64_t tiles = static_cast<int64_t>(p.m_tiles) * p.n_tiles * p.ksplit;
+  const int max_pairs = num_sms() / 2;
+  const int grid = 2 * static_cast<int>(tiles < max_pairs ? tiles : max_pairs);
   constexpr int smem = gemm_smem_bytes<kEpi>();
-  int rc = once_per_device(configured, [] {
-    cudaError_t e = cudaFuncSetAttribute(tdnn_gemm_kernel<kTf32, kEpi>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    if (e != cudaSuccess) return set_error(XVEC_E_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    return static_cast<int>(XVEC_OK);
-  });
-  if (rc) return rc;
-  rc = bind_watchdog_gemm();
-  if (rc) return rc;
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(GEMM_THREADS);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, tdnn_gemm_kernel<kTf32, kEpi>, ta, tb, ty, p);
-  if (e != cudaSuccess) return set_error(XVEC_E_CUDA, "tdnn_gemm_kernel launch: %s", cudaGetErrorString(e));
-  return XVEC_OK;
+  if (tf32) return launch_pair<tdnn_gemm_kernel<true, kEpi>>("tdnn_gemm_kernel", GEMM_THREADS, smem, grid, bind_watchdog_gemm, st, ta, tb, ty, p);
+  return launch_pair<tdnn_gemm_kernel<false, kEpi>>("tdnn_gemm_kernel", GEMM_THREADS, smem, grid, bind_watchdog_gemm, st, ta, tb, ty, p);
 }
 
 // Split-K plan for GEMMs with too few output tiles to fill the machine (segment6/7: a few hundred rows, K = 3000).
@@ -459,7 +441,7 @@ static void splitk_plan(int64_t rows, int n, int kblocks, int* ksplit, int* kb_p
 }
 
 int64_t splitk_workspace_bytes(int64_t rows, int cin, int taps, int n, int dtype) {
-  const int bke = dtype == XVEC_F32 ? 32 : 64;
+  const int bke = chunk_elems(dtype);
   int ksplit, kbs;
   splitk_plan(rows, n, taps * ((cin + bke - 1) / bke), &ksplit, &kbs);
   if (ksplit <= 1) return 0;
@@ -467,70 +449,34 @@ int64_t splitk_workspace_bytes(int64_t rows, int cin, int taps, int n, int dtype
   return static_cast<int64_t>(ksplit) * rows_pad * ((n + BN - 1) / BN * BN) * 4;
 }
 
-int gemm_dispatch(const void* x, int x_dtype, int64_t x_rows, int cin, int64_t x_ld, const void* w_packed, int n,
-                  const int32_t* tap_offsets, int taps, const float* bias, const float* scale, const float* shift, int relu,
-                  void* y, int y_dtype, int64_t y_ld, const int32_t* row_utt, const int32_t* blk_slot_base, float* part,
-                  int64_t rows, bool pool, void* ws, int64_t ws_bytes, void* stream) {
+// What both epilogues share: the checks of the layer and its input, the kernel parameters of the whole K loop with the bias and
+// no other epilogue operand, and the tensor maps of the input (ta) and the packed weights (tb).  ty is a placeholder until an
+// epilogue stores through TMA.
+static int gemm_setup(const XvecLayerDesc& l, const void* x, int64_t x_rows, int64_t x_ld, int64_t rows, GemmParams& p, CUtensorMap& ta,
+                      CUtensorMap& tb, CUtensorMap& ty) {
   int rc = device_check();
   if (rc) return rc;
-  if (!x || !w_packed || (!pool && !y) || (pool && (!row_utt || !blk_slot_base || !part)))
-    return set_error(XVEC_E_ARG, "null pointer argument");
-  if (x_dtype != XVEC_F32 && x_dtype != XVEC_BF16) return set_error(XVEC_E_ARG, "bad x_dtype %d", x_dtype);
-  if (!pool && y_dtype != XVEC_F32 && y_dtype != XVEC_BF16) return set_error(XVEC_E_ARG, "bad y_dtype %d", y_dtype);
-  if (taps < 1 || taps > XVEC_MAX_TAPS) return set_error(XVEC_E_ARG, "taps must be in [1,%d]", XVEC_MAX_TAPS);
-  if (rows <= 0 || x_rows <= 0 || cin <= 0 || n <= 0) return set_error(XVEC_E_ARG, "non-positive size");
+  if (!x || !l.w_packed_dev) return set_error(XVEC_E_ARG, "null pointer argument");
+  if (l.dtype != XVEC_F32 && l.dtype != XVEC_BF16) return set_error(XVEC_E_ARG, "bad x_dtype %d", l.dtype);
+  if (l.taps < 1 || l.taps > XVEC_MAX_TAPS) return set_error(XVEC_E_ARG, "taps must be in [1,%d]", XVEC_MAX_TAPS);
+  if (rows <= 0 || x_rows <= 0 || l.cin <= 0 || l.n <= 0) return set_error(XVEC_E_ARG, "non-positive size");
   if (rows > 0x7fffff00LL || x_rows > 0x7fffff00LL) return set_error(XVEC_E_ARG, "too many rows");
-  if ((scale == nullptr) != (shift == nullptr)) return set_error(XVEC_E_ARG, "bn_scale and bn_shift must be given together");
-  const bool tf32 = x_dtype == XVEC_F32;
-  const int bke = tf32 ? 32 : 64;
-  GemmParams p{};
+  const int bke = chunk_elems(l.dtype);
+  p = GemmParams{};
   p.rows = static_cast<int>(rows);
-  p.n = n;
+  p.n = l.n;
   p.m_tiles = static_cast<int>((rows + BM - 1) / BM);
-  p.n_tiles = (n + BN - 1) / BN;
-  p.taps = taps;
-  p.cpt = (cin + bke - 1) / bke;
-  for (int j = 0; j < taps; ++j) {
-    if (tap_offsets[j] < 0) return set_error(XVEC_E_ARG, "tap offsets must be non-negative");
-    p.tap_off[j] = tap_offsets[j];
+  p.n_tiles = (l.n + BN - 1) / BN;
+  p.taps = l.taps;
+  p.cpt = (l.cin + bke - 1) / bke;
+  for (int j = 0; j < l.taps; ++j) {
+    if (l.tap_offsets[j] < 0) return set_error(XVEC_E_ARG, "tap offsets must be non-negative");
+    p.tap_off[j] = l.tap_offsets[j];
   }
-  if (!pool && ((reinterpret_cast<uintptr_t>(bias) & 15u) || (reinterpret_cast<uintptr_t>(scale) & 15u) || (reinterpret_cast<uintptr_t>(shift) & 15u)))
-    return set_error(XVEC_E_ARG, "bias / bn_scale / bn_shift must be 16-byte aligned (and hold ceil(n/32)*32 floats)");
-  p.bias = bias;
-  p.scale = scale;
-  p.shift = shift;
-  p.relu = relu;
-  p.out = y;
-  p.ldo = y_ld;
-  const int64_t yes = y_dtype == XVEC_BF16 ? 2 : 4;
-  p.vec_store = (!pool && (reinterpret_cast<uintptr_t>(y) & 15u) == 0 && (y_ld * yes) % 16 == 0) ? 1 : 0;
-  if (!pool && y_ld < n) return set_error(XVEC_E_ARG, "y_ld < n");
-  p.row_utt = row_utt;
-  p.blk_slot_base = blk_slot_base;
-  p.part = part;
+  p.bias = l.bias_dev;
   p.ksplit = 1;
-  p.kb_per_split = taps * p.cpt;
+  p.kb_per_split = l.taps * p.cpt;
   p.rows_pad = p.m_tiles * BM;
-  // split-K: partial sums go to the caller's workspace, a second pass applies the epilogue
-  const int64_t ws_need = pool ? 0 : splitk_workspace_bytes(rows, cin, taps, n, x_dtype);
-  const bool split = ws_need > 0 && ws != nullptr && ws_bytes >= ws_need && (reinterpret_cast<uintptr_t>(ws) & 15u) == 0;
-  const int ws_ld = p.n_tiles * BN;
-  void* final_y = y;
-  const int final_dtype = y_dtype;
-  const int64_t final_ld = y_ld;
-  if (split) {
-    splitk_plan(rows, n, taps * p.cpt, &p.ksplit, &p.kb_per_split);
-    p.bias = nullptr;
-    p.scale = nullptr;
-    p.shift = nullptr;
-    p.relu = 0;
-    p.out = ws;
-    p.ldo = ws_ld;
-    p.vec_store = 1;
-    y = ws;
-    y_dtype = XVEC_F32;
-    y_ld = ws_ld;
-  }
   l2_policies(&p.pol_a, &p.pol_b, &p.pol_y);
 #ifdef XVEC_DEBUG
   {  // developer instrumentation (XVEC_DBG epilogue/mainloop skip switches, XVEC_TRACE per-tile clock stamps): debug builds only
@@ -546,41 +492,76 @@ int gemm_dispatch(const void* x, int x_dtype, int64_t x_rows, int cin, int64_t x
     g_trace_buf = trace_buf;
   }
 #endif
+  const int64_t a_rows = window_rows(x_rows, l.cin, x_ld);
+  if (a_rows < 0) return static_cast<int>(a_rows);
+  rc = make_tmap_2d(&ta, x, l.dtype, static_cast<uint64_t>(l.cin), static_cast<uint64_t>(a_rows), static_cast<uint64_t>(x_ld), bke, BM_CTA);
+  if (rc) return rc;
+  ty = ta;
+  return make_weight_tmap(&tb, l);
+}
 
+// Destination of a store epilogue: y_rows x n of y_dtype, row stride y_ld.  16-byte aligned rows are staged in swizzled shared
+// memory and TMA-stored through ty; other rows are stored element by element.
+static int set_store_output(GemmParams& p, CUtensorMap& ty, void* y, int y_dtype, int64_t y_ld, int64_t y_rows) {
+  const int64_t es = y_dtype == XVEC_BF16 ? 2 : 4;
+  p.out = y;
+  p.ldo = y_ld;
+  p.vec_store = ((reinterpret_cast<uintptr_t>(y) & 15u) == 0 && (y_ld * es) % 16 == 0) ? 1 : 0;
+  if (!p.vec_store) return XVEC_OK;
+  return make_tmap_2d(&ty, y, y_dtype, static_cast<uint64_t>(p.n), static_cast<uint64_t>(y_rows), static_cast<uint64_t>(y_ld),
+                      static_cast<uint32_t>(128 / es), 32);
+}
+
+int gemm_pool(const XvecLayerDesc& l, const void* x, int64_t x_rows, int64_t x_ld, int64_t rows, const int32_t* row_utt,
+              const int32_t* blk_slot_base, float* part, void* stream) {
+  GemmParams p;
   CUtensorMap ta, tb, ty;
-  // window form (x_ld < cin: overlapping rows): only rows whose whole window lies inside the matrix exist, the rest read as zero
-  const int64_t a_rows = x_ld < cin ? x_rows - (cin + x_ld - 1) / x_ld + 1 : x_rows;
-  if (a_rows <= 0) return set_error(XVEC_E_ARG, "window form: fewer rows than one window");
-  rc = make_tmap_2d(&ta, x, x_dtype, static_cast<uint64_t>(cin), static_cast<uint64_t>(a_rows), static_cast<uint64_t>(x_ld), bke, BM_CTA);
+  int rc = gemm_setup(l, x, x_rows, x_ld, rows, p, ta, tb, ty);
   if (rc) return rc;
-  // packed weights are chunk-major (xvec_pack_weight): a (kblocks * n_pad) x bke matrix, one contiguous 16 KiB box per load
-  rc = make_tmap_2d(&tb, w_packed, x_dtype, bke, static_cast<uint64_t>(taps) * p.cpt * p.n_tiles * BN, bke, bke, BN_CTA);
-  if (rc) return rc;
-  if (p.vec_store) {
-    const uint64_t yrows = split ? static_cast<uint64_t>(p.ksplit) * p.rows_pad : static_cast<uint64_t>(rows);
-    rc = make_tmap_2d(&ty, y, y_dtype, static_cast<uint64_t>(n), yrows, static_cast<uint64_t>(y_ld),
-                      static_cast<uint32_t>(128 / (y_dtype == XVEC_BF16 ? 2 : 4)), 32);
-    if (rc) return rc;
-  } else {
-    ty = ta;  // unused by the kernel
-  }
+  if (!row_utt || !blk_slot_base || !part) return set_error(XVEC_E_ARG, "null pointer argument");
+  p.row_utt = row_utt;
+  p.blk_slot_base = blk_slot_base;
+  p.part = part;
+  return launch<EPI_POOL>(l.dtype == XVEC_F32, ta, tb, ty, p, static_cast<cudaStream_t>(stream));
+}
 
-  const int64_t tiles = static_cast<int64_t>(p.m_tiles) * p.n_tiles * p.ksplit;
-  const int max_pairs = num_sms() / 2;
-  const int pairs = static_cast<int>(tiles < max_pairs ? tiles : max_pairs);
-  const int grid = 2 * pairs;
+int gemm_store(const XvecLayerDesc& l, const void* x, int64_t x_rows, int64_t x_ld, int64_t rows, const float* bn_scale,
+               const float* bn_shift, int relu, void* y, int y_dtype, int64_t y_ld, void* ws, int64_t ws_bytes, void* stream) {
+  GemmParams p;
+  CUtensorMap ta, tb, ty;
+  int rc = gemm_setup(l, x, x_rows, x_ld, rows, p, ta, tb, ty);
+  if (rc) return rc;
+  if (!y) return set_error(XVEC_E_ARG, "null pointer argument");
+  if (y_dtype != XVEC_F32 && y_dtype != XVEC_BF16) return set_error(XVEC_E_ARG, "bad y_dtype %d", y_dtype);
+  if ((bn_scale == nullptr) != (bn_shift == nullptr)) return set_error(XVEC_E_ARG, "bn_scale and bn_shift must be given together");
+  if ((reinterpret_cast<uintptr_t>(l.bias_dev) & 15u) || (reinterpret_cast<uintptr_t>(bn_scale) & 15u) || (reinterpret_cast<uintptr_t>(bn_shift) & 15u))
+    return set_error(XVEC_E_ARG, "bias / bn_scale / bn_shift must be 16-byte aligned (and hold ceil(n/32)*32 floats)");
+  if (y_ld < l.n) return set_error(XVEC_E_ARG, "y_ld < n");
+  const bool tf32 = l.dtype == XVEC_F32;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (pool) return tf32 ? launch<true, EPI_POOL>(ta, tb, ty, p, grid, st) : launch<false, EPI_POOL>(ta, tb, ty, p, grid, st);
-  if (y_dtype == XVEC_BF16)
-    return tf32 ? launch<true, EPI_STORE_BF16>(ta, tb, ty, p, grid, st) : launch<false, EPI_STORE_BF16>(ta, tb, ty, p, grid, st);
-  rc = tf32 ? launch<true, EPI_STORE_F32>(ta, tb, ty, p, grid, st) : launch<false, EPI_STORE_F32>(ta, tb, ty, p, grid, st);
-  if (rc || !split) return rc;
-  const long long total = rows * static_cast<long long>(n);
+  const int64_t ws_need = splitk_workspace_bytes(rows, l.cin, l.taps, l.n, l.dtype);
+  if (ws_need == 0 || !ws || ws_bytes < ws_need || (reinterpret_cast<uintptr_t>(ws) & 15u)) {
+    p.scale = bn_scale;
+    p.shift = bn_shift;
+    p.relu = relu;
+    rc = set_store_output(p, ty, y, y_dtype, y_ld, rows);
+    if (rc) return rc;
+    return y_dtype == XVEC_BF16 ? launch<EPI_STORE_BF16>(tf32, ta, tb, ty, p, st) : launch<EPI_STORE_F32>(tf32, ta, tb, ty, p, st);
+  }
+  // split-K, step 1: a GEMM with no epilogue; split s of the K loop writes the sums of output row r to workspace row s * rows_pad + r
+  splitk_plan(rows, l.n, l.taps * p.cpt, &p.ksplit, &p.kb_per_split);
+  p.bias = nullptr;
+  const int ws_ld = p.n_tiles * BN;
+  rc = set_store_output(p, ty, ws, XVEC_F32, ws_ld, static_cast<int64_t>(p.ksplit) * p.rows_pad);
+  if (rc) return rc;
+  rc = launch<EPI_STORE_F32>(tf32, ta, tb, ty, p, st);
+  if (rc) return rc;
+  // step 2: the splits summed in fixed order (deterministic), then the caller's epilogue into y
+  const long long total = rows * static_cast<long long>(l.n);
   long long blocks = (total + 255) / 256;
   if (blocks > num_sms() * 8LL) blocks = num_sms() * 8LL;
-  splitk_reduce_kernel<<<static_cast<unsigned>(blocks), 256, 0, st>>>(static_cast<const float*>(ws), p.ksplit, static_cast<int>(rows), p.rows_pad, n,
-                                                                    ws_ld, bias, scale, shift, relu, final_y, final_dtype == XVEC_BF16 ? 1 : 0,
-                                                                    final_ld);
+  splitk_reduce_kernel<<<static_cast<unsigned>(blocks), 256, 0, st>>>(static_cast<const float*>(ws), p.ksplit, p.rows, p.rows_pad, l.n, ws_ld,
+                                                                    l.bias_dev, bn_scale, bn_shift, relu, y, y_dtype == XVEC_BF16 ? 1 : 0, y_ld);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return set_error(XVEC_E_CUDA, "splitk_reduce_kernel launch: %s", cudaGetErrorString(e));
   return XVEC_OK;

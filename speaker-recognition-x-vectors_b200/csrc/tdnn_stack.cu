@@ -826,35 +826,6 @@ int64_t stack_ctrl_bytes(int64_t rows, int n_layers) {
 
 XVEC_DEFINE_WATCHDOG_BINDER(bind_watchdog_stack)
 
-template <bool kAllTf32>
-static int launch_stack(const StackMaps& maps, const StackParams& p, int grid, cudaStream_t st) {
-  static PerDeviceInit configured;  // per instantiation
-  constexpr int smem = stack_smem_bytes<kAllTf32>();
-  int rc = once_per_device(configured, [] {
-    cudaError_t e = cudaFuncSetAttribute(tdnn_stack_kernel<kAllTf32>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    if (e != cudaSuccess) return set_error(XVEC_E_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    return static_cast<int>(XVEC_OK);
-  });
-  if (rc) return rc;
-  rc = bind_watchdog_stack();
-  if (rc) return rc;
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(STACK_THREADS);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, tdnn_stack_kernel<kAllTf32>, maps, p);
-  if (e != cudaSuccess) return set_error(XVEC_E_CUDA, "tdnn_stack_kernel launch: %s", cudaGetErrorString(e));
-  return XVEC_OK;
-}
-
 bool stack_supported(const XvecLayerDesc* tdnn, int n_tdnn, int64_t rows) {
   if (n_tdnn < 2 || n_tdnn > XVEC_MAX_STACK || rows <= 0 || rows > 0x7fffff00LL) return false;
   if (tdnn[0].dtype != XVEC_F32 && tdnn[0].dtype != XVEC_BF16) return false;
@@ -915,7 +886,7 @@ static int build_plan(StackPlan& pl, const XvecLayerDesc* tdnn, int n_tdnn, cons
   for (int l = 0; l < n_tdnn; ++l) {
     const XvecLayerDesc& d = tdnn[l];
     StackLayer& L = p.L[l];
-    const int bke = d.dtype == XVEC_F32 ? 32 : 64;
+    const int bke = chunk_elems(d.dtype);
     L.n = d.n;
     L.n_tiles = (d.n + BN - 1) / BN;
     L.taps = d.taps;
@@ -931,16 +902,13 @@ static int build_plan(StackPlan& pl, const XvecLayerDesc* tdnn, int n_tdnn, cons
     L.slab_rows = BM_CTA + max_off;
     L.bias = d.bias_dev;
     if (reinterpret_cast<uintptr_t>(d.bias_dev) & 15u) return set_error(XVEC_E_ARG, "bias must be 16-byte aligned");
-    // window form (h_ld < cin: overlapping rows): only rows whose whole window lies inside the matrix exist, the rest read as zero
-    const int64_t h_rows = h_ld < d.cin ? rows - (d.cin + h_ld - 1) / h_ld + 1 : rows;
-    if (h_rows <= 0) return set_error(XVEC_E_ARG, "window form: fewer rows than one window");
+    const int64_t h_rows = window_rows(rows, d.cin, h_ld);
+    if (h_rows < 0) return static_cast<int>(h_rows);
     rc = make_tmap_2d(&maps.a[l], h, h_dtype, static_cast<uint64_t>(d.cin), static_cast<uint64_t>(h_rows), static_cast<uint64_t>(h_ld),
                       bke, static_cast<uint32_t>(L.slab_rows));
     if (rc) return rc;
-    // packed weights are chunk-major (xvec_pack_weight): a (kblocks * n_pad) x bke matrix, one contiguous 16 KiB box per load
-    const uint64_t n_pad = static_cast<uint64_t>(L.n_tiles) * BN;
-    L.n_pad = static_cast<int>(n_pad);
-    rc = make_tmap_2d(&maps.b[l], d.w_packed_dev, d.dtype, bke, static_cast<uint64_t>(d.taps) * L.cpt * n_pad, bke, bke, BN_CTA);
+    L.n_pad = L.n_tiles * BN;
+    rc = make_weight_tmap(&maps.b[l], d);
     if (rc) return rc;
     if (l + 1 < n_tdnn) {
       // store boxes: 32 rows x 32 columns (64-byte rows / SWIZZLE_64B for bf16, 128-byte rows / SWIZZLE_128B for float32)
@@ -989,15 +957,9 @@ int stack_dispatch(const XvecLayerDesc* tdnn, int n_tdnn, const void* x, int64_t
   key.x = x;
   key.act0 = act0;
   key.act1 = act1;
-  for (int l = 0; l < n_tdnn; ++l) {
-    XvecLayerDesc& k = key.L[l];  // field by field: the caller's struct may carry garbage in unused tap slots
-    k.w_packed_dev = tdnn[l].w_packed_dev;
-    k.bias_dev = tdnn[l].bias_dev;
-    k.n = tdnn[l].n;
-    k.cin = tdnn[l].cin;
-    k.taps = tdnn[l].taps;
-    k.dtype = tdnn[l].dtype;
-    for (int j = 0; j < tdnn[l].taps; ++j) k.tap_offsets[j] = tdnn[l].tap_offsets[j];
+  for (int l = 0; l < n_tdnn; ++l) {  // without the garbage the caller's struct may carry in unused tap slots
+    rc = layer_desc(&key.L[l], tdnn[l].w_packed_dev, tdnn[l].bias_dev, tdnn[l].n, tdnn[l].cin, tdnn[l].taps, tdnn[l].dtype, tdnn[l].tap_offsets);
+    if (rc) return rc;
   }
   StackMaps maps;
   StackParams p;
@@ -1041,7 +1003,9 @@ int stack_dispatch(const XvecLayerDesc* tdnn, int n_tdnn, const void* x, int64_t
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   cudaError_t e = cudaMemsetAsync(ctrl, 0, static_cast<size_t>(stack_ctrl_bytes(rows, n_tdnn)), st);
   if (e != cudaSuccess) return set_error(XVEC_E_CUDA, "cudaMemsetAsync(ctrl): %s", cudaGetErrorString(e));
-  return all_tf32 ? launch_stack<true>(maps, p, grid, st) : launch_stack<false>(maps, p, grid, st);
+  if (all_tf32)
+    return launch_pair<tdnn_stack_kernel<true>>("tdnn_stack_kernel", STACK_THREADS, stack_smem_bytes<true>(), grid, bind_watchdog_stack, st, maps, p);
+  return launch_pair<tdnn_stack_kernel<false>>("tdnn_stack_kernel", STACK_THREADS, stack_smem_bytes<false>(), grid, bind_watchdog_stack, st, maps, p);
 }
 
 }  // namespace xvec

@@ -23,10 +23,17 @@ int num_sms();
 // Driver entry point for tensor-map creation, resolved through the runtime (no link-time libcuda dependency).
 PFN_encodeTiled get_encode_tiled();
 
-int gemm_dispatch(const void* x, int x_dtype, int64_t x_rows, int cin, int64_t x_ld, const void* w_packed, int n,
-                  const int32_t* tap_offsets, int taps, const float* bias, const float* scale, const float* shift, int relu,
-                  void* y, int y_dtype, int64_t y_ld, const int32_t* row_utt, const int32_t* blk_slot_base, float* part,
-                  int64_t rows, bool pool, void* ws, int64_t ws_bytes, void* stream);
+// Elements of `dtype` in one 128-byte K chunk of a packed operand: 32 float32 (TF32 math) or 64 bfloat16.
+inline int chunk_elems(int dtype) { return dtype == XVEC_F32 ? 32 : 64; }
+
+// `l` with the given operands and zeros everywhere else (tap slots past `taps`, w_plain_dev); XVEC_E_ARG for bad taps.
+int layer_desc(XvecLayerDesc* l, const void* w_packed, const float* bias, int n, int cin, int taps, int dtype, const int32_t* tap_offsets);
+// tdnn_gemm.cu: layer `l` as a tcgen05 GEMM over output rows [0, rows) of x ((x_rows, l.cin) of l.dtype, row stride x_ld).
+// gemm_store: as xvec_tdnn_layer (split-K over `ws` when that helps and ws is large enough); gemm_pool: as xvec_tdnn_pool_fused.
+int gemm_store(const XvecLayerDesc& l, const void* x, int64_t x_rows, int64_t x_ld, int64_t rows, const float* bn_scale,
+               const float* bn_shift, int relu, void* y, int y_dtype, int64_t y_ld, void* ws, int64_t ws_bytes, void* stream);
+int gemm_pool(const XvecLayerDesc& l, const void* x, int64_t x_rows, int64_t x_ld, int64_t rows, const int32_t* row_utt,
+              const int32_t* blk_slot_base, float* part, void* stream);
 // tdnn_stack.cu: all TDNN layers (the last one fused with the pooling partials) as one persistent kernel.
 bool stack_supported(const XvecLayerDesc* tdnn, int n_tdnn, int64_t rows);
 int64_t stack_ctrl_bytes(int64_t rows, int n_layers);

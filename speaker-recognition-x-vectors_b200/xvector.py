@@ -329,10 +329,10 @@ class XVectorModel(nn.Module):
         return x
 
     # ------------------------------------------------------------------ the hot path
-    def pooled_stats_flat(self, flat_x: torch.Tensor, lengths, slot: int = 0) -> "tuple[torch.Tensor, torch.Tensor | None]":
-        """TDNN stack + statistics pooling over a flat (rows, input_size) float32 frame matrix.
-        Returns (pooled float32 (U, 3000), same in the activation dtype or None).  The returned tensors are scratch of
-        the (lengths, slot) plan: they are overwritten by the next call with the same lengths and slot."""
+    def _extract_forward(self, flat_x: torch.Tensor, lengths, slot: int, head: bool, out: torch.Tensor | None = None):
+        """ONE C-ABI call (xvec_extract_forward) that enqueues the path on the current stream: the TDNN stack (the persistent
+        stack kernel, or one launch per layer for stacks it does not take) with the pooling partials, the pooling finalize into
+        the slot's scratch and, when `head`, the segment layer(s) into `out` (allocated when None).  Returns (layout, scratch, out)."""
         self._check_eval()
         if not flat_x.is_cuda:
             raise ValueError("xvec_b200 has no CPU path: move the input (and the model) to a CUDA device")
@@ -341,31 +341,36 @@ class XVectorModel(nn.Module):
         lay = self._layout_for(lengths)
         if lay.rows != flat_x.shape[0]:
             raise ValueError("sum(lengths) does not match the number of rows")
+        pipe = self._pipeline()
         sc = self._scratch_for(slot)
         sc.ensure(lay.rows, lay.n_slots, lay.n_utts)
         if flat_x.dtype != torch.float32:
             flat_x = flat_x.float()
-        pipe = self._pipeline()
-        last = self.time_context_layers[-1]
-        part = sc.part[: lay.n_slots]
-        pooled = sc.pooled[: lay.n_utts]
-        pooled_lp = None if sc.pooled_lp is None else sc.pooled_lp[: lay.n_utts]
         x = self._frames_for(flat_x, pipe)  # layer 1 always reads the float32 frames (TF32 math): no cast pass over the input
-        if self._stack_kernel_ok():
-            ops.tdnn_stack(pipe["tdnn"], pipe["n_tdnn"], x, sc.act[0], sc.act[1], lay.row_utt, lay.blk_slot_base, part, sc.ctrl)
-        else:  # layer widths the one-launch stack kernel does not take: one launch per layer
-            layers = list(self.time_context_layers)
-            stack = pipe["keep"][0]
-            h = x
-            for i, layer in enumerate(layers[:-1]):
-                w, bias, offs = stack[i]
-                h = ops.tdnn_layer_flat(h, w, layer.output_size, offs, bias, None, None, relu=True,
-                                        out=sc.act[i & 1][: lay.rows, : layer.output_size], cin=layer.input_size)
-            w, bias, offs = stack[-1]
-            ops.tdnn_pool_fused(h, w, last.output_size, offs, bias, lay.row_utt, lay.blk_slot_base, part)
-        ops.pool_finalize(part, lay.utt_slot_start, lay.n_pool, last.output_size, pipe["scale5"], pipe["shift5"], out=pooled, out_lp=pooled_lp)
-        return pooled, pooled_lp
+        fc, n_fc, fc_tmp, ws = None, 0, None, None
+        if head:
+            sc.ensure_head(lay.n_utts, pipe["fc_shapes"], pipe["hidden"])
+            fc, n_fc, fc_tmp, ws = pipe["fc"], pipe["n_fc"], sc.fc_tmp, sc.ws
+            if out is None:
+                out = torch.empty((lay.n_utts, pipe["out_dim"]), dtype=torch.float32, device=flat_x.device)
+            elif (out.dtype != torch.float32 or out.device != flat_x.device or out.shape != (lay.n_utts, pipe["out_dim"]) or out.stride(1) != 1):
+                raise ValueError(f"out must be a float32 ({lay.n_utts}, {pipe['out_dim']}) tensor on the input's device with unit column stride")
+        lib = _lib.load()
+        p = _lib.ptr
+        with _lib.on_device(flat_x.device):
+            _lib.check(lib.xvec_extract_forward(
+                pipe["tdnn"], pipe["n_tdnn"], p(x), lay.rows, x.stride(0), p(sc.act[0]), p(sc.act[1]), sc.ld, p(lay.row_utt),
+                p(lay.blk_slot_base), p(lay.utt_slot_start), p(lay.n_pool), lay.n_utts, p(sc.part), p(pipe["scale5"]), p(pipe["shift5"]),
+                p(sc.pooled), p(sc.pooled_lp), fc, n_fc, p(fc_tmp), p(ws), 0 if ws is None else ws.numel(),
+                p(out), 0 if out is None else out.stride(0), p(sc.ctrl), sc.ctrl.numel(), _lib.stream_ptr()))
+        return lay, sc, out
 
+    def pooled_stats_flat(self, flat_x: torch.Tensor, lengths, slot: int = 0) -> "tuple[torch.Tensor, torch.Tensor | None]":
+        """TDNN stack + statistics pooling over a flat (rows, input_size) float32 frame matrix.
+        Returns (pooled float32 (U, 3000), same in the activation dtype or None).  The returned tensors are scratch of
+        the (lengths, slot) plan: they are overwritten by the next call with the same lengths and slot."""
+        lay, sc, _ = self._extract_forward(flat_x, lengths, slot, head=False)
+        return sc.pooled[: lay.n_utts], None if sc.pooled_lp is None else sc.pooled_lp[: lay.n_utts]
 
     def _head(self, pooled, pooled_lp, layer) -> torch.Tensor:
         a = pooled if pooled_lp is None else pooled_lp
@@ -380,34 +385,7 @@ class XVectorModel(nn.Module):
         (len(lengths), x_vector_size), unit column stride) receives the x-vectors in place, e.g. a row range of a whole set's matrix.
         The whole path is ONE C-ABI call (xvec_extract_forward) that enqueues its kernels on the current stream: the
         persistent TDNN-stack kernel (all five layers + pooling partials), the pooling finalize and the segment layer(s)."""
-        self._check_eval()
-        if not flat_x.is_cuda:
-            raise ValueError("xvec_b200 has no CPU path: move the input (and the model) to a CUDA device")
-        if flat_x.dim() != 2 or flat_x.shape[1] != self.input_size:
-            raise ValueError(f"expected a flat (rows, {self.input_size}) frame matrix")
-        lay = self._layout_for(lengths)
-        if lay.rows != flat_x.shape[0]:
-            raise ValueError("sum(lengths) does not match the number of rows")
-        pipe = self._pipeline()
-        sc = self._scratch_for(slot)
-        sc.ensure(lay.rows, lay.n_slots, lay.n_utts)
-        sc.ensure_head(lay.n_utts, pipe["fc_shapes"], pipe["hidden"])
-        if flat_x.dtype != torch.float32:
-            flat_x = flat_x.float()
-        x = self._frames_for(flat_x, pipe)
-        if out is None:
-            out = torch.empty((lay.n_utts, pipe["out_dim"]), dtype=torch.float32, device=flat_x.device)
-        elif (out.dtype != torch.float32 or out.device != flat_x.device or out.shape != (lay.n_utts, pipe["out_dim"]) or out.stride(1) != 1):
-            raise ValueError(f"out must be a float32 ({lay.n_utts}, {pipe['out_dim']}) tensor on the input's device with unit column stride")
-        lib = _lib.load()
-        p = _lib.ptr
-        with _lib.on_device(flat_x.device):
-            _lib.check(lib.xvec_extract_forward(
-                pipe["tdnn"], pipe["n_tdnn"], p(x), lay.rows, x.stride(0), p(sc.act[0]), p(sc.act[1]), sc.ld, p(lay.row_utt),
-                p(lay.blk_slot_base), p(lay.utt_slot_start), p(lay.n_pool), lay.n_utts, p(sc.part), p(pipe["scale5"]), p(pipe["shift5"]),
-                p(sc.pooled), p(sc.pooled_lp), pipe["fc"], pipe["n_fc"], p(sc.fc_tmp), p(sc.ws),
-                0 if sc.ws is None else sc.ws.numel(), p(out), out.stride(0), p(sc.ctrl), sc.ctrl.numel(), _lib.stream_ptr()))
-        return out
+        return self._extract_forward(flat_x, lengths, slot, head=True, out=out)[2]
 
     # ------------------------------------------------------------------ reference surface
     def extract_x_vec(self, x: torch.Tensor) -> torch.Tensor:

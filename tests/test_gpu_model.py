@@ -221,9 +221,9 @@ def test_strided_frame_matrix_is_not_read_as_windows(xb, state_dict, precision):
 
 @pytest.mark.parametrize("precision", ["tf32", "bf16"])
 def test_wide_context_falls_back_to_per_layer_launches(xb, precision):
-    """A stack the one-launch kernel does not take (tap span 10 > XVEC_STACK_MAX_TAP_OFFSET = 8): extract_x_vec_flat (C-side
-    fallback) and pooled_stats_flat / forward (Python-side fallback) must both run it one launch per layer, and agree with a
-    plain torch fp32 statement of the reference's op sequence (tdnn_layer.py:26-41, main.py:59-63, 81-94)."""
+    """A stack the one-launch kernel does not take (tap span 10 > XVEC_STACK_MAX_TAP_OFFSET = 8): xvec_extract_forward falls back
+    to one launch per layer, and what it computes through extract_x_vec_flat and through pooled_stats_flat / forward must agree
+    with a plain torch fp32 statement of the reference's op sequence (tdnn_layer.py:26-41, main.py:59-63, 81-94)."""
     torch.manual_seed(3)
     m = xb.XVectorModel(precision=precision)
     m.time_context_layers[1] = xb.TdnnLayer(input_size=512, output_size=512, context=[-5, 0, 5])

@@ -55,6 +55,25 @@ def test_fails_loudly_without_gpu():
         m.stat_pool(torch.randn(2, 40, 1500))
 
 
+def test_extract_forward_segment_layer_count():
+    """xvec_extract_forward takes 0 to 2 segment layers.  Its arguments are checked before any CUDA call, so this needs no
+    device: 3 layers are rejected; 0 layers with NULL fc_host / out_dev pass the checks and fail only at the missing device."""
+    lib = xvec_b200._lib.load()
+    tdnn = (xvec_b200._lib.LayerDesc * 2)()
+    for d in tdnn:
+        d.w_packed_dev, d.bias_dev, d.n, d.cin, d.taps, d.dtype = 256, 256, 256, 256, 1, xvec_b200._lib.F32
+    fc = (xvec_b200._lib.LayerDesc * 3)()
+    buf = 256  # stands for device pointers; nothing is dereferenced on these paths
+
+    def call(fc_host, n_fc, out):
+        return lib.xvec_extract_forward(tdnn, 2, buf, 300, 256, buf, buf, 256, buf, buf, buf, buf, 1, buf, None, None, buf, None,
+                                        fc_host, n_fc, buf, None, 0, out, 256, None, 0, None)
+
+    assert call(fc, 3, buf) == xvec_b200._lib.E_ARG
+    if lib.xvec_device_check() != 0:  # no usable device: the call gets as far as the first CUDA call and reports its error
+        assert call(None, 0, None) == lib.xvec_device_check() != xvec_b200._lib.E_ARG
+
+
 def _emulate_fused_pool(lay, r):
     """numpy model of the EPI_POOL epilogue + finalize: per 128-row block, per utterance present -> one slot."""
     P = r.shape[1]
