@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define XVEC_ABI_VERSION 7
+#define XVEC_ABI_VERSION 8
 
 #if defined(__GNUC__)
 #define XVEC_API __attribute__((visibility("default")))
@@ -37,6 +37,8 @@ extern "C" {
 /* element types of activations / packed weights */
 #define XVEC_F32 0  /* float32 storage, tensor-core math in TF32 (kind::tf32), fp32 accumulate */
 #define XVEC_BF16 1 /* bfloat16 storage, kind::f16 bf16 math, fp32 accumulate */
+#define XVEC_F16 2  /* float16 storage, kind::f16 f16 math, fp32 accumulate: the 10-bit mantissa of TF32 operands at the rate and
+                       bytes of bf16, range |x| < 65504 (a larger activation becomes +inf, see DESIGN.md section 4) */
 
 #define XVEC_OK 0
 #define XVEC_E_ARG (-1)    /* bad shape / alignment / null pointer */
@@ -65,7 +67,7 @@ XVEC_API void xvec_watchdog_reset(void);
  * copies up to n of them to out_host and returns the count (0 when tracing is off). */
 XVEC_API int xvec_debug_trace(long long* out_host, int n);
 
-/* Number of K elements one packed weight row holds: taps * ceil(cin / kc) * kc, kc = 32 (F32) or 64 (BF16). */
+/* Number of K elements one packed weight row holds: taps * ceil(cin / kc) * kc, kc = 32 (F32) or 64 (BF16, F16). */
 XVEC_API int64_t xvec_packed_k(int cin, int taps, int dtype);
 /* Rows of a packed weight matrix: n rounded up to XVEC_TILE_N. */
 XVEC_API int64_t xvec_packed_n(int n);
@@ -73,7 +75,7 @@ XVEC_API int64_t xvec_packed_n(int n);
 /* Pack a Linear weight for xvec_tdnn_layer.
  * replaces: the layout nn.Linear(input_size*len(context), output_size) stores (tdnn_layer.py:19): W (n, taps*cin)
  * row-major, column index = tap*cin + channel (context-major, because of torch.cat(..., 2) at tdnn_layer.py:29).
- * w_dev: float32 (n, taps*cin).  out_dev: xvec_packed_n(n) * xvec_packed_k(cin,taps,dtype) elements of `dtype`, zero padded,
+ * w_dev: float32 (n, taps*cin); dtype XVEC_F32, XVEC_BF16 or XVEC_F16 (round to nearest).  out_dev: xvec_packed_n(n) * xvec_packed_k(cin,taps,dtype) elements of `dtype`, zero padded,
  * stored K-chunk-major ([128-byte K chunk][row][element]: every 128-row x 128-byte TMA box is one contiguous 16 KiB run);
  * the layout is private to this library — treat the buffer as opaque. */
 XVEC_API int xvec_pack_weight(const float* w_dev, int n, int taps, int cin, int dtype, void* out_dev, void* stream);
@@ -83,13 +85,13 @@ XVEC_API int xvec_pack_weight(const float* w_dev, int n, int taps, int cin, int 
  * replaces: TdnnLayer.forward (tdnn_layer.py:26-41) = get_time_context (tdnn_layer.py:43-60) + torch.cat +
  * nn.Linear + ReLU + eval-mode BatchNorm1d; with taps == 1 and relu/bn optional it is also nn.Linear
  * (segment_layer6/7, output: main.py:45-47, 87-90, 71-74).
- *   x_dev      (x_rows, cin) of x_dtype, row stride x_ld elements (x_ld*elsize multiple of 16 bytes, base 16-byte aligned)
+ *   x_dev      (x_rows, cin) of x_dtype (XVEC_F32 / XVEC_BF16 / XVEC_F16), row stride x_ld elements (x_ld*elsize multiple of 16 bytes, base 16-byte aligned)
  *   w_packed   from xvec_pack_weight with the same taps/cin/dtype
  *   tap_offsets_host  taps non-negative row offsets c_j - c_0 (HOST array)
  *   bias_dev   float32 or NULL;  bn_scale_dev/bn_shift_dev float32 or both NULL:
  *              scale = gamma/sqrt(running_var+eps), shift = beta - running_mean*scale.
  *              These vectors are read 32 columns at a time: each must be 16-byte aligned and hold ceil(n/32)*32 floats.
- *   y_dev      (rows, n) of y_dtype, row stride y_ld elements.  Input rows beyond x_rows read as zero.
+ *   y_dev      (rows, n) of y_dtype (XVEC_F32 / XVEC_BF16 / XVEC_F16), row stride y_ld elements.  Input rows beyond x_rows read as zero.
  *   splitk_ws_dev / splitk_ws_bytes  optional scratch (16-byte aligned) of at least xvec_splitk_workspace_bytes(...)
  *              bytes: when the GEMM has too few output tiles to fill the GPU (segment6: a few hundred rows, K = 3000)
  *              the K loop is split over CTA pairs into this workspace and a fixed-order second pass applies the
@@ -126,7 +128,7 @@ XVEC_API int xvec_build_layout(const int32_t* starts_dev, const int32_t* n_pool_
  * column sums of x and x*x over rows [row_start[u] + j*XVEC_POOL_CHUNK, ...) -> part_dev[slot_start[u] + j][2][p].
  * replaces: the reads of torch.mean / torch.std in XVectorModel.stat_pool (main.py:59-63) on a materialised
  * (B, T', p) activation; ragged lengths are an extension (the reference pads/cuts to 3 s, dataset.py:204).
- *   x_dev (.., p) of x_dtype with row stride x_ld elements; p multiple of 4
+ *   x_dev (.., p) of x_dtype (XVEC_F32 or XVEC_BF16; XVEC_F16 is not taken) with row stride x_ld elements; p multiple of 4
  *   row_start_dev int64 (n_utts), n_rows_dev int32 (n_utts), slot_start_dev int32 (n_utts+1) = exclusive prefix
  *   sum of ceil(n_rows/XVEC_POOL_CHUNK); max_chunks = max over utterances of that count.
  *   pivot_dev float32 (n_utts, p), 16-byte aligned, or NULL: when given, the sums are taken of x - pivot with pivot = the
@@ -143,8 +145,8 @@ XVEC_API int xvec_stats_pool_partial(const void* x_dev, int x_dtype, int64_t x_l
  * replaces: torch.mean, torch.std, torch.cat in stat_pool (main.py:60-62) (+ the BatchNorm of TDNN5 folded
  * through the statistics when bn_scale/shift are given; both NULL = plain pooling).
  *   pivot_dev float32 (n_utts, p) or NULL: the partial sums are of x - pivot (xvec_stats_pool_partial); the mean gets it back.
- *   out_f32_dev float32 (n_utts, 2p) [mean || std], row stride 2p;  out_lp_dev optional second copy in out_lp_dtype
- *   with row stride out_lp_ld (feeds segment_layer6 directly), or NULL.
+ *   out_f32_dev float32 (n_utts, 2p) [mean || std], row stride 2p;  out_lp_dev optional second copy in out_lp_dtype (XVEC_F32,
+ *   XVEC_BF16 or XVEC_F16; NaN stays NaN) with row stride out_lp_ld (feeds segment_layer6 directly), or NULL.
  */
 XVEC_API int xvec_pool_finalize(const float* part_dev, const int32_t* slot_start_dev, const int32_t* n_rows_dev, int n_utts,
                        int p, const float* bn_scale_dev, const float* bn_shift_dev, const float* pivot_dev, float* out_f32_dev,
@@ -158,7 +160,7 @@ typedef struct XvecLayerDesc {
   int32_t n;      /* output channels */
   int32_t cin;    /* input channels per tap */
   int32_t taps;
-  int32_t dtype;  /* XVEC_F32 / XVEC_BF16: element type of this layer's INPUT activations and packed weights */
+  int32_t dtype;  /* XVEC_F32 / XVEC_BF16 / XVEC_F16: element type of this layer's INPUT activations and packed weights */
   int32_t tap_offsets[XVEC_MAX_TAPS];
   const void* w_plain_dev; /* segment layers only, optional: the nn.Linear weight itself in `dtype`, (n, cin) row-major, row
                               stride cin — lets xvec_extract_forward run the layer with xvec_linear_small; NULL otherwise */
@@ -169,7 +171,8 @@ typedef struct XvecLayerDesc {
  * 256-channel tile) is a work item drawn in order from a global counter by the CTA pairs; a tile of layer l+1 starts as soon as
  * the tiles of layer l it reads are complete (per-tile flags in ctrl_dev), so the layers overlap inside the launch.
  * replaces: time_context_layers (main.py:38-44) applied by extract_x_vec (main.py:82) + the reads of stat_pool (main.py:59-63).
- *   x_dev is of tdnn_host[0].dtype; layers 1.. share one dtype (the activation dtype); layers 0..n-2 need n % XVEC_TILE_N == 0
+ *   x_dev is of tdnn_host[0].dtype; layers 1.. share one dtype (the activation dtype: XVEC_F32, XVEC_BF16 or XVEC_F16); layer 0
+ *   is XVEC_F32 (TF32 math) or the activation dtype (a float32 layer 0 with XVEC_BF16 activations may also be XVEC_BF16); layers 0..n-2 need n % XVEC_TILE_N == 0
  *   and a bias; eval-mode BatchNorm folded forward as for xvec_extract_forward.
  *   Window form of a layer with consecutive taps (context [-2..2] of TDNN1, tdnn_layer.py:43-60): when its input rows are
  *   dense (x_ld == channels) the taps*channels window of output row r is ONE contiguous run starting at row r, so the layer
@@ -195,7 +198,7 @@ XVEC_API int xvec_tdnn_stack(const struct XvecLayerDesc* tdnn_host, int n_tdnn, 
                     float* part_dev, void* ctrl_dev, int64_t ctrl_bytes, int band, void* stream);
 
 /* Small-footprint linear layer: y = act(x W' + bias), x (rows, k) and W (n, k) row-major (the nn.Linear layout, NOT packed) of
- * `dtype` (XVEC_BF16, or XVEC_F32 = TF32 math), float32 accumulation, y float32 or bfloat16.  128 threads, 5 KiB of shared
+ * `dtype` (XVEC_BF16, XVEC_F16, or XVEC_F32 = TF32 math), float32 accumulation, y float32, bfloat16 or float16 (y_dtype).  128 threads, 5 KiB of shared
  * memory, no tensor memory: its CTAs fit next to a resident CTA of the persistent xvec_tdnn_stack kernel, so the segment layers
  * of one batch run concurrently with the frame-level stack of the next one instead of waiting for free SMs.
  * replaces: segment_layer6 / segment_layer7 (main.py:45-46, 87-90) on the pooled statistics.
@@ -213,8 +216,9 @@ XVEC_API int xvec_linear_small(const void* x_dev, int dtype, int64_t rows, int k
  * layer's packed weights, the last TDNN layer's BatchNorm is passed as bn_last_scale/shift (or NULL).
  *   x_dev (rows, tdnn[0].cin) of tdnn[0].dtype, row stride x_ld (window form: see xvec_tdnn_stack);  act0/act1: ping-pong activation buffers (rows, act_ld) of the
  *   dtype of tdnn[1];  layout arrays as for xvec_tdnn_pool_fused / xvec_pool_finalize;  part_dev (n_slots, 2, n_last);
- *   pooled_dev float32 (n_utts, 2 n_last);  pooled_lp_dev NULL or a bfloat16 copy of it (n_utts, 2 n_last), required when
- *   fc[0].dtype is XVEC_BF16 (the first segment layer reads it);  fc: n_fc segment layers (taps == 1);
+ *   pooled_dev float32 (n_utts, 2 n_last);  pooled_lp_dev NULL or a 16-bit copy of it (n_utts, 2 n_last): in fc[0].dtype when that
+ *   is XVEC_BF16 or XVEC_F16 (the first segment layer reads it; required then), else in float16 when the TDNN layers are
+ *   XVEC_F16, else in bfloat16;  fc: n_fc segment layers (taps == 1);
  *   fc_tmp_dev (n_utts, fc[0].n) of fc[1].dtype when n_fc == 2;  out_dev float32 (n_utts, fc[n_fc-1].n), row stride out_ld;
  *   splitk_ws_dev: scratch for the segment layers (see xvec_splitk_workspace_bytes) or NULL;
  *   ctrl_dev / ctrl_bytes: scratch of xvec_tdnn_stack or NULL / 0.
@@ -246,8 +250,9 @@ XVEC_API int xvec_mfcc(const void* wav_dev, int wav_is_int16, const int64_t* wav
 XVEC_API int xvec_wav_minmax(const void* wav_dev, int wav_is_int16, const int64_t* wav_start_dev, const int32_t* wav_len_dev,
                     int n_utts, float* norm_offset_dev, float* norm_scale_dev, void* stream);
 
-/* float32 -> dtype copy of a (rows, cols) matrix (row strides in elements); XVEC_F32 is a strided copy.
- * replaces: samples.float() (main.py:137) for the bf16 pipeline. */
+/* float32 -> dtype copy of a (rows, cols) matrix (row strides in elements); XVEC_F32 is a strided copy, XVEC_BF16 / XVEC_F16 round
+ * to nearest (NaN stays NaN).
+ * replaces: samples.float() (main.py:137) for the 16-bit pipelines. */
 XVEC_API int xvec_cast(const float* src_dev, int64_t src_ld, void* dst_dev, int dst_dtype, int64_t dst_ld, int64_t rows,
               int cols, void* stream);
 

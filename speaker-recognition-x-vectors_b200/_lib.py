@@ -13,10 +13,10 @@ from ctypes import POINTER, c_char_p, c_float, c_int, c_int32, c_int64, c_void_p
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("XVEC_LIB") or os.path.join(HERE, "libxvec_b200.so")  # XVEC_LIB: developer A/B builds
 
-F32, BF16 = 0, 1
+F32, BF16, F16 = 0, 1, 2
 E_ARG, E_CUDA, E_DEVICE = -1, -2, -3
 TILE_N, POOL_BLOCK, POOL_CHUNK, MAX_TAPS = 256, 128, 128, 8
-ABI_VERSION = 7
+ABI_VERSION = 8
 MAX_STACK = 6
 STACK_MAX_TAP_OFFSET = 8  # XVEC_STACK_MAX_TAP_OFFSET
 
@@ -140,7 +140,9 @@ def dtype_code(torch_dtype) -> int:
         return F32
     if torch_dtype == torch.bfloat16:
         return BF16
-    raise ValueError(f"unsupported dtype {torch_dtype}; the kernels take float32 (TF32 math) or bfloat16")
+    if torch_dtype == torch.float16:
+        return F16
+    raise ValueError(f"unsupported dtype {torch_dtype}; the kernels take float32 (TF32 math), bfloat16 or float16")
 
 
 def taps_array(offsets):

@@ -217,14 +217,18 @@ int xvec_extract_forward(const XvecLayerDesc* tdnn, int n_tdnn, const void* x_de
     return set_error(XVEC_E_ARG, "need >= 2 TDNN layers and 0 to 2 segment layers");
   if (!x_dev || !act0_dev || !act1_dev || !pooled_dev || (n_fc > 0 && !out_dev)) return set_error(XVEC_E_ARG, "null pointer argument");
   if (n_fc == 2 && !fc_tmp_dev) return set_error(XVEC_E_ARG, "fc_tmp_dev is NULL");
-  const bool lp_head = n_fc > 0 && fc[0].dtype == XVEC_BF16;
-  if (lp_head && !pooled_lp_dev) return set_error(XVEC_E_ARG, "pooled_lp_dev is required for bf16 segment layers");
+  // lp_head: the first segment layer is 16-bit and reads the pooled statistics in its own dtype
+  const bool lp_head = n_fc > 0 && (fc[0].dtype == XVEC_BF16 || fc[0].dtype == XVEC_F16);
+  if (lp_head && !pooled_lp_dev) return set_error(XVEC_E_ARG, "pooled_lp_dev is required for 16-bit segment layers");
+  // the 16-bit copy: in the first segment layer's dtype when that reads it, else (n_fc == 0: the caller runs the head itself) in
+  // float16 for a float16 frame stack, else in bfloat16
+  const int lp_dtype = lp_head ? fc[0].dtype : tdnn[n_tdnn - 1].dtype == XVEC_F16 ? XVEC_F16 : XVEC_BF16;
   int rc = frame_stack(tdnn, n_tdnn, x_dev, rows, x_ld, act0_dev, act1_dev, act_ld, row_utt_dev, blk_slot_base_dev, part_dev, ctrl_dev,
                        ctrl_bytes, stream);
   if (rc) return rc;
   const int64_t pooled_ld = 2 * static_cast<int64_t>(tdnn[n_tdnn - 1].n);
   rc = xvec_pool_finalize(part_dev, utt_slot_start_dev, n_pool_dev, n_utts, tdnn[n_tdnn - 1].n, bn_last_scale_dev, bn_last_shift_dev, nullptr,
-                          pooled_dev, pooled_lp_dev, XVEC_BF16, pooled_ld, stream);
+                          pooled_dev, pooled_lp_dev, lp_dtype, pooled_ld, stream);
   if (rc) return rc;
   return segment_head(fc, n_fc, lp_head ? pooled_lp_dev : static_cast<const void*>(pooled_dev), pooled_ld, n_utts, fc_tmp_dev, splitk_ws_dev,
                       splitk_ws_bytes, out_dev, out_ld, stream);

@@ -38,6 +38,32 @@ __device__ __forceinline__ uint32_t pack_bf16x2_relu(float lo, float hi) {
   asm("cvt.rn.relu.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
   return r;
 }
+// The same for float16.  No .satfinite: a value beyond the float16 range becomes +inf and reaches the x-vector as a non-finite
+// value instead of a plausible wrong number (DESIGN.md section 4).
+__device__ __forceinline__ uint32_t pack_f16x2(float lo, float hi) {
+  uint32_t r;
+  asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
+  return r;
+}
+__device__ __forceinline__ uint32_t pack_f16x2_relu(float lo, float hi) {
+  uint32_t r;
+  asm("cvt.rn.relu.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
+  return r;
+}
+// 16-bit pair packs of activation dtype kDtype (XVEC_BF16 or XVEC_F16).
+template <int kDtype>
+__device__ __forceinline__ uint32_t pack16x2(float lo, float hi) {
+  if constexpr (kDtype == XVEC_F16) return pack_f16x2(lo, hi);
+  else return pack_bf16x2(lo, hi);
+}
+template <int kDtype>
+__device__ __forceinline__ uint32_t pack16x2_relu(float lo, float hi) {
+  if constexpr (kDtype == XVEC_F16) return pack_f16x2_relu(lo, hi);
+  else return pack_bf16x2_relu(lo, hi);
+}
+
+// Operand format of the UMMA instruction descriptor for operands of element type `dtype` (umma_idesc, ptx.cuh).
+__host__ __device__ constexpr uint32_t umma_format(int dtype) { return dtype == XVEC_F32 ? 2u : dtype == XVEC_BF16 ? 1u : 0u; }
 
 // Statistics-pooling epilogue of one TRANSPOSED accumulator tile for one epilogue warp (replaces the reads of torch.mean /
 // torch.std in stat_pool, main.py:59-63).  The MMA warp swaps the operands of the pooled layer (weights = M operand, frames = N
@@ -167,14 +193,16 @@ inline int make_tmap_2d(CUtensorMap* map, const void* ptr, int dtype, uint64_t i
                         uint32_t box_inner, uint32_t box_outer, CUtensorMapSwizzle swizzle = CU_TENSOR_MAP_SWIZZLE_128B) {
   PFN_encodeTiled enc = get_encode_tiled();
   if (!enc) return set_error(XVEC_E_CUDA, "cuTensorMapEncodeTiled is not available from the driver");
-  const uint64_t es = dtype == XVEC_BF16 ? 2 : 4;
+  const uint64_t es = elem_bytes(dtype);
   if ((reinterpret_cast<uintptr_t>(ptr) & 15u) != 0) return set_error(XVEC_E_ARG, "matrix base pointer must be 16-byte aligned");
   if ((ld_elems * es) % 16 != 0) return set_error(XVEC_E_ARG, "row stride must be a multiple of 16 bytes");
   cuuint64_t dims[2] = {inner, outer};
   cuuint64_t strides[1] = {ld_elems * es};
   cuuint32_t box[2] = {box_inner, box_outer};
   cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(map, dtype == XVEC_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2,
+  const CUtensorMapDataType type = dtype == XVEC_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16
+                                 : dtype == XVEC_F16  ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
+  CUresult r = enc(map, type, 2,
                    const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                    swizzle, l2_promotion(), CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) return set_error(XVEC_E_CUDA, "cuTensorMapEncodeTiled failed (CUresult %d)", static_cast<int>(r));

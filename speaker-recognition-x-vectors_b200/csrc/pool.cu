@@ -1,7 +1,8 @@
 // Bandwidth-bound kernels of the extraction path: standalone statistics pooling (partial + finalize), the
-// float32 -> bf16 cast, weight packing and per-trial cosine scoring.  sm_100a build; plain coalesced streaming code —
+// float32 -> bf16 / f16 cast, weight packing and per-trial cosine scoring.  sm_100a build; plain coalesced streaming code —
 // these are HBM/L2-bound reductions, not tensor-core work.
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 
 #include "xvec_internal.h"
 
@@ -138,6 +139,10 @@ pool_finalize_kernel(const float* __restrict__ part, const int* __restrict__ slo
       __nv_bfloat16* o = reinterpret_cast<__nv_bfloat16*>(out_lp) + static_cast<size_t>(u) * lp_ld;
       o[col] = __float2bfloat16_rn(m);
       o[p + col] = __float2bfloat16_rn(sd);
+    } else if (lp_dtype == XVEC_F16) {  // round to nearest, NaN stays NaN (a single-frame utterance, like torch.std)
+      __half* o = reinterpret_cast<__half*>(out_lp) + static_cast<size_t>(u) * lp_ld;
+      o[col] = __float2half_rn(m);
+      o[p + col] = __float2half_rn(sd);
     } else {
       float* o = reinterpret_cast<float*>(out_lp) + static_cast<size_t>(u) * lp_ld;
       o[col] = m;
@@ -190,6 +195,8 @@ __global__ void cast_kernel(const float* __restrict__ src, long long src_ld, voi
     const float v = src[r * src_ld + c];
     if (dst_dtype == XVEC_BF16)
       reinterpret_cast<__nv_bfloat16*>(dst)[r * dst_ld + c] = __float2bfloat16_rn(v);
+    else if (dst_dtype == XVEC_F16)
+      reinterpret_cast<__half*>(dst)[r * dst_ld + c] = __float2half_rn(v);
     else
       reinterpret_cast<float*>(dst)[r * dst_ld + c] = v;
   }
@@ -207,10 +214,12 @@ __global__ void pack_weight_kernel(const float* __restrict__ w, int n, int taps,
     const float v = (row < n && ch < cin) ? w[row * (static_cast<long long>(taps) * cin) + tap * cin + ch] : 0.f;
     // chunk-major: [K chunk of 128 bytes][row][element in chunk] — the 128-row x 128-byte box the GEMM producers load per
     // K chunk is then one contiguous 16 KiB run of global memory instead of 128 pieces k_pad*elsize bytes apart
-    const int bke = dtype == XVEC_BF16 ? 64 : 32;
+    const int bke = dtype == XVEC_F32 ? 32 : 64;
     const long long o = (static_cast<long long>(kk / bke) * n_pad + row) * bke + kk % bke;
     if (dtype == XVEC_BF16)
       reinterpret_cast<__nv_bfloat16*>(out)[o] = __float2bfloat16_rn(v);
+    else if (dtype == XVEC_F16)
+      reinterpret_cast<__half*>(out)[o] = __float2half_rn(v);
     else
       reinterpret_cast<float*>(out)[o] = v;
   }
@@ -354,7 +363,7 @@ int xvec_pool_finalize(const float* part_dev, const int32_t* slot_start_dev, con
   if (!part_dev || !slot_start_dev || !n_rows_dev || !out_f32_dev) return set_error(XVEC_E_ARG, "null pointer argument");
   if (n_utts <= 0 || p <= 0) return set_error(XVEC_E_ARG, "non-positive size");
   if ((bn_scale_dev == nullptr) != (bn_shift_dev == nullptr)) return set_error(XVEC_E_ARG, "bn_scale and bn_shift must be given together");
-  if (out_lp_dev && (out_lp_dtype != XVEC_F32 && out_lp_dtype != XVEC_BF16)) return set_error(XVEC_E_ARG, "bad out_lp_dtype");
+  if (out_lp_dev && !valid_dtype(out_lp_dtype)) return set_error(XVEC_E_ARG, "bad out_lp_dtype");
   if (out_lp_dev && out_lp_ld < 2 * p) return set_error(XVEC_E_ARG, "out_lp_ld < 2p");
   dim3 grid(n_utts, (p + 127) / 128);
   pool_finalize_kernel<<<grid, 128, 0, static_cast<cudaStream_t>(stream)>>>(part_dev, slot_start_dev, n_rows_dev, p, bn_scale_dev,
@@ -368,7 +377,7 @@ int xvec_cast(const float* src_dev, int64_t src_ld, void* dst_dev, int dst_dtype
   if (rc) return rc;
   if (!src_dev || !dst_dev) return set_error(XVEC_E_ARG, "null pointer argument");
   if (rows <= 0 || cols <= 0 || src_ld < cols || dst_ld < cols) return set_error(XVEC_E_ARG, "bad shape");
-  if (dst_dtype != XVEC_F32 && dst_dtype != XVEC_BF16) return set_error(XVEC_E_ARG, "bad dst_dtype");
+  if (!valid_dtype(dst_dtype)) return set_error(XVEC_E_ARG, "bad dst_dtype");
   const long long total = rows * cols;
   const int blocks = grid_for(total);
   cast_kernel<<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(src_dev, src_ld, dst_dev, dst_dtype, dst_ld, rows, cols);
@@ -380,7 +389,7 @@ int xvec_pack_weight(const float* w_dev, int n, int taps, int cin, int dtype, vo
   if (rc) return rc;
   if (!w_dev || !out_dev) return set_error(XVEC_E_ARG, "null pointer argument");
   if (n <= 0 || cin <= 0 || taps < 1 || taps > XVEC_MAX_TAPS) return set_error(XVEC_E_ARG, "bad shape");
-  if (dtype != XVEC_F32 && dtype != XVEC_BF16) return set_error(XVEC_E_ARG, "bad dtype");
+  if (!valid_dtype(dtype)) return set_error(XVEC_E_ARG, "bad dtype");
   const long long k_pad = xvec_packed_k(cin, taps, dtype);
   const long long n_pad = xvec_packed_n(n);
   const long long total = n_pad * k_pad;

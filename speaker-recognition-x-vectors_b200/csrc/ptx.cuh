@@ -218,7 +218,7 @@ __device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t smem_addr) {
 }
 
 // Instruction descriptor for kind::f16 / kind::tf32, fp32 accumulate, both operands K-major.
-// fmt: 1 = bf16, 2 = tf32.  (c_format [4,6) | a_format [7,10) | b_format [10,13) | N>>3 [17,23) | M>>4 [24,29))
+// fmt: 0 = f16, 1 = bf16, 2 = tf32 (umma_format in gemm_tile.cuh).  (c_format [4,6) | a_format [7,10) | b_format [10,13) | N>>3 [17,23) | M>>4 [24,29))
 __host__ __device__ constexpr uint32_t umma_idesc(uint32_t fmt, uint32_t m, uint32_t n) {
   return (1u << 4) | (fmt << 7) | (fmt << 10) | ((n >> 3) << 17) | ((m >> 4) << 24);
 }

@@ -29,10 +29,14 @@
 // fused kernel does not take.
 #include "gemm_tile.cuh"
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 
 namespace xvec {
 
-enum { EPI_STORE_F32 = 0, EPI_STORE_BF16 = 1, EPI_POOL = 2 };
+enum { EPI_STORE_F32 = 0, EPI_STORE_BF16 = 1, EPI_POOL = 2, EPI_STORE_F16 = 3 };
+// Flag of the kernel's epilogue argument: the operands are float16 (kind::f16 in f16 format) instead of bfloat16.  A flag rather
+// than a third template parameter, so that the bf16 / TF32 kernels keep their template arguments and symbol names.
+constexpr int EPI_IN_F16 = 8;
 
 struct GemmParams {
   int rows;     // output rows
@@ -83,10 +87,14 @@ constexpr int gemm_smem_bytes() {
   return 1024 + num_stages<kEpi>() * STAGE_BYTES + epi_smem_bytes<kEpi>();
 }
 
+// Operands: float32 with kind::tf32 (kTf32), else bfloat16, or float16 when kEpi carries EPI_IN_F16; kEpi & ~EPI_IN_F16 is the
+// epilogue.  It is written out where it is used: a kernel-scope constexpr variable for it (or for the operand dtype) changes
+// nvcc's register allocation in the bf16 / TF32 pooling kernels, whose code stays as it was measured.
 template <bool kTf32, int kEpi>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 tdnn_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                  const __grid_constant__ CUtensorMap tmY, const GemmParams p) {
+  static_assert(!(kTf32 && (kEpi & EPI_IN_F16)), "float16 operands run kind::f16");
   constexpr int STAGES = num_stages<kEpi>();
   extern __shared__ uint8_t smem_raw[];
   __shared__ uint64_t full_bar[STAGES], empty_bar[STAGES], tfull_bar[2], tempty_bar[2];
@@ -111,7 +119,7 @@ tdnn_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmA);
     tma_prefetch_desc(&tmB);
-    if constexpr (kEpi != EPI_POOL) tma_prefetch_desc(&tmY);
+    if constexpr ((kEpi & ~EPI_IN_F16) != EPI_POOL) tma_prefetch_desc(&tmY);
     for (int s = 0; s < STAGES; ++s) {
       mbar_init(&full_bar[s], 1);   // leader's arrive.expect_tx (bytes of both CTAs)
       mbar_init(&empty_bar[s], 1);  // leader's multicast commit
@@ -178,7 +186,7 @@ tdnn_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     // elected lane issues tcgen05.mma / tcgen05.commit; the readiness of the NEXT stage is probed before the MMAs are
     // issued so the probe latency is off the critical path)
     if (rank == 0) {
-      constexpr uint32_t idesc = umma_idesc(kTf32 ? 2u : 1u, BM, BN);
+      constexpr uint32_t idesc = umma_idesc(umma_format(kTf32 ? XVEC_F32 : (kEpi & EPI_IN_F16) ? XVEC_F16 : XVEC_BF16), BM, BN);
       int stage = 0;
       uint32_t phase = 0;
       int it = 0;
@@ -197,8 +205,8 @@ tdnn_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
           if (kb == kb0 && lane == 0) trace(p, it, 3);
           const uint32_t a_addr = smem_u32(base + stage * STAGE_BYTES);
           // EPI_POOL computes the tile transposed (weights = M operand): see pool_epilogue_tile_t
-          const uint64_t da = umma_desc_sw128(kEpi == EPI_POOL ? a_addr + A_BYTES : a_addr);
-          const uint64_t db = umma_desc_sw128(kEpi == EPI_POOL ? a_addr : a_addr + A_BYTES);
+          const uint64_t da = umma_desc_sw128((kEpi & ~EPI_IN_F16) == EPI_POOL ? a_addr + A_BYTES : a_addr);
+          const uint64_t db = umma_desc_sw128((kEpi & ~EPI_IN_F16) == EPI_POOL ? a_addr : a_addr + A_BYTES);
           int stage_n = stage + 1;
           uint32_t phase_n = phase;
           if (stage_n == STAGES) { stage_n = 0; phase_n ^= 1u; }
@@ -251,14 +259,17 @@ tdnn_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
       };
       const int c_last = min(cend, p.n - n0) - 1;  // last valid column of this warp's range (may be < cbeg)
 
-      if constexpr (kEpi == EPI_POOL) {
+      if constexpr ((kEpi & ~EPI_IN_F16) == EPI_POOL) {
         const PoolArgs pa{p.rows, p.n, p.bias, p.row_utt, p.blk_slot_base, p.part};
         const int pch = n0 + static_cast<int>(rank) * BN_CTA + q * 32 + lane, pf0 = (tt / p.n_tiles) * BM + cbeg;
         pool_epilogue_tile_t(pa, pool_prefetch(pa, pch, pf0, lane), tmem_base + buf * BN + (static_cast<uint32_t>(q * 32) << 16) + cbeg, pch,
                              pf0, lane, release_tmem);
       } else {
         uint8_t* out_stage = epi_smem + (warp - 2) * (OUT_BUFS * OUT_BUF_BYTES);  // 32-row x 128-byte staging boxes
-        constexpr int OUT_ES = kEpi == EPI_STORE_BF16 ? 2 : 4;
+        constexpr int kStore = kEpi & ~EPI_IN_F16;
+        constexpr bool k16 = kStore == EPI_STORE_BF16 || kStore == EPI_STORE_F16;  // 16-bit output
+        constexpr int kOut = kStore == EPI_STORE_F16 ? XVEC_F16 : XVEC_BF16;        // ... and its type
+        constexpr int OUT_ES = k16 ? 2 : 4;
         constexpr int GROUP_COLS = 128 / OUT_ES;     // columns per TMA-store box (128 bytes per row)
         constexpr int CHUNKS = GROUP_COLS / 32;      // tcgen05.ld chunks per box
         for (int c = cbeg; c < cend && n0 + c < p.n; c += GROUP_COLS) {
@@ -293,7 +304,7 @@ tdnn_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                 const float2 d = __fadd2_rn(make_float2(__uint_as_float(v[j4 + 2]), __uint_as_float(v[j4 + 3])), make_float2(bb.z, bb.w));
                 o[j4 + 0] = a.x; o[j4 + 1] = a.y; o[j4 + 2] = d.x; o[j4 + 3] = d.y;
               }
-              if (p.relu && kEpi != EPI_STORE_BF16) {  // bf16 output: ReLU is folded into the convert below
+              if (p.relu && !k16) {  // 16-bit output: ReLU is folded into the convert below
 #pragma unroll
                 for (int j = 0; j < 32; ++j) o[j] = relu_keep_nan(o[j]);
               }
@@ -313,27 +324,27 @@ tdnn_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                 o[j4 + 0] = a.x; o[j4 + 1] = a.y; o[j4 + 2] = d.x; o[j4 + 3] = d.y;
               }
             }
-            const bool cvt_relu = p.relu && p.scale == nullptr;  // ReLU not applied yet (bf16 fast path)
+            const bool cvt_relu = p.relu && p.scale == nullptr;  // ReLU not applied yet (16-bit fast path)
             if (warp == 2 && lane == 0 && c == cbeg && cc == 0) trace(p, it, 10);
             if (XVEC_DBG(p, 2)) {
               if (o[0] == 123.456f && o[31] == 1.f) ob[lane] = 1;
             } else if (p.vec_store) {
               // row `lane` of the box, 16-byte pieces XOR-swizzled like CU_TENSOR_MAP_SWIZZLE_128B expects
               uint8_t* orow = ob + lane * 128;
-              if constexpr (kEpi == EPI_STORE_BF16) {
+              if constexpr (k16) {
 #pragma unroll
                 for (int j = 0; j < 4; ++j) {
                   uint4 w;
                   if (cvt_relu) {
-                    w.x = pack_bf16x2_relu(o[8 * j + 0], o[8 * j + 1]);
-                    w.y = pack_bf16x2_relu(o[8 * j + 2], o[8 * j + 3]);
-                    w.z = pack_bf16x2_relu(o[8 * j + 4], o[8 * j + 5]);
-                    w.w = pack_bf16x2_relu(o[8 * j + 6], o[8 * j + 7]);
+                    w.x = pack16x2_relu<kOut>(o[8 * j + 0], o[8 * j + 1]);
+                    w.y = pack16x2_relu<kOut>(o[8 * j + 2], o[8 * j + 3]);
+                    w.z = pack16x2_relu<kOut>(o[8 * j + 4], o[8 * j + 5]);
+                    w.w = pack16x2_relu<kOut>(o[8 * j + 6], o[8 * j + 7]);
                   } else {
-                    w.x = pack_bf16x2(o[8 * j + 0], o[8 * j + 1]);
-                    w.y = pack_bf16x2(o[8 * j + 2], o[8 * j + 3]);
-                    w.z = pack_bf16x2(o[8 * j + 4], o[8 * j + 5]);
-                    w.w = pack_bf16x2(o[8 * j + 6], o[8 * j + 7]);
+                    w.x = pack16x2<kOut>(o[8 * j + 0], o[8 * j + 1]);
+                    w.y = pack16x2<kOut>(o[8 * j + 2], o[8 * j + 3]);
+                    w.z = pack16x2<kOut>(o[8 * j + 4], o[8 * j + 5]);
+                    w.w = pack16x2<kOut>(o[8 * j + 6], o[8 * j + 7]);
                   }
                   const int piece = cc * 4 + j;
                   *reinterpret_cast<uint4*>(orow + ((piece ^ (lane & 7)) << 4)) = w;
@@ -346,11 +357,16 @@ tdnn_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                 }
               }
             } else if (row < p.rows) {
-              if constexpr (kEpi == EPI_STORE_BF16) {
+              if constexpr (kStore == EPI_STORE_BF16) {
                 __nv_bfloat16* dst = reinterpret_cast<__nv_bfloat16*>(p.out) + static_cast<size_t>(row) * p.ldo + col0;
 #pragma unroll
                 for (int j = 0; j < 32; ++j)
                   if (col0 + j < p.n) dst[j] = __float2bfloat16_rn(cvt_relu ? relu_keep_nan(o[j]) : o[j]);
+              } else if constexpr (kStore == EPI_STORE_F16) {
+                __half* dst = reinterpret_cast<__half*>(p.out) + static_cast<size_t>(row) * p.ldo + col0;
+#pragma unroll
+                for (int j = 0; j < 32; ++j)
+                  if (col0 + j < p.n) dst[j] = __float2half_rn(cvt_relu ? relu_keep_nan(o[j]) : o[j]);
               } else {
                 float* dst = reinterpret_cast<float*>(p.out) + static_cast<size_t>(row) * p.ldo + col0;
 #pragma unroll
@@ -376,7 +392,7 @@ tdnn_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
       if (!released) release_tmem();  // nothing was read (no pooled rows / no valid columns in this warp's range)
       if (warp == 2 && lane == 0) trace(p, it, 7);
     }
-    if constexpr (kEpi != EPI_POOL) {
+    if constexpr ((kEpi & ~EPI_IN_F16) != EPI_POOL) {
       if (lane == 0) tma_store_wait_all();
     }
   }
@@ -393,7 +409,7 @@ tdnn_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
 // Split-K second pass: y[r, c] = epi( sum_s ws[s*rows_pad + r, c] ) in fixed split order (deterministic).
 __global__ void __launch_bounds__(256)
 splitk_reduce_kernel(const float* __restrict__ ws, int ksplit, int rows, int rows_pad, int n, int ws_ld, const float* __restrict__ bias,
-                     const float* __restrict__ scale, const float* __restrict__ shift, int relu, void* __restrict__ out, int out_bf16,
+                     const float* __restrict__ scale, const float* __restrict__ shift, int relu, void* __restrict__ out, int out_dtype,
                      long long ldo) {
   const long long total = static_cast<long long>(rows) * n;
   for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < total;
@@ -405,8 +421,10 @@ splitk_reduce_kernel(const float* __restrict__ ws, int ksplit, int rows, int row
     if (bias) a += bias[c];
     if (relu) a = a < 0.f ? 0.f : a;  // keeps NaN like torch.relu
     if (scale) a = fmaf(a, scale[c], shift[c]);
-    if (out_bf16)
+    if (out_dtype == XVEC_BF16)
       reinterpret_cast<__nv_bfloat16*>(out)[static_cast<size_t>(r) * ldo + c] = __float2bfloat16_rn(a);
+    else if (out_dtype == XVEC_F16)
+      reinterpret_cast<__half*>(out)[static_cast<size_t>(r) * ldo + c] = __float2half_rn(a);
     else
       reinterpret_cast<float*>(out)[static_cast<size_t>(r) * ldo + c] = a;
   }
@@ -417,13 +435,16 @@ static long long* g_trace_buf = nullptr;
 
 // Persistent grid: one CTA pair per tile, at most one pair per two SMs.
 template <int kEpi>
-static int launch(bool tf32, const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& ty, const GemmParams& p, cudaStream_t st) {
+static int launch(int dtype, const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& ty, const GemmParams& p, cudaStream_t st) {
   const int64_t tiles = static_cast<int64_t>(p.m_tiles) * p.n_tiles * p.ksplit;
   const int max_pairs = num_sms() / 2;
   const int grid = 2 * static_cast<int>(tiles < max_pairs ? tiles : max_pairs);
   constexpr int smem = gemm_smem_bytes<kEpi>();
-  if (tf32) return launch_pair<tdnn_gemm_kernel<true, kEpi>>("tdnn_gemm_kernel", GEMM_THREADS, smem, grid, bind_watchdog_gemm, st, ta, tb, ty, p);
-  return launch_pair<tdnn_gemm_kernel<false, kEpi>>("tdnn_gemm_kernel", GEMM_THREADS, smem, grid, bind_watchdog_gemm, st, ta, tb, ty, p);
+  if (dtype == XVEC_F32)
+    return launch_pair<tdnn_gemm_kernel<true, kEpi>>("tdnn_gemm_kernel", GEMM_THREADS, smem, grid, bind_watchdog_gemm, st, ta, tb, ty, p);
+  if (dtype == XVEC_BF16)
+    return launch_pair<tdnn_gemm_kernel<false, kEpi>>("tdnn_gemm_kernel", GEMM_THREADS, smem, grid, bind_watchdog_gemm, st, ta, tb, ty, p);
+  return launch_pair<tdnn_gemm_kernel<false, kEpi | EPI_IN_F16>>("tdnn_gemm_kernel", GEMM_THREADS, smem, grid, bind_watchdog_gemm, st, ta, tb, ty, p);
 }
 
 // Split-K plan for GEMMs with too few output tiles to fill the machine (segment6/7: a few hundred rows, K = 3000).
@@ -457,7 +478,7 @@ static int gemm_setup(const XvecLayerDesc& l, const void* x, int64_t x_rows, int
   int rc = device_check();
   if (rc) return rc;
   if (!x || !l.w_packed_dev) return set_error(XVEC_E_ARG, "null pointer argument");
-  if (l.dtype != XVEC_F32 && l.dtype != XVEC_BF16) return set_error(XVEC_E_ARG, "bad x_dtype %d", l.dtype);
+  if (!valid_dtype(l.dtype)) return set_error(XVEC_E_ARG, "bad x_dtype %d", l.dtype);
   if (l.taps < 1 || l.taps > XVEC_MAX_TAPS) return set_error(XVEC_E_ARG, "taps must be in [1,%d]", XVEC_MAX_TAPS);
   if (rows <= 0 || x_rows <= 0 || l.cin <= 0 || l.n <= 0) return set_error(XVEC_E_ARG, "non-positive size");
   if (rows > 0x7fffff00LL || x_rows > 0x7fffff00LL) return set_error(XVEC_E_ARG, "too many rows");
@@ -503,7 +524,7 @@ static int gemm_setup(const XvecLayerDesc& l, const void* x, int64_t x_rows, int
 // Destination of a store epilogue: y_rows x n of y_dtype, row stride y_ld.  16-byte aligned rows are staged in swizzled shared
 // memory and TMA-stored through ty; other rows are stored element by element.
 static int set_store_output(GemmParams& p, CUtensorMap& ty, void* y, int y_dtype, int64_t y_ld, int64_t y_rows) {
-  const int64_t es = y_dtype == XVEC_BF16 ? 2 : 4;
+  const int64_t es = elem_bytes(y_dtype);
   p.out = y;
   p.ldo = y_ld;
   p.vec_store = ((reinterpret_cast<uintptr_t>(y) & 15u) == 0 && (y_ld * es) % 16 == 0) ? 1 : 0;
@@ -522,7 +543,7 @@ int gemm_pool(const XvecLayerDesc& l, const void* x, int64_t x_rows, int64_t x_l
   p.row_utt = row_utt;
   p.blk_slot_base = blk_slot_base;
   p.part = part;
-  return launch<EPI_POOL>(l.dtype == XVEC_F32, ta, tb, ty, p, static_cast<cudaStream_t>(stream));
+  return launch<EPI_POOL>(l.dtype, ta, tb, ty, p, static_cast<cudaStream_t>(stream));
 }
 
 int gemm_store(const XvecLayerDesc& l, const void* x, int64_t x_rows, int64_t x_ld, int64_t rows, const float* bn_scale,
@@ -532,12 +553,11 @@ int gemm_store(const XvecLayerDesc& l, const void* x, int64_t x_rows, int64_t x_
   int rc = gemm_setup(l, x, x_rows, x_ld, rows, p, ta, tb, ty);
   if (rc) return rc;
   if (!y) return set_error(XVEC_E_ARG, "null pointer argument");
-  if (y_dtype != XVEC_F32 && y_dtype != XVEC_BF16) return set_error(XVEC_E_ARG, "bad y_dtype %d", y_dtype);
+  if (!valid_dtype(y_dtype)) return set_error(XVEC_E_ARG, "bad y_dtype %d", y_dtype);
   if ((bn_scale == nullptr) != (bn_shift == nullptr)) return set_error(XVEC_E_ARG, "bn_scale and bn_shift must be given together");
   if ((reinterpret_cast<uintptr_t>(l.bias_dev) & 15u) || (reinterpret_cast<uintptr_t>(bn_scale) & 15u) || (reinterpret_cast<uintptr_t>(bn_shift) & 15u))
     return set_error(XVEC_E_ARG, "bias / bn_scale / bn_shift must be 16-byte aligned (and hold ceil(n/32)*32 floats)");
   if (y_ld < l.n) return set_error(XVEC_E_ARG, "y_ld < n");
-  const bool tf32 = l.dtype == XVEC_F32;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int64_t ws_need = splitk_workspace_bytes(rows, l.cin, l.taps, l.n, l.dtype);
   if (ws_need == 0 || !ws || ws_bytes < ws_need || (reinterpret_cast<uintptr_t>(ws) & 15u)) {
@@ -546,7 +566,9 @@ int gemm_store(const XvecLayerDesc& l, const void* x, int64_t x_rows, int64_t x_
     p.relu = relu;
     rc = set_store_output(p, ty, y, y_dtype, y_ld, rows);
     if (rc) return rc;
-    return y_dtype == XVEC_BF16 ? launch<EPI_STORE_BF16>(tf32, ta, tb, ty, p, st) : launch<EPI_STORE_F32>(tf32, ta, tb, ty, p, st);
+    if (y_dtype == XVEC_BF16) return launch<EPI_STORE_BF16>(l.dtype, ta, tb, ty, p, st);
+    if (y_dtype == XVEC_F16) return launch<EPI_STORE_F16>(l.dtype, ta, tb, ty, p, st);
+    return launch<EPI_STORE_F32>(l.dtype, ta, tb, ty, p, st);
   }
   // split-K, step 1: a GEMM with no epilogue; split s of the K loop writes the sums of output row r to workspace row s * rows_pad + r
   splitk_plan(rows, l.n, l.taps * p.cpt, &p.ksplit, &p.kb_per_split);
@@ -554,14 +576,14 @@ int gemm_store(const XvecLayerDesc& l, const void* x, int64_t x_rows, int64_t x_
   const int ws_ld = p.n_tiles * BN;
   rc = set_store_output(p, ty, ws, XVEC_F32, ws_ld, static_cast<int64_t>(p.ksplit) * p.rows_pad);
   if (rc) return rc;
-  rc = launch<EPI_STORE_F32>(tf32, ta, tb, ty, p, st);
+  rc = launch<EPI_STORE_F32>(l.dtype, ta, tb, ty, p, st);
   if (rc) return rc;
   // step 2: the splits summed in fixed order (deterministic), then the caller's epilogue into y
   const long long total = rows * static_cast<long long>(l.n);
   long long blocks = (total + 255) / 256;
   if (blocks > num_sms() * 8LL) blocks = num_sms() * 8LL;
   splitk_reduce_kernel<<<static_cast<unsigned>(blocks), 256, 0, st>>>(static_cast<const float*>(ws), p.ksplit, p.rows, p.rows_pad, l.n, ws_ld,
-                                                                    l.bias_dev, bn_scale, bn_shift, relu, y, y_dtype == XVEC_BF16 ? 1 : 0, y_ld);
+                                                                    l.bias_dev, bn_scale, bn_shift, relu, y, y_dtype, y_ld);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return set_error(XVEC_E_CUDA, "splitk_reduce_kernel launch: %s", cudaGetErrorString(e));
   return XVEC_OK;

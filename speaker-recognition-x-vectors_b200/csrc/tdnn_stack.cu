@@ -25,12 +25,14 @@
 //     dependency resolver, 11 weight-tile producer.  What paces the tensor pipe is the instruction stream of the ONE MMA warp
 //     (512 cycles of tensor work per K step): its loop keeps everything in registers and probes barriers without blocking.
 //
-// TMEM double buffering and the tcgen05 step are the ones of tdnn_gemm.cu.  Layers 1.. run kind::f16 (bf16) or kind::tf32
-// (kAllTf32); layer 0 runs in its own dtype: kind::tf32 on the float32 MFCCs, or kind::f16 on a bf16 copy of them in "window
-// form" (taps = 1, cin = taps*channels over overlapping rows; include/xvec_b200.h).  The last layer is computed TRANSPOSED
-// (weights as the M operand) so that its pooling epilogue reduces over time in registers.
+// TMEM double buffering and the tcgen05 step are the ones of tdnn_gemm.cu.  Layers 1.. run in the activation dtype kAct:
+// kind::f16 with bf16 or f16 operands, or kind::tf32; layer 0 runs in its own dtype: kind::tf32 on the float32 MFCCs, or
+// kind::f16 on a 16-bit copy of them in "window form" (taps = 1, cin = taps*channels over overlapping rows;
+// include/xvec_b200.h).  The last layer is computed TRANSPOSED (weights as the M operand) so that its pooling epilogue reduces
+// over time in registers.
 #include "gemm_tile.cuh"
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 
 #include <mutex>
 #include <type_traits>
@@ -91,7 +93,7 @@ constexpr int STACK_MAX_REGS = 112;
 
 struct StackLayer {
   int n, n_tiles, taps, cpt;  // K loop = taps * cpt chunks of 128 bytes
-  int tf32;                   // operand kind of this layer (1: float32 activations / TF32 math, 0: bf16)
+  int tf32;                   // operand kind of this layer (1: float32 activations / TF32 math, 0: 16-bit, the kernel's kAct)
   int slab_rows;              // 128 + largest tap offset: frame rows one activation slab holds (= the A tensor map's box)
   int n_pad;                  // rows of one K chunk of the chunk-major packed weights (n_tiles * 256)
   int tap_off[XVEC_MAX_TAPS];
@@ -200,10 +202,12 @@ struct TileK {
 };
 static_assert(XVEC_MAX_TAPS <= 8 && XVEC_STACK_MAX_TAP_OFFSET < 16, "tap offsets are packed into 8 x 4 bits");
 
-template <bool kTf32, int kSlots>
+// kDtype: operand element type of the layer (XVEC_F32: kind::tf32; XVEC_BF16 / XVEC_F16: kind::f16 in that format).
+template <int kDtype, int kSlots>
 __device__ __forceinline__ void mma_tile(uint32_t ring_addr, uint32_t full_addr, uint32_t empty_addr, uint32_t d, const TileK k, MmaRing<kSlots>& r,
                                          bool swap_ab, unsigned long long& c_wait, unsigned long long& c_step) {
-  constexpr uint32_t idesc = umma_idesc(kTf32 ? 2u : 1u, BM, BN);
+  constexpr bool kTf32 = kDtype == XVEC_F32;
+  constexpr uint32_t idesc = umma_idesc(umma_format(kDtype), BM, BN);
   const uint64_t desc0 = umma_desc_sw128(ring_addr);  // descriptor of slot 0, row 0
   uint32_t acc = 0;
   for (int ch = 0; ch < k.cpt; ++ch) {
@@ -254,10 +258,11 @@ __device__ __forceinline__ void mma_tile(uint32_t ring_addr, uint32_t full_addr,
 // argument, single-tap layers unroll two chunks, so the descriptor arithmetic of one step is scheduled under the issue of its
 // neighbour.  Same ring protocol and the same MMAs in the same order as mma_tile (which stays for every other tap count).
 // Measured against mma_tile for every layer (B200, 256 x 300, us per launch): 277.0 vs 277.9 in bf16, 509.4 vs 512.0 in TF32.
-template <bool kTf32, int kSlots, int kTaps, bool kSwap>
+template <int kDtype, int kSlots, int kTaps, bool kSwap>
 __device__ __forceinline__ void mma_tile_fixed(uint32_t ring_addr, uint32_t full_addr, uint32_t empty_addr, uint32_t d, const TileK k,
                                                MmaRing<kSlots>& r, unsigned long long& c_wait, unsigned long long& c_step) {
-  constexpr uint32_t idesc = umma_idesc(kTf32 ? 2u : 1u, BM, BN);
+  constexpr bool kTf32 = kDtype == XVEC_F32;
+  constexpr uint32_t idesc = umma_idesc(umma_format(kDtype), BM, BN);
   const uint64_t desc0 = umma_desc_sw128(ring_addr);  // descriptor of slot 0, row 0
   const uint32_t lo0 = static_cast<uint32_t>(desc0), hi = static_cast<uint32_t>(desc0 >> 32);
   const uint32_t elected = elect_one() ? 1u : 0u;  // the same lane issues every MMA and commit of the tile
@@ -314,9 +319,12 @@ static_assert(228 * 1024 - stack_smem_bytes<false>() - 2048 - 2 * 1024 >= STACK_
               228 * 1024 - stack_smem_bytes<true>() - 2048 - 2 * 1024 >= STACK_SMEM_LEFT_FOR_TAIL,
               "the stack kernel must leave room on the SM for the tail kernels of the previous batch");
 
-template <bool kAllTf32>
+// kAct: the activation dtype of layers 1.. (XVEC_F32, XVEC_BF16 or XVEC_F16).  The two 16-bit kinds share everything but the
+// UMMA operand format and the convert of the store epilogue.
+template <int kAct>
 __global__ void __maxnreg__(STACK_MAX_REGS)
 tdnn_stack_kernel(const __grid_constant__ StackMaps maps, const __grid_constant__ StackParams p) {
+  constexpr bool kAllTf32 = kAct == XVEC_F32;
   extern __shared__ uint8_t smem_raw[];
   constexpr int RING_SLOTS = StackCfg<kAllTf32>::SLOTS;
   __shared__ uint64_t full_bar[RING_SLOTS], empty_bar[RING_SLOTS], tfull_bar[2], tempty_bar[2];
@@ -467,23 +475,23 @@ tdnn_stack_kernel(const __grid_constant__ StackMaps maps, const __grid_constant_
         const bool pooled = static_cast<int>(item & 7u) == p.n_layers - 1;  // last layer: transposed accumulator (see the epilogue)
         XVEC_CNT(const long long tk = clock64(); const unsigned long long full0 = c_full, step0 = c_step;)
         const TileK tk_(L);
-        auto run = [&](auto tf_c) {
-          constexpr bool tf = decltype(tf_c)::value;
+        auto run = [&](auto dt_c) {
+          constexpr int dt = decltype(dt_c)::value;  // operand dtype of this layer
           if (tk_.taps == 1) {
-            if (pooled) mma_tile_fixed<tf, RING_SLOTS, 1, true>(ring_addr, full_addr, empty_addr, d, tk_, ring, c_full, c_step);
-            else mma_tile_fixed<tf, RING_SLOTS, 1, false>(ring_addr, full_addr, empty_addr, d, tk_, ring, c_full, c_step);
+            if (pooled) mma_tile_fixed<dt, RING_SLOTS, 1, true>(ring_addr, full_addr, empty_addr, d, tk_, ring, c_full, c_step);
+            else mma_tile_fixed<dt, RING_SLOTS, 1, false>(ring_addr, full_addr, empty_addr, d, tk_, ring, c_full, c_step);
           } else if (tk_.taps == 3) {
-            if (pooled) mma_tile_fixed<tf, RING_SLOTS, 3, true>(ring_addr, full_addr, empty_addr, d, tk_, ring, c_full, c_step);
-            else mma_tile_fixed<tf, RING_SLOTS, 3, false>(ring_addr, full_addr, empty_addr, d, tk_, ring, c_full, c_step);
+            if (pooled) mma_tile_fixed<dt, RING_SLOTS, 3, true>(ring_addr, full_addr, empty_addr, d, tk_, ring, c_full, c_step);
+            else mma_tile_fixed<dt, RING_SLOTS, 3, false>(ring_addr, full_addr, empty_addr, d, tk_, ring, c_full, c_step);
           } else {
-            mma_tile<tf, RING_SLOTS>(ring_addr, full_addr, empty_addr, d, tk_, ring, pooled, c_full, c_step);
+            mma_tile<dt, RING_SLOTS>(ring_addr, full_addr, empty_addr, d, tk_, ring, pooled, c_full, c_step);
           }
         };
         if constexpr (kAllTf32) {
-          run(std::true_type{});
+          run(std::integral_constant<int, XVEC_F32>{});
         } else {
-          if (L.tf32) run(std::true_type{});
-          else run(std::false_type{});
+          if (L.tf32) run(std::integral_constant<int, XVEC_F32>{});
+          else run(std::integral_constant<int, kAct>{});
         }
         XVEC_CNT(if (lane == 0) {  // per layer: whole K loop, explicit operand waits, time inside the fused issue + probe step
           atomicAdd(p.counter + 40 + (item & 7u), static_cast<unsigned>((clock64() - tk) >> 4));
@@ -576,7 +584,7 @@ tdnn_stack_kernel(const __grid_constant__ StackMaps maps, const __grid_constant_
     const int cbeg = ((warp - 2) >> 2) * (BN / 2);  // this warp's half of the tile's columns
     uint8_t* out_stage = epi_smem + (warp - 2) * StackCfg<kAllTf32>::STAGE_BYTES;
     int store_seq = 0;
-    // Store staging: one TMA-store box per tcgen05.ld chunk (32 rows x 32 columns).  bf16: 64-byte rows (SWIZZLE_64B), the warp's
+    // Store staging: one TMA-store box per tcgen05.ld chunk (32 rows x 32 columns).  16-bit: 64-byte rows (SWIZZLE_64B), the warp's
     // 4 KiB hold two boxes, so staging chunk k+1 overlaps the store of chunk k; float32: 128-byte rows, one box.
     constexpr int BOX_W = kAllTf32 ? 128 : 64;                              // bytes per box row
     constexpr int BOX_BYTES = 32 * BOX_W;
@@ -695,10 +703,10 @@ tdnn_stack_kernel(const __grid_constant__ StackMaps maps, const __grid_constant_
 #pragma unroll
             for (int j = 0; j < 4; ++j) {
               uint4 w;
-              w.x = pack_bf16x2_relu(o[8 * j + 0], o[8 * j + 1]);
-              w.y = pack_bf16x2_relu(o[8 * j + 2], o[8 * j + 3]);
-              w.z = pack_bf16x2_relu(o[8 * j + 4], o[8 * j + 5]);
-              w.w = pack_bf16x2_relu(o[8 * j + 6], o[8 * j + 7]);
+              w.x = pack16x2_relu<kAct>(o[8 * j + 0], o[8 * j + 1]);
+              w.y = pack16x2_relu<kAct>(o[8 * j + 2], o[8 * j + 3]);
+              w.z = pack16x2_relu<kAct>(o[8 * j + 4], o[8 * j + 5]);
+              w.w = pack16x2_relu<kAct>(o[8 * j + 6], o[8 * j + 7]);
               *reinterpret_cast<uint4*>(orow + ((j ^ ((lane >> 1) & 3)) << 4)) = w;
             }
           } else {                    // SWIZZLE_128B: piece index ^ address bits [7,10) = row % 8
@@ -828,7 +836,9 @@ XVEC_DEFINE_WATCHDOG_BINDER(bind_watchdog_stack)
 
 bool stack_supported(const XvecLayerDesc* tdnn, int n_tdnn, int64_t rows) {
   if (n_tdnn < 2 || n_tdnn > XVEC_MAX_STACK || rows <= 0 || rows > 0x7fffff00LL) return false;
-  if (tdnn[0].dtype != XVEC_F32 && tdnn[0].dtype != XVEC_BF16) return false;
+  if (!valid_dtype(tdnn[0].dtype) || !valid_dtype(tdnn[1].dtype)) return false;
+  // float16 runs in its own kernel instance: layer 0 is then TF32 or float16 as well, and float16 activations take no bf16 layer 0
+  if ((tdnn[0].dtype == XVEC_F16 || tdnn[1].dtype == XVEC_F16) && tdnn[0].dtype != XVEC_F32 && tdnn[0].dtype != tdnn[1].dtype) return false;
   for (int i = 0; i < n_tdnn; ++i) {
     if (tdnn[i].taps < 1 || tdnn[i].taps > XVEC_MAX_TAPS) return false;
     if (i > 0 && (tdnn[i].dtype != tdnn[1].dtype || tdnn[i].cin != tdnn[i - 1].n)) return false;
@@ -860,7 +870,7 @@ struct StackPlan {
   StackMaps maps;
   StackParams p;
   int grid;
-  bool all_tf32;
+  int act_dtype;   // kernel instance: the dtype of layers 1..
   uint64_t stamp;  // 0 = empty
 };
 constexpr int STACK_PLAN_CACHE = 64;
@@ -870,8 +880,7 @@ static uint64_t g_plan_clock = 0;
 
 static int build_plan(StackPlan& pl, const XvecLayerDesc* tdnn, int n_tdnn, const void* x, int64_t rows, int64_t x_ld, void* act0, void* act1,
                       int64_t act_ld, int band) {
-  pl.all_tf32 = tdnn[1].dtype == XVEC_F32;
-  const int act_dtype = tdnn[1].dtype;
+  const int act_dtype = pl.act_dtype = tdnn[1].dtype;
   StackMaps& maps = pl.maps;
   StackParams& p = pl.p;
   p = StackParams{};
@@ -911,9 +920,9 @@ static int build_plan(StackPlan& pl, const XvecLayerDesc* tdnn, int n_tdnn, cons
     rc = make_weight_tmap(&maps.b[l], d);
     if (rc) return rc;
     if (l + 1 < n_tdnn) {
-      // store boxes: 32 rows x 32 columns (64-byte rows / SWIZZLE_64B for bf16, 128-byte rows / SWIZZLE_128B for float32)
+      // store boxes: 32 rows x 32 columns (64-byte rows / SWIZZLE_64B for 16-bit, 128-byte rows / SWIZZLE_128B for float32)
       rc = make_tmap_2d(&maps.y[l], act[l & 1], act_dtype, static_cast<uint64_t>(d.n), static_cast<uint64_t>(rows),
-                        static_cast<uint64_t>(act_ld), 32, 32, act_dtype == XVEC_BF16 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B);
+                        static_cast<uint64_t>(act_ld), 32, 32, act_dtype == XVEC_F32 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B);
       if (rc) return rc;
       h = act[l & 1];
       h_ld = act_ld;
@@ -964,7 +973,7 @@ int stack_dispatch(const XvecLayerDesc* tdnn, int n_tdnn, const void* x, int64_t
   StackMaps maps;
   StackParams p;
   int grid;
-  bool all_tf32;
+  int act_dtype;
   {
     std::lock_guard<std::mutex> lock(g_plan_mu);
     StackPlan* hit = nullptr;
@@ -987,7 +996,7 @@ int stack_dispatch(const XvecLayerDesc* tdnn, int n_tdnn, const void* x, int64_t
     maps = hit->maps;
     p = hit->p;
     grid = hit->grid;
-    all_tf32 = hit->all_tf32;
+    act_dtype = hit->act_dtype;
   }
   p.counter = static_cast<unsigned*>(ctrl);
   p.ready = reinterpret_cast<unsigned*>(static_cast<char*>(ctrl) + 256);
@@ -1003,9 +1012,11 @@ int stack_dispatch(const XvecLayerDesc* tdnn, int n_tdnn, const void* x, int64_t
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   cudaError_t e = cudaMemsetAsync(ctrl, 0, static_cast<size_t>(stack_ctrl_bytes(rows, n_tdnn)), st);
   if (e != cudaSuccess) return set_error(XVEC_E_CUDA, "cudaMemsetAsync(ctrl): %s", cudaGetErrorString(e));
-  if (all_tf32)
-    return launch_pair<tdnn_stack_kernel<true>>("tdnn_stack_kernel", STACK_THREADS, stack_smem_bytes<true>(), grid, bind_watchdog_stack, st, maps, p);
-  return launch_pair<tdnn_stack_kernel<false>>("tdnn_stack_kernel", STACK_THREADS, stack_smem_bytes<false>(), grid, bind_watchdog_stack, st, maps, p);
+  if (act_dtype == XVEC_F32)
+    return launch_pair<tdnn_stack_kernel<XVEC_F32>>("tdnn_stack_kernel", STACK_THREADS, stack_smem_bytes<true>(), grid, bind_watchdog_stack, st, maps, p);
+  if (act_dtype == XVEC_F16)
+    return launch_pair<tdnn_stack_kernel<XVEC_F16>>("tdnn_stack_kernel", STACK_THREADS, stack_smem_bytes<false>(), grid, bind_watchdog_stack, st, maps, p);
+  return launch_pair<tdnn_stack_kernel<XVEC_BF16>>("tdnn_stack_kernel", STACK_THREADS, stack_smem_bytes<false>(), grid, bind_watchdog_stack, st, maps, p);
 }
 
 }  // namespace xvec

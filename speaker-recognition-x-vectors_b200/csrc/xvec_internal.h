@@ -23,8 +23,12 @@ int num_sms();
 // Driver entry point for tensor-map creation, resolved through the runtime (no link-time libcuda dependency).
 PFN_encodeTiled get_encode_tiled();
 
-// Elements of `dtype` in one 128-byte K chunk of a packed operand: 32 float32 (TF32 math) or 64 bfloat16.
+// Elements of `dtype` in one 128-byte K chunk of a packed operand: 32 float32 (TF32 math) or 64 bfloat16 / float16.
 inline int chunk_elems(int dtype) { return dtype == XVEC_F32 ? 32 : 64; }
+// Bytes per element of XVEC_F32 / XVEC_BF16 / XVEC_F16.
+inline int elem_bytes(int dtype) { return dtype == XVEC_F32 ? 4 : 2; }
+// The element types of activations and packed weights.
+inline bool valid_dtype(int dtype) { return dtype == XVEC_F32 || dtype == XVEC_BF16 || dtype == XVEC_F16; }
 
 // `l` with the given operands and zeros everywhere else (tap slots past `taps`, w_plain_dev); XVEC_E_ARG for bad taps.
 int layer_desc(XvecLayerDesc* l, const void* w_packed, const float* bias, int n, int cin, int taps, int dtype, const int32_t* tap_offsets);

@@ -41,7 +41,8 @@ def pad32(vec: torch.Tensor | None) -> torch.Tensor | None:
 
 
 def pack_weight(weight: torch.Tensor, taps: int, cin: int, dtype: torch.dtype) -> torch.Tensor:
-    """nn.Linear weight (n, taps*cin) float32 -> packed (n_pad, k_pad) operand for xvec_tdnn_layer."""
+    """nn.Linear weight (n, taps*cin) float32 -> packed (n_pad, k_pad) operand for xvec_tdnn_layer, in float32, bfloat16 or
+    float16 (round to nearest)."""
     _require_cuda(weight)
     lib = _lib.load()
     w = weight.detach().to(torch.float32).contiguous()
@@ -58,7 +59,8 @@ def pack_weight(weight: torch.Tensor, taps: int, cin: int, dtype: torch.dtype) -
 def tdnn_layer_flat(x: torch.Tensor, w_packed: torch.Tensor, n: int, offsets, bias=None, bn_scale=None, bn_shift=None,
                     relu: bool = True, out: torch.Tensor | None = None, out_dtype: torch.dtype | None = None, cin: int | None = None,
                     workspace: torch.Tensor | None = None):
-    """y[r] = bn(relu(sum_j W_j x[r + offsets[j]] + bias)) over a flat (rows, cin) frame matrix; returns (rows, n)."""
+    """y[r] = bn(relu(sum_j W_j x[r + offsets[j]] + bias)) over a flat (rows, cin) frame matrix; returns (rows, n).
+    x and w_packed: float32 (TF32 math), bfloat16 or float16; the output dtype is any of the three."""
     _require_cuda(x, w_packed, bias, bn_scale, bn_shift, out)
     lib = _lib.load()
     x_ld = _rowmajor_2d(x, "x")
@@ -236,6 +238,7 @@ def mfcc(wav: torch.Tensor, wav_lengths, normalize: bool = True, out: torch.Tens
 
 
 def cast(src: torch.Tensor, dtype: torch.dtype, out: torch.Tensor | None = None) -> torch.Tensor:
+    """float32 -> float32 / bfloat16 / float16 copy (round to nearest; NaN stays NaN)."""
     _require_cuda(src, out)
     lib = _lib.load()
     if src.dtype != torch.float32:
@@ -301,11 +304,12 @@ def plda_trials(xvecs: torch.Tensor, mean: torch.Tensor, w_phi: torch.Tensor, b_
 def linear_small(x: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor | None = None, relu: bool = False,
                  out_dtype: torch.dtype = torch.float32) -> torch.Tensor:
     """y = act(x W' + bias) with the small-footprint mma.sync kernel (xvec_linear_small): x (rows, k) and weight (n, k)
-    row-major (the nn.Linear layout), both bf16 or both float32 (TF32 math), float32 accumulation; float32 or bf16 result."""
+    row-major (the nn.Linear layout), both bfloat16, both float16 or both float32 (TF32 math), float32 accumulation; float32,
+    bfloat16 or float16 result."""
     _require_cuda(x, weight, bias)
     lib = _lib.load()
     if x.dtype != weight.dtype:
-        raise ValueError("x and weight must share a dtype (bfloat16 or float32)")
+        raise ValueError("x and weight must share a dtype (float32, bfloat16 or float16)")
     x_ld, w_ld = _rowmajor_2d(x, "x"), _rowmajor_2d(weight, "weight")
     if x.shape[1] != weight.shape[1]:
         raise ValueError("x and weight disagree on k")

@@ -74,6 +74,8 @@ class TdnnLayer(nn.Module):
             with torch.cuda.device(hit[1][0].device):
                 torch.cuda.synchronize()
         offs = tap_offsets(self.context)
+        if dtype == torch.float16:
+            check_fp16_range("TdnnLayer", self.linear.weight.detach(), self.linear.bias)
         w = ops.pack_weight(self.linear.weight, len(offs), self.input_size, dtype)
         bias = ops.pad32(self.linear.bias)
         scale = shift = None
@@ -115,7 +117,7 @@ class TdnnLayer(nn.Module):
 
     # ------------------------------------------------------------------ reference surface
     def forward(self, x: torch.Tensor) -> torch.Tensor:
-        """x: (B, T, input_size) CUDA float32 (TF32 tensor-core math) or bfloat16 -> (B, T - (c[-1]-c[0]), output_size)."""
+        """x: (B, T, input_size) CUDA float32 (TF32 tensor-core math), bfloat16 or float16 -> (B, T - (c[-1]-c[0]), output_size)."""
         if x.dim() != 3 or x.shape[2] != self.input_size:
             raise ValueError(f"expected (B, T, {self.input_size}), got {tuple(x.shape)}")
         if not x.is_cuda:
@@ -125,11 +127,23 @@ class TdnnLayer(nn.Module):
         t_out = T - offs[-1]
         if t_out <= 0:
             raise ValueError(f"input of {T} frames is shorter than the context span {offs[-1]}+1")
-        if x.dtype not in (torch.float32, torch.bfloat16):
+        if x.dtype not in (torch.float32, torch.bfloat16, torch.float16):
             x = x.float()
         flat = _aligned_rows(x.reshape(B * T, C))
         y = self.forward_flat(flat)
         return y.view(B, T, self.output_size)[:, :t_out, :]
+
+
+FP16_MAX = 65504.0
+
+
+def check_fp16_range(what: str, weight: torch.Tensor, bias: torch.Tensor | None = None) -> None:
+    """float16 holds magnitudes below 65504: a weight or bias at or beyond that would be stored as inf.  Raise instead of
+    computing with it (float16 has no range scaling here; the "tf32" precision has the float32 range)."""
+    for name, t in (("weight", weight), ("bias", bias)):
+        if t is not None and t.numel() and float(t.detach().abs().max()) >= FP16_MAX:
+            raise ValueError(f"{what}: a {name} of magnitude {float(t.detach().abs().max()):.6g} does not fit float16 (max 65504); "
+                             "use precision \"tf32\"")
 
 
 def _aligned_rows(x2d: torch.Tensor) -> torch.Tensor:

@@ -21,12 +21,15 @@ import torch.nn as nn
 
 from . import _lib, ops
 from .layout import utterance_layout
-from .tdnn_layer import TdnnLayer, _aligned_rows, tap_offsets
+from .tdnn_layer import TdnnLayer, _aligned_rows, check_fp16_range, tap_offsets
 
 # "tf32": float32 storage, tensor-core math in TF32 (10-bit mantissa operands, fp32 accumulate; measured 1e-4 of the row norm
 # against the reference's fp32, bound 1e-3).  "fp32" is kept as an alias for callers that name the reference's dtype
 # (main.py:137 samples.float()); it is the SAME TF32 arithmetic, not IEEE fp32 products.  "bf16": bfloat16 activations/weights.
-PRECISIONS = {"tf32": torch.float32, "fp32": torch.float32, "bf16": torch.bfloat16}
+# "fp16": float16 activations/weights on the same kind::f16 pipe and bytes as bf16, with the 10-bit mantissa of TF32 operands;
+# its range is |x| < 65504: a folded weight or bias outside it is refused when the model is prepared (ValueError), an activation
+# outside it becomes inf and reaches the x-vector as a non-finite value (DESIGN.md section 4).
+PRECISIONS = {"tf32": torch.float32, "fp32": torch.float32, "bf16": torch.bfloat16, "fp16": torch.float16}
 
 
 def _prep_fence(device, drain_all: bool):
@@ -234,6 +237,8 @@ class XVectorModel(nn.Module):
                 b = b + W @ h.repeat(len(offs))
                 W = W * s.repeat(len(offs))[None, :]
             dtype = torch.float32 if i == 0 else self.act_dtype
+            if dtype == torch.float16:
+                check_fp16_range(f"time_context_layers[{i}] with the BatchNorm of layer {i - 1} folded in", W, b)
             out.append((ops.pack_weight(W.float(), len(offs), layer.input_size, dtype), ops.pad32(b.float()), offs))
             prev = layer.bn_affine64()
         last_bn = (None, None) if prev is None else (prev[0].float().contiguous(), prev[1].float().contiguous())
@@ -304,6 +309,8 @@ class XVectorModel(nn.Module):
             return hit[1]
         if hit is not None:
             _prep_fence(lin.weight.device, drain_all=True)
+        if dtype == torch.float16:
+            check_fp16_range(next((n for n, m in self.named_modules() if m is lin), "nn.Linear"), lin.weight, lin.bias)
         w = ops.pack_weight(lin.weight, 1, lin.in_features, dtype)
         b = ops.pad32(lin.bias)
         self._fc_prep[(id(lin), dtype)] = (fp, (w, b))
