@@ -4,6 +4,8 @@ this package accelerates extraction, not training.
 """
 from __future__ import annotations
 
+from operator import attrgetter
+
 import torch
 import torch.nn as nn
 
@@ -40,58 +42,18 @@ class TdnnLayer(nn.Module):
             self.norm = nn.BatchNorm1d(output_size)
         if self.dropout_p:
             self.drop = nn.Dropout(p=self.dropout_p)
-        self._prep = {}
+        self._prep = OperandCache()
 
     # ------------------------------------------------------------------ parameter preparation (cached)
-    def _fingerprint(self):
-        """(identity, in-place version) per parameter / buffer: .to()/.cuda() create new tensors (new identity), load_state_dict
-        and optimiser steps bump the version, replacing a sub-module changes the dicts.  Read straight from the modules'
-        parameter dicts — this runs once per batch and layer, and nn.Module.__getattr__ costs more than the comparison."""
-        mods = self._modules
-        lin = mods["linear"]
-        out = [id(lin)]
-        for t in lin._parameters.values():
-            if t is not None:
-                out.append(id(t))
-                out.append(t._version)
-        if self.batch_norm:
-            norm = mods["norm"]
-            out.append(id(norm))
-            for d in (norm._parameters, norm._buffers):
-                for t in d.values():
-                    if t is not None:
-                        out.append(id(t))
-                        out.append(t._version)
-        return tuple(out)
-
     def prepared(self, dtype: torch.dtype, fold_bn: bool = True):
         """(w_packed, bias, bn_scale, bn_shift) on the parameters' device; re-packed when parameters change."""
-        fp = self._fingerprint()
-        hit = self._prep.get(dtype)
-        if hit is not None and hit[0] == fp:
-            return hit[1]
-        if hit is not None and hit[1][0].is_cuda:  # operands about to be dropped may still be read by kernels in flight
-            with torch.cuda.device(hit[1][0].device):
-                torch.cuda.synchronize()
-        offs = tap_offsets(self.context)
-        if dtype == torch.float16:
-            check_fp16_range("TdnnLayer", self.linear.weight.detach(), self.linear.bias)
-        w = ops.pack_weight(self.linear.weight, len(offs), self.input_size, dtype)
-        bias = ops.pad32(self.linear.bias)
-        scale = shift = None
-        if self.batch_norm:
-            n = self.norm
-            gamma = n.weight.detach().double() if n.weight is not None else torch.ones_like(n.running_var, dtype=torch.float64)
-            beta = n.bias.detach().double() if n.bias is not None else torch.zeros_like(n.running_var, dtype=torch.float64)
-            s = gamma / torch.sqrt(n.running_var.detach().double() + n.eps)
-            scale = ops.pad32(s.float())
-            shift = ops.pad32((beta - n.running_mean.detach().double() * s).float())
-        out = (w, bias, scale, shift)
-        self._prep[dtype] = (fp, out)
-        if w.is_cuda:  # the cached operands may be used from any stream from here on (see xvector._prep_fence)
-            with torch.cuda.device(w.device):
-                torch.cuda.current_stream().synchronize()
-        return out
+        def build():
+            w, bias = pack_checked("TdnnLayer", self.linear.weight, self.linear.bias, len(tap_offsets(self.context)), self.input_size,
+                                   dtype)
+            affine = self.bn_affine64()
+            return (w, bias) + ((None, None) if affine is None else (ops.pad32(affine[0]), ops.pad32(affine[1])))
+
+        return self._prep.get(dtype, param_fingerprint(self), build)
 
     def bn_affine64(self):
         """(scale, shift) of this layer's eval-mode BatchNorm in float64, or None."""
@@ -144,6 +106,61 @@ def check_fp16_range(what: str, weight: torch.Tensor, bias: torch.Tensor | None 
         if t is not None and t.numel() and float(t.detach().abs().max()) >= FP16_MAX:
             raise ValueError(f"{what}: a {name} of magnitude {float(t.detach().abs().max()):.6g} does not fit float16 (max 65504); "
                              "use precision \"tf32\"")
+
+
+def pack_checked(what: str, weight: torch.Tensor, bias: torch.Tensor | None, taps: int, cin: int, dtype: torch.dtype):
+    """(packed weight, padded float32 bias) of one layer; float16 operands are range-checked first (check_fp16_range)."""
+    if dtype == torch.float16:
+        check_fp16_range(what, weight, bias)
+    return ops.pack_weight(weight, taps, cin, dtype), ops.pad32(bias)
+
+
+_version = attrgetter("_version")
+
+
+def param_fingerprint(*modules):
+    """(key, tensors) of every parameter and buffer of `modules` and their sub-modules.  The key holds the identity and in-place
+    version of each tensor: .to()/.cuda() and replacing a sub-module create new tensors, load_state_dict and optimiser steps bump
+    the version.  Ids are only unique among live tensors, so whoever keeps the key keeps the tensors too.  Reads the module dicts
+    directly: this runs once per batch, and nn.Module.__getattr__ costs more than the comparison."""
+    tensors, todo = [], list(modules)
+    for m in todo:  # sub-modules are appended while the list is walked
+        if m is None:
+            continue
+        if params := m._parameters:
+            tensors += params.values()
+        if buffers := m._buffers:
+            tensors += buffers.values()
+        if children := m._modules:
+            todo += children.values()
+    tensors = [t for t in tensors if t is not None]
+    return tuple(map(id, tensors)) + tuple(map(_version, tensors)), tensors
+
+
+class OperandCache:
+    """Kernel operands prepared from module parameters (packed weights, folded BatchNorm), each rebuilt when the parameters it
+    was built from change.  Preparation is enqueued on the current stream, and its results are then read by kernels on other
+    streams (one per pipeline slot) with no event in between; so a build blocks the host until the current stream is done, and
+    stale operands are dropped only once every stream of their device is idle, as kernels in flight may still read them.  Both
+    happen once per parameter change, never per batch."""
+
+    def __init__(self):
+        self._entries = {}
+
+    def get(self, key, fingerprint, build):
+        """The value cached under `key` if it was built at `fingerprint` (param_fingerprint), else build() stored in its place."""
+        fp, tensors = fingerprint
+        old = self._entries.get(key)
+        if old is not None:
+            if old[0] == fp:
+                return old[2]
+            for dev in {t.device for t in old[1] if t.is_cuda}:  # where the parameters the old operands came from live
+                torch.cuda.synchronize(dev)
+        value = build()
+        for dev in {t.device for t in tensors if t.is_cuda}:
+            torch.cuda.current_stream(dev).synchronize()
+        self._entries[key] = (fp, tensors, value)
+        return value
 
 
 def _aligned_rows(x2d: torch.Tensor) -> torch.Tensor:

@@ -21,7 +21,7 @@ import torch.nn as nn
 
 from . import _lib, ops
 from .layout import utterance_layout
-from .tdnn_layer import TdnnLayer, _aligned_rows, check_fp16_range, tap_offsets
+from .tdnn_layer import OperandCache, TdnnLayer, _aligned_rows, pack_checked, param_fingerprint, tap_offsets
 
 # "tf32": float32 storage, tensor-core math in TF32 (10-bit mantissa operands, fp32 accumulate; measured 1e-4 of the row norm
 # against the reference's fp32, bound 1e-3).  "fp32" is kept as an alias for callers that name the reference's dtype
@@ -30,21 +30,6 @@ from .tdnn_layer import TdnnLayer, _aligned_rows, check_fp16_range, tap_offsets
 # its range is |x| < 65504: a folded weight or bias outside it is refused when the model is prepared (ValueError), an activation
 # outside it becomes inf and reaches the x-vector as a non-finite value (DESIGN.md section 4).
 PRECISIONS = {"tf32": torch.float32, "fp32": torch.float32, "bf16": torch.bfloat16, "fp16": torch.float16}
-
-
-def _prep_fence(device, drain_all: bool):
-    """Parameter preparation (float64 BN fold, weight packing, casts) is enqueued on whatever stream is current and its
-    results are cached and then read by kernels on OTHER streams (one per pipeline slot) with no event in between.  Make the
-    hand-over explicit: block the host until the preparing stream is done (drain_all=False, after building), or until every
-    stream of the device is idle (drain_all=True, before dropping operands that kernels in flight may still read).  Runs
-    once per parameter change, never per batch."""
-    if device.type != "cuda":
-        return
-    with torch.cuda.device(device):
-        if drain_all:
-            torch.cuda.synchronize()
-        else:
-            torch.cuda.current_stream().synchronize()
 
 
 class _Layout:
@@ -126,13 +111,19 @@ class _Scratch:
         """Scratch of the segment layers: the hidden (n_utts, width) activation and the split-K workspace."""
         if self.fc_tmp is None or self.fc_tmp.shape[0] < n_utts or self.fc_tmp.shape[1] != width:
             self.fc_tmp = torch.empty((max(n_utts, self.utts_cap), width), dtype=self.act_dtype, device=self.device)
-        key = (n_utts, tuple(fc_shapes))
+        self.splitk_ws(n_utts, fc_shapes)
+
+    def splitk_ws(self, rows, fc_shapes):
+        """The slot's one split-K workspace (None until a shape splits), grown to what any (cin, n) segment shape in fc_shapes
+        needs at `rows` rows: it only ever grows, so it is sized for the largest need seen."""
+        key = (rows, tuple(fc_shapes))
         if self.ws_for != key:
             lib = _lib.load()
-            need = max(lib.xvec_splitk_workspace_bytes(n_utts, cin, 1, n, _lib.dtype_code(self.act_dtype)) for cin, n in fc_shapes)
+            need = max(lib.xvec_splitk_workspace_bytes(rows, cin, 1, n, _lib.dtype_code(self.act_dtype)) for cin, n in fc_shapes)
             if need > 0 and (self.ws is None or self.ws.numel() < need):
                 self.ws = torch.empty(need, dtype=torch.uint8, device=self.device)
             self.ws_for = key
+        return self.ws
 
 
 class XVectorModel(nn.Module):
@@ -160,7 +151,7 @@ class XVectorModel(nn.Module):
         self.precision = precision
         self._layouts: "OrderedDict[tuple, _Layout]" = OrderedDict()
         self._scratch = {}
-        self._fc_prep = {}
+        self._prep = OperandCache()
 
     # ------------------------------------------------------------------ helpers
     @property
@@ -218,13 +209,10 @@ class XVectorModel(nn.Module):
         so each epilogue is just relu(acc + b'); the last layer's BN is folded through the statistics by
         xvec_pool_finalize (mean' = s.mean + h, std' = |s|.std).  Computed once in float64, cached until parameters change.
         Layer 1 reads the float32 MFCCs (TF32 math) in both precisions; the fused pipeline uses its window form (_pipeline)."""
+        return self._prep.get(("stack", self.act_dtype), param_fingerprint(self._modules["time_context_layers"]), self._fold_stack)
+
+    def _fold_stack(self):
         layers = list(self.time_context_layers)
-        fp = tuple(l._fingerprint() for l in layers) + (self.precision,)
-        hit = self._fc_prep.get("stack")
-        if hit is not None and hit[0] == fp:
-            return hit[1]
-        if hit is not None:
-            _prep_fence(self._device(), drain_all=True)  # kernels in flight may still read the operands about to be dropped
         out, prev = [], None
         for i, layer in enumerate(layers):
             layer._check_eval()
@@ -236,30 +224,23 @@ class XVectorModel(nn.Module):
                 s, h = prev
                 b = b + W @ h.repeat(len(offs))
                 W = W * s.repeat(len(offs))[None, :]
-            dtype = torch.float32 if i == 0 else self.act_dtype
-            if dtype == torch.float16:
-                check_fp16_range(f"time_context_layers[{i}] with the BatchNorm of layer {i - 1} folded in", W, b)
-            out.append((ops.pack_weight(W.float(), len(offs), layer.input_size, dtype), ops.pad32(b.float()), offs))
+            what = f"time_context_layers[{i}] with the BatchNorm of layer {i - 1} folded in"
+            out.append((*pack_checked(what, W, b, len(offs), layer.input_size, torch.float32 if i == 0 else self.act_dtype), offs))
             prev = layer.bn_affine64()
         last_bn = (None, None) if prev is None else (prev[0].float().contiguous(), prev[1].float().contiguous())
-        res = (out, last_bn)
-        self._fc_prep["stack"] = (fp, res)
-        _prep_fence(self._device(), drain_all=False)
-        return res
+        return out, last_bn
 
     def _pipeline(self):
         """XvecLayerDesc arrays for xvec_extract_forward (one C call per batch), rebuilt when parameters change."""
         mods = self._modules
-        layers = list(mods["time_context_layers"]._modules.values())
         use7 = self.x_vec_extract_layer == 7
-        fcs = [mods["segment_layer6"], mods["segment_layer7"]] if use7 else [mods["segment_layer6"]]
-        fp = (tuple(l._fingerprint() for l in layers), self.precision, use7,
-              tuple((id(t), t._version) for f in fcs for t in f._parameters.values() if t is not None))
-        hit = self._fc_prep.get("pipeline")
-        if hit is not None and hit[0] == fp:
-            return hit[1]
-        if hit is not None:
-            _prep_fence(self._device(), drain_all=True)
+        fp = param_fingerprint(mods["time_context_layers"], mods["segment_layer6"], mods["segment_layer7"] if use7 else None)
+        return self._prep.get(("pipeline", self.act_dtype, use7), fp, lambda: self._build_pipeline(use7))
+
+    def _build_pipeline(self, use7):
+        layers = list(self.time_context_layers)
+        names = ("segment_layer6", "segment_layer7") if use7 else ("segment_layer6",)
+        fcs = [self._modules[n] for n in names]
         stack, (scale5, shift5) = self._stack_params()
         code = _lib.dtype_code
         tdnn = (_lib.LayerDesc * len(layers))()
@@ -280,9 +261,9 @@ class XVectorModel(nn.Module):
             for j, o in enumerate(offs):
                 d.tap_offsets[j] = o
         fc = (_lib.LayerDesc * len(fcs))()
-        keep = []
-        for i, lin in enumerate(fcs):
-            w, b = self._fc(lin, self.act_dtype)
+        keep = [stack, window]  # the descriptors hold raw pointers: these own what they point to
+        for i, (name, lin) in enumerate(zip(names, fcs)):
+            w, b = self._fc(name, self.act_dtype)
             keep.append((w, b))
             d = fc[i]
             d.w_packed_dev, d.bias_dev = w.data_ptr(), (b.data_ptr() if b is not None else None)
@@ -295,35 +276,23 @@ class XVectorModel(nn.Module):
                 w_plain = w32.clone() if self.act_dtype == torch.float32 else ops.cast(w32, self.act_dtype)
                 keep.append(w_plain)
                 d.w_plain_dev = w_plain.data_ptr()
-        res = {"tdnn": tdnn, "n_tdnn": len(layers), "fc": fc, "n_fc": len(fcs), "keep": (stack, keep, scale5, shift5, window), "window": window,
-               "scale5": scale5, "shift5": shift5, "out_dim": fcs[-1].out_features, "hidden": fcs[0].out_features,
-               "fc_shapes": [(f.in_features, f.out_features) for f in fcs]}
-        self._fc_prep["pipeline"] = (fp, res)
-        _prep_fence(self._device(), drain_all=False)  # every slot's stream may use the operands from here on
-        return res
+        return {"tdnn": tdnn, "n_tdnn": len(layers), "fc": fc, "n_fc": len(fcs), "keep": keep, "window": window,
+                "scale5": scale5, "shift5": shift5, "out_dim": fcs[-1].out_features, "hidden": fcs[0].out_features,
+                "fc_shapes": [(f.in_features, f.out_features) for f in fcs]}
 
-    def _fc(self, lin: nn.Linear, dtype):
-        fp = (id(lin.weight), lin.weight._version, id(lin.bias), lin.bias._version if lin.bias is not None else 0)
-        hit = self._fc_prep.get((id(lin), dtype))
-        if hit is not None and hit[0] == fp:
-            return hit[1]
-        if hit is not None:
-            _prep_fence(lin.weight.device, drain_all=True)
-        if dtype == torch.float16:
-            check_fp16_range(next((n for n, m in self.named_modules() if m is lin), "nn.Linear"), lin.weight, lin.bias)
-        w = ops.pack_weight(lin.weight, 1, lin.in_features, dtype)
-        b = ops.pad32(lin.bias)
-        self._fc_prep[(id(lin), dtype)] = (fp, (w, b))
-        _prep_fence(lin.weight.device, drain_all=False)
-        return w, b
+    def _fc(self, name: str, dtype):
+        """(packed weight, padded bias) of the segment layer `name` (an nn.Linear attribute) in `dtype`."""
+        lin = self._modules[name]
+        return self._prep.get((name, dtype), param_fingerprint(lin),
+                              lambda: pack_checked(name, lin.weight, lin.bias, 1, lin.in_features, dtype))
 
-    def _linear(self, lin: nn.Linear, x2d: torch.Tensor, relu: bool, out_dtype) -> torch.Tensor:
-        w, b = self._fc(lin, x2d.dtype)
-        key = ("ws", x2d.shape[0], lin.in_features, lin.out_features, x2d.dtype, str(x2d.device), _lib.stream_ptr(x2d.device.index))
-        if key not in self._fc_prep:
-            self._fc_prep[key] = ops.splitk_workspace(x2d.shape[0], lin.in_features, 1, lin.out_features, x2d.dtype, x2d.device)
+    def _linear(self, name: str, x2d: torch.Tensor, relu: bool, out_dtype) -> torch.Tensor:
+        """Segment layer `name` on x2d, split-K through slot 0's workspace (forward() runs in slot 0's scratch)."""
+        lin = self._modules[name]
+        w, b = self._fc(name, x2d.dtype)
+        ws = self._scratch_for(0).splitk_ws(x2d.shape[0], ((lin.in_features, lin.out_features),))
         return ops.tdnn_layer_flat(x2d, w, lin.out_features, [0], b, None, None, relu=relu, out_dtype=out_dtype, cin=lin.in_features,
-                                   workspace=self._fc_prep[key])
+                                   workspace=ws)
 
     def _frames_for(self, flat_x: torch.Tensor, pipe) -> torch.Tensor:
         """The frame matrix as layer 1 reads it: 16-byte aligned rows, and DENSE rows (stride == input_size) when layer 1 is in
@@ -382,9 +351,9 @@ class XVectorModel(nn.Module):
     def _head(self, pooled, pooled_lp, layer) -> torch.Tensor:
         a = pooled if pooled_lp is None else pooled_lp
         if layer == 7:  # main.py:88-90
-            h6 = self._linear(self.segment_layer6, a, relu=True, out_dtype=a.dtype)
-            return self._linear(self.segment_layer7, h6, relu=False, out_dtype=torch.float32)
-        return self._linear(self.segment_layer6, a, relu=False, out_dtype=torch.float32)  # 6 and "anything else" (main.py:86-87,91-92)
+            h6 = self._linear("segment_layer6", a, relu=True, out_dtype=a.dtype)
+            return self._linear("segment_layer7", h6, relu=False, out_dtype=torch.float32)
+        return self._linear("segment_layer6", a, relu=False, out_dtype=torch.float32)  # 6 and "anything else" (main.py:86-87,91-92)
 
     def extract_x_vec_flat(self, flat_x: torch.Tensor, lengths, slot: int = 0, out: torch.Tensor | None = None) -> torch.Tensor:
         """Ragged extraction: flat (sum(lengths), input_size) frames -> float32 (len(lengths), x_vector_size).
@@ -410,9 +379,9 @@ class XVectorModel(nn.Module):
         B, T, C = x.shape
         pooled, pooled_lp = self.pooled_stats_flat(x.reshape(B * T, C), [T] * B)
         a = pooled if pooled_lp is None else pooled_lp
-        h = self._linear(self.segment_layer6, a, relu=True, out_dtype=a.dtype)
-        h = self._linear(self.segment_layer7, h, relu=True, out_dtype=a.dtype)
-        return self._linear(self.output, h, relu=False, out_dtype=torch.float32)
+        h = self._linear("segment_layer6", a, relu=True, out_dtype=a.dtype)
+        h = self._linear("segment_layer7", h, relu=True, out_dtype=a.dtype)
+        return self._linear("output", h, relu=False, out_dtype=torch.float32)
 
     def stat_pool(self, x: torch.Tensor) -> torch.Tensor:
         """main.py:59-63: (B, T', P) -> (B, 2P) = [mean over time || unbiased std over time] (standalone HBM-bound kernel)."""

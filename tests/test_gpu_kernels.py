@@ -216,11 +216,12 @@ def test_argument_errors(xb):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("precision", ["bf16", "tf32"])
+@pytest.mark.parametrize("precision", ["tf32", "bf16", "fp16"])
 @pytest.mark.parametrize("band", [0, 5, 7, 1000])
 def test_stack_kernel_equals_per_layer_launches(xb, state_dict, precision, band, monkeypatch):
     """xvec_tdnn_stack (one persistent launch, dynamic tile queue, per-tile dependency flags) must reproduce the per-layer
-    launches bit for bit — same tiles, same K order, same epilogues — for every band height of the work-item order."""
+    launches bit for bit — same tiles, same K order, same epilogues — for every band height of the work-item order, in every
+    precision (layer 1 always reads the float32 frames)."""
     from xvec_b200 import ops
     from oracle import xvector_oracle as ox
     m = xb.XVectorModel(precision=precision)
@@ -231,7 +232,8 @@ def test_stack_kernel_equals_per_layer_launches(xb, state_dict, precision, band,
     flat = torch.cat(utts).cuda()
     lay = m._layout_for(lens)
     pipe = m._pipeline()
-    stack = pipe["keep"][0]
+    assert pipe["tdnn"][0].dtype == xb._lib.F32 and pipe["tdnn"][1].dtype == xb._lib.dtype_code(m.act_dtype)
+    stack = m._stack_params()[0]
     layers = list(m.time_context_layers)
     sc = m._scratch_for(0)
     sc.ensure(lay.rows, lay.n_slots, lay.n_utts)
@@ -262,12 +264,13 @@ def test_stack_kernel_equals_per_layer_launches(xb, state_dict, precision, band,
     assert xb._lib.load().xvec_watchdog_code() == 0
 
 
-def test_stack_kernel_two_launches_in_flight(xb, state_dict, monkeypatch):
+@pytest.mark.parametrize("precision", ["bf16", "fp16"])
+def test_stack_kernel_two_launches_in_flight(xb, state_dict, precision, monkeypatch):
     """Two tdnn_stack_kernel launches on two streams (separate scratch, dynamic tile queues) cannot starve or corrupt each other:
     every result equals the single-launch result bit for bit (tools/stack_stress.py is the long version)."""
     from xvec_b200 import ops
     from oracle import xvector_oracle as ox
-    m = xb.XVectorModel(precision="bf16")
+    m = xb.XVectorModel(precision=precision)
     m.load_state_dict(state_dict)
     m = m.cuda().eval()
     lens = np.random.default_rng(3).integers(15, 900, size=90)
@@ -284,6 +287,8 @@ def test_stack_kernel_two_launches_in_flight(xb, state_dict, monkeypatch):
     streams = [torch.cuda.Stream() for _ in range(2)]
     for band in (0, 7):
         parts = [[torch.zeros_like(ref) for _ in range(4)] for _ in range(2)]
+        for st in streams:  # the zero fills above run on the current stream
+            st.wait_stream(torch.cuda.current_stream())
         for rep in range(4):
             for s in range(2):
                 with torch.cuda.stream(streams[s]):

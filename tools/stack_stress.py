@@ -17,7 +17,7 @@ for precision in ("bf16", "tf32"):
         flat = torch.randn(int(lens.sum()), 24, device="cuda")
         lay = m._layout_for(lens)
         pipe = m._pipeline()
-        stack = pipe["keep"][0]
+        stack = m._stack_params()[0]
         layers = list(m.time_context_layers)
         scs = [m._scratch_for(s) for s in range(2)]
         for sc in scs:

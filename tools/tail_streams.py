@@ -17,6 +17,7 @@ pipe = m._pipeline()
 scs = []
 for s in range(2 * NS):
     sc = m._scratch_for(s); sc.ensure(lay.rows, lay.n_slots, lay.n_utts); sc.ensure_head(lay.n_utts, pipe["fc_shapes"], pipe["hidden"]); scs.append(sc)
+w6, b6 = m._fc("segment_layer6", m.act_dtype)
 main = [torch.cuda.Stream() for _ in range(NS)]
 tail = [torch.cuda.Stream() for _ in range(NS)]
 evs = [[torch.cuda.Event() for _ in range(2)] for _ in range(2 * NS)]
@@ -34,7 +35,8 @@ def step(i, split):
     with torch.cuda.stream(tail[s] if split else main[s]):
         if split: tail[s].wait_event(evs[k][0])
         ops.pool_finalize(part, lay.utt_slot_start, lay.n_pool, 1500, pipe["scale5"], pipe["shift5"], out=pooled, out_lp=pooled_lp)
-        m._head(pooled, pooled_lp, 6)
+        # segment6 split-K through this scratch set's own workspace (model._head uses slot 0's, which both streams would share)
+        ops.tdnn_layer_flat(pooled_lp, w6, 512, [0], b6, None, None, relu=False, out_dtype=torch.float32, cin=3000, workspace=sc.ws)
         if split: evs[k][1].record(tail[s])
 
 for split in (False, True, False, True):
