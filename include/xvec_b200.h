@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define XVEC_ABI_VERSION 8
+#define XVEC_ABI_VERSION 9
 
 #if defined(__GNUC__)
 #define XVEC_API __attribute__((visibility("default")))
@@ -230,6 +230,30 @@ XVEC_API int xvec_extract_forward(const XvecLayerDesc* tdnn_host, int n_tdnn, co
                          float* pooled_dev, void* pooled_lp_dev, const XvecLayerDesc* fc_host, int n_fc, void* fc_tmp_dev,
                          void* splitk_ws_dev, int64_t splitk_ws_bytes, float* out_dev, int64_t out_ld, void* ctrl_dev,
                          int64_t ctrl_bytes, void* stream);
+
+/* x-vectors of windows of recordings (many overlapping windows of a long recording for diarization / segment-level verification)
+ * from ONE pass of the frame-level stack over the recordings, in one call: xvec_tdnn_stack (or one launch per layer, as for
+ * xvec_extract_forward), a finalize over independent slot ranges, then the n_fc segment layers.  Window w of recording k,
+ * frames [a, a + n), gives the x-vector xvec_extract_forward gives for those n frames cut out as an utterance: its pooled rows
+ * are the TDNN-stack output rows a .. a+n-1-lost (lost = sum of the layers' c_last - c_0), and output row r reads input rows
+ * r .. r+lost only, so one pass over the recording computes them with the same bits; only the fp32 summation order of the
+ * pooling differs, through where the rows sit in the 128-row blocks.
+ * replaces: XVectorModel.extract_x_vec (main.py:81-94) applied to mfcc[k, a:a+n] for every window; the reference has no window API.
+ *   Arguments as for xvec_extract_forward, except the finalize layout: the pooled rows are cut at every window's first and
+ *   one-past-last pooled row into disjoint PIECES; pieces are the "utterances" of row_utt_dev / blk_slot_base_dev / part_dev
+ *   (xvec_build_layout takes their first rows, pooled counts and slot prefix; rows no window pools are -1), and window w owns the
+ *   consecutive partial slots [win_slot_lo_dev[w], win_slot_hi_dev[w]) of the pieces it covers.
+ *   win_slot_lo_dev, win_slot_hi_dev, win_n_pool_dev  int32 (n_windows): slot range and pooled-frame count n - lost of each
+ *   window (n - lost == 1 gives a NaN std, like torch.std of one frame);  n_windows >= 1;  pooled_dev / pooled_lp_dev /
+ *   fc_tmp_dev / out_dev hold n_windows rows.  Windows may come in any order and may repeat or nest.  The finalize reads every
+ *   slot of every window: with dense overlap (a 300-frame window every 10 frames) that is ~30 slots per window. */
+XVEC_API int xvec_extract_windows(const XvecLayerDesc* tdnn_host, int n_tdnn, const void* x_dev, int64_t rows, int64_t x_ld,
+                         void* act0_dev, void* act1_dev, int64_t act_ld, const int32_t* row_utt_dev,
+                         const int32_t* blk_slot_base_dev, const int32_t* win_slot_lo_dev, const int32_t* win_slot_hi_dev,
+                         const int32_t* win_n_pool_dev, int n_windows, float* part_dev, const float* bn_last_scale_dev,
+                         const float* bn_last_shift_dev, float* pooled_dev, void* pooled_lp_dev, const XvecLayerDesc* fc_host,
+                         int n_fc, void* fc_tmp_dev, void* splitk_ws_dev, int64_t splitk_ws_bytes, float* out_dev, int64_t out_ld,
+                         void* ctrl_dev, int64_t ctrl_bytes, void* stream);
 
 /* MFCC front end (the step BEFORE the path; SURVEY §8 row f4): waveform -> (frames, 24) float32 rows of the flat frame
  * matrix, with the reference's fixed parameters: 16 kHz, pre-emphasis 0.97, 400-sample frames every 160 samples (zero padded,

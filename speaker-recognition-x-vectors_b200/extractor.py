@@ -15,6 +15,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from .layout import check_windows, window_layout
 
 
 
@@ -41,11 +42,13 @@ class HostExtractor:
         self.h2d_bytes = 0
         self.d2h_bytes = 0
 
-    def reserve(self, max_rows: int, max_utts: int, channels: int) -> None:
+    def reserve(self, max_rows: int, max_utts: int, channels: int, max_slots: int | None = None) -> None:
         """Size the staging buffer, the pinned result buffer and the model scratch of every slot for batches of up to
-        max_rows frames / max_utts utterances (allocation synchronises the device; do it before the pipeline runs)."""
+        max_rows frames / max_utts utterances (or windows) / max_slots pooling partial slots (default: the most max_utts
+        utterances in max_rows frames can have); allocation synchronises the device, so do it before the pipeline runs."""
         dim = (self.model.segment_layer7 if self.model.x_vec_extract_layer == 7 else self.model.segment_layer6).out_features
-        pooled_slots = max_rows // 128 + 2 * max_utts + 2  # partial slots: an utterance of n pooled frames touches <= n/128 + 2 groups
+        # partial slots: an utterance of n pooled frames touches <= n/128 + 2 groups
+        pooled_slots = max_rows // 128 + 2 * max_utts + 2 if max_slots is None else max_slots
         with torch.cuda.device(self.device):
             for i, sl in enumerate(self.slots):
                 if sl.x_dev is None or sl.x_dev.shape[0] < max_rows or sl.x_dev.shape[1] != channels:
@@ -54,11 +57,12 @@ class HostExtractor:
                     sl.out_host = torch.empty((max_utts, dim), dtype=torch.float32, pin_memory=True)
                 self.model._scratch_for(i).ensure(max_rows, pooled_slots, max_utts)
 
-    def submit(self, x_host: torch.Tensor, lengths, out_dev: torch.Tensor | None = None) -> int:
+    def submit(self, x_host: torch.Tensor, lengths, out_dev: torch.Tensor | None = None, windows=None) -> int:
         """Enqueue one batch: x_host is a float32 host tensor (rows, C) or (B, T, C), ideally pinned.  Returns a ticket.
         out_dev: float32 (len(lengths), dim) CUDA tensor that receives the x-vectors ON THE DEVICE instead of the slot's pinned
         host buffer (no device->host copy; result(ticket) then only waits) — for consumers that stay on the GPU (the sharded
-        gather over NCCL, trial scoring)."""
+        gather over NCCL, trial scoring).  windows: (W, 3) (recording, first_frame, n_frames) of the batch's recordings: one
+        x-vector per window (XVectorModel.extract_x_vec_windows) instead of one per recording; out_dev is then (W, dim)."""
         if x_host.is_cuda:
             raise ValueError("HostExtractor.submit takes host tensors; call model.extract_x_vec for device tensors")
         if x_host.dim() == 3:
@@ -71,7 +75,7 @@ class HostExtractor:
         if sl.busy:
             sl.done.synchronize()
         rows, c = x_host.shape
-        n_utts = len(lengths)
+        n_utts = len(lengths) if windows is None else len(windows)
         dim = (self.model.segment_layer7 if self.model.x_vec_extract_layer == 7 else self.model.segment_layer6).out_features
         with _lib.on_device(self.device), torch.cuda.stream(sl.stream):
             if sl.x_dev is None or sl.x_dev.shape[0] < rows or sl.x_dev.shape[1] != c:
@@ -80,7 +84,10 @@ class HostExtractor:
                 sl.out_host = torch.empty((n_utts, dim), dtype=torch.float32, pin_memory=True)
             xd = sl.x_dev[:rows]
             xd.copy_(x_host, non_blocking=True)
-            xv = self.model.extract_x_vec_flat(xd, lengths, slot=i, out=out_dev)
+            if windows is None:
+                xv = self.model.extract_x_vec_flat(xd, lengths, slot=i, out=out_dev)
+            else:
+                xv = self.model.extract_x_vec_windows(xd, lengths, windows, slot=i, out=out_dev)
             if out_dev is None:
                 sl.out_host[:n_utts].copy_(xv, non_blocking=True)
                 self.d2h_bytes += n_utts * dim * 4
@@ -157,6 +164,54 @@ class HostExtractor:
             pending.append((self.submit(flat_host[row0:row1], lengths[lo:hi], None if to_host else out_dev[lo:hi]), lo, hi))
         drain(0)
         return out if to_host else out_dev
+
+    def extract_windows(self, flat_host: torch.Tensor, lengths, windows, max_frames: int = 1 << 17, to_host: bool = True):
+        """x-vectors of windows (recording, first_frame, n_frames) of recordings given as ONE flat host tensor (sum(lengths), C)
+        float32 (pinned for full speed): one pass of the frame-level stack over each recording (XVectorModel.extract_x_vec_windows).
+        Batches are runs of consecutive WHOLE recordings of at most max_frames frames; a longer recording is a batch of its own.
+        Returns float64 numpy (W, dim) in the order of `windows` — or, with to_host=False, a float32 CUDA tensor (W, dim)."""
+        lengths, windows = check_windows(lengths, windows, self.model.lost_frames)
+        if flat_host.dim() != 2 or flat_host.shape[0] != int(lengths.sum()):
+            raise ValueError("flat_host must be (sum(lengths), C)")
+        dim = (self.model.segment_layer7 if self.model.x_vec_extract_layer == 7 else self.model.segment_layer6).out_features
+        order = np.argsort(windows[:, 0], kind="stable")  # the windows of a batch are then one run of `order`
+        sorted_w = windows[order]
+        ends = np.cumsum(lengths)
+        # plan the batches first and size every slot's scratch once for the largest (see extract_flat)
+        plan = []
+        lo, n = 0, len(lengths)
+        while lo < n:
+            row0 = int(ends[lo - 1]) if lo else 0
+            hi = max(lo + 1, min(int(np.searchsorted(ends, row0 + max_frames, side="right")), n))
+            w0, w1 = np.searchsorted(sorted_w[:, 0], [lo, hi], side="left")
+            if w1 > w0:  # recordings without a window are not read at all
+                wins = sorted_w[w0:w1] - np.asarray([lo, 0, 0])
+                wl = window_layout(lengths[lo:hi], wins, self.model.lost_frames)
+                plan.append((lo, hi, row0, int(ends[hi - 1]), int(w0), int(w1), wins, wl.n_slots))
+            lo = hi
+        self.reserve(max(p[3] - p[2] for p in plan), max(p[5] - p[4] for p in plan), flat_host.shape[1],
+                     max_slots=max(p[7] for p in plan))
+        out_sorted = None if to_host else torch.empty((len(windows), dim), dtype=torch.float32, device=self.device)
+        out = np.empty((len(windows), dim), dtype=np.float64) if to_host else None
+        pending = []
+
+        def drain(k):
+            while len(pending) > k:
+                ticket, w0, w1 = pending.pop(0)
+                r = self.result(ticket)
+                if to_host:
+                    out[order[w0:w1]] = r.numpy()
+
+        for lo, hi, row0, row1, w0, w1, wins, _ in plan:
+            drain(len(self.slots) - 1)
+            dst = None if to_host else out_sorted[w0:w1]
+            pending.append((self.submit(flat_host[row0:row1], lengths[lo:hi], dst, windows=wins), w0, w1))
+        drain(0)
+        if to_host:
+            return out
+        res = torch.empty_like(out_sorted)
+        res[torch.from_numpy(order).to(self.device)] = out_sorted
+        return res
 
     def extract_all(self, utts, max_frames: int = 1 << 17, max_utts: int = 1 << 30) -> np.ndarray:
         """Extract a list of host (T_i, C) float32 tensors: concatenated once into a pinned flat buffer, then extract_flat."""

@@ -74,10 +74,108 @@ def utterance_layout(lengths, lost_frames: int = TOTAL_CONTEXT):
     if rows >= 2**31 - 256:
         raise ValueError("batch too large for 32-bit row indices; split it")
     n_pool = lengths - lost_frames
+    slot_start = _slot_prefix(starts, n_pool)
+    return starts.astype(np.int32), n_pool.astype(np.int32), slot_start.astype(np.int32), rows, int(slot_start[-1])
+
+
+def _slot_prefix(starts, n_pool):
+    """Exclusive prefix sum of the partial slots of runs of pooled rows [starts[i], starts[i] + n_pool[i]) (sorted, disjoint):
+    the fused pooling epilogue gives a run one slot per 128-row block it has a row in."""
     blk = _lib.POOL_BLOCK
     cnt = (starts + n_pool - 1) // blk - starts // blk + 1
-    slot_start = np.concatenate(([0], np.cumsum(cnt)))
-    return starts.astype(np.int32), n_pool.astype(np.int32), slot_start.astype(np.int32), rows, int(slot_start[-1])
+    return np.concatenate(([0], np.cumsum(cnt))).astype(np.int64)
+
+
+@dataclass
+class WindowLayout:
+    """Pooling bookkeeping of windows of recordings (window_layout).  Rows are relative to `row0`, the first input row the
+    frame-level stack has to read: rows before the first window's first frame are not passed to it at all."""
+    row0: int                    # first row of the flat recordings matrix that the stack reads
+    rows: int                    # rows the stack reads: [row0, row0 + rows)
+    starts: np.ndarray           # int32 (P) first row (relative to row0) of each piece
+    n_pool: np.ndarray           # int32 (P) pooled rows of each piece
+    slot_start: np.ndarray       # int32 (P+1) partial slots of piece i are [slot_start[i], slot_start[i+1])
+    slot_lo: np.ndarray          # int32 (W) window w reduces the partial slots [slot_lo[w], slot_hi[w])
+    slot_hi: np.ndarray          # int32 (W)
+    win_n_pool: np.ndarray       # int32 (W) pooled frames of each window, n - lost_frames
+    n_slots: int
+
+
+def check_windows(lengths, windows, lost_frames: int = TOTAL_CONTEXT):
+    """(lengths int64 (R), windows int64 (W, 3)) after the checks of window_layout; ValueError for a bad window."""
+    lengths = np.asarray(lengths, dtype=np.int64).reshape(-1)
+    w = np.asarray(windows)
+    if w.ndim != 2 or w.shape[1] != 3 or w.shape[0] < 1:
+        raise ValueError("windows must be a (W >= 1, 3) integer array of (recording, first_frame, n_frames)")
+    if w.dtype.kind not in "iu":
+        raise ValueError("windows must be integers")
+    w = w.astype(np.int64)
+    rec, a, n = w[:, 0], w[:, 1], w[:, 2]
+    if ((rec < 0) | (rec >= lengths.size)).any():
+        raise ValueError(f"window recording index out of range [0, {lengths.size})")
+    if (a < 0).any():
+        raise ValueError("window first_frame must be >= 0")
+    if (n <= lost_frames).any():
+        raise ValueError(f"every window needs more than {lost_frames} frames (the TDNN context); got min {int(n.min())}")
+    if (a + n > lengths[rec]).any():
+        raise ValueError("a window runs past the end of its recording (first_frame + n_frames > length)")
+    return lengths, w
+
+
+def window_layout(lengths, windows, lost_frames: int = TOTAL_CONTEXT) -> WindowLayout:
+    """Pooling layout of windows (recording, first_frame, n_frames) of the recordings of a flat matrix (recording k owns rows
+    [sum(lengths[:k]), sum(lengths[:k+1]))), computed in O(W log W).
+
+    Window [a, a+n) of a recording pools the stack's output rows a .. a+n-1-lost_frames, and output row r reads input rows
+    r .. r+lost_frames only, so ONE pass over the recording yields them.  The pooled rows are cut at every window's first and
+    one-past-last pooled row; the intervals between consecutive cuts that some window covers are the PIECES: disjoint, sorted by
+    row, so the fused pooling epilogue sums each into its own slots exactly as it does utterances (xvec_build_layout takes them as
+    they are).  A window then covers a run of consecutive pieces and with it the contiguous slot range [slot_lo, slot_hi).
+    With windows = the whole recordings in order, starts / n_pool / slot_start equal utterance_layout's."""
+    lengths, w = check_windows(lengths, windows, lost_frames)
+    rec_start = np.concatenate(([0], np.cumsum(lengths)[:-1]))
+    lo = rec_start[w[:, 0]] + w[:, 1]              # first pooled row of each window (absolute)
+    hi = lo + w[:, 2] - lost_frames                # one past its last pooled row
+    row0 = int(lo.min())
+    rows = int((lo + w[:, 2]).max()) - row0        # the last input row any window reads, plus one
+    if rows >= 2**31 - 256:
+        raise ValueError("batch too large for 32-bit row indices; split it")
+    cuts, inv = np.unique(np.concatenate((lo, hi)), return_inverse=True)
+    cover = np.zeros(cuts.size, dtype=np.int64)    # windows covering [cuts[i], cuts[i+1])
+    np.add.at(cover, inv[: lo.size], 1)
+    np.add.at(cover, inv[lo.size:], -1)
+    cover = np.cumsum(cover)[:-1]
+    keep = np.nonzero(cover > 0)[0]                # interval i = [cuts[i], cuts[i+1]) is a piece
+    starts = cuts[keep] - row0
+    n_pool = cuts[keep + 1] - cuts[keep]
+    slot_start = _slot_prefix(starts, n_pool)
+    # first piece of a window: the one starting at its first pooled row; one past its last: the first piece starting at or after hi
+    p_lo = np.searchsorted(starts, lo - row0, side="left")
+    p_hi = np.searchsorted(starts, hi - row0, side="left")
+    i32 = lambda v: np.ascontiguousarray(v, dtype=np.int32)
+    return WindowLayout(row0, rows, i32(starts), i32(n_pool), i32(slot_start), i32(slot_start[p_lo]), i32(slot_start[p_hi]),
+                        i32(w[:, 2] - lost_frames), int(slot_start[-1]))
+
+
+def sliding_windows(lengths, window: int, shift: int) -> np.ndarray:
+    """Windows (recording, first_frame, n_frames) of `window` frames every `shift` frames over each recording, int64 (W, 3), in
+    recording order: starts 0, shift, 2 shift, ... while start + window <= T; when the last of them does not end at T, one more
+    window [T - window, T) so that the end of the recording is covered; a recording shorter than `window` gets one window over
+    all of it."""
+    lengths = np.asarray(lengths, dtype=np.int64).reshape(-1)
+    window, shift = int(window), int(shift)
+    if window < 1 or shift < 1:
+        raise ValueError("window and shift must be positive")
+    out = []
+    for k, t in enumerate(lengths.tolist()):
+        if t <= window:
+            out.append(np.asarray([[k, 0, t]], dtype=np.int64))
+            continue
+        a = np.arange(0, t - window + 1, shift, dtype=np.int64)
+        if a[-1] + window < t:
+            a = np.append(a, t - window)
+        out.append(np.stack((np.full_like(a, k), a, np.full_like(a, window)), axis=1))
+    return np.concatenate(out) if out else np.zeros((0, 3), dtype=np.int64)
 
 
 def lpt_partition(lengths, n_parts: int, lost_frames: int = TOTAL_CONTEXT):

@@ -20,7 +20,7 @@ import torch
 import torch.nn as nn
 
 from . import _lib, ops
-from .layout import utterance_layout
+from .layout import utterance_layout, window_layout
 from .tdnn_layer import OperandCache, TdnnLayer, _aligned_rows, pack_checked, param_fingerprint, tap_offsets
 
 # "tf32": float32 storage, tensor-core math in TF32 (10-bit mantissa operands, fp32 accumulate; measured 1e-4 of the row norm
@@ -33,20 +33,35 @@ PRECISIONS = {"tf32": torch.float32, "fp32": torch.float32, "bf16": torch.bfloat
 
 
 class _Layout:
-    """Device-side pooling bookkeeping of one batch layout (cached by lengths for repeated shapes)."""
+    """Device-side pooling bookkeeping of one batch layout (cached by lengths, and windows, for repeated shapes).
+    Without windows the pooled runs are the utterances and the finalize writes one row per utterance (n_out == n_utts); with
+    windows (layout.window_layout) they are the windows' pieces, the finalize writes one row per window and the stack reads the
+    rows [row0, row0 + rows) of the frame matrix."""
 
-    def __init__(self, lengths, lost_frames, device, staging):
-        starts, n_pool, slot_start, rows, n_slots = utterance_layout(lengths, lost_frames)
+    def __init__(self, lengths, lost_frames, device, staging, windows=None):
+        if windows is None:
+            starts, n_pool, slot_start, rows, n_slots = utterance_layout(lengths, lost_frames)
+            self.row0, fin = 0, ()
+        else:
+            wl = window_layout(lengths, windows, lost_frames)
+            starts, n_pool, slot_start, rows, n_slots = wl.starts, wl.n_pool, wl.slot_start, wl.rows, wl.n_slots
+            self.row0, fin = wl.row0, (wl.slot_lo, wl.slot_hi, wl.win_n_pool)
         self.rows, self.n_slots, self.n_utts = rows, n_slots, int(starts.shape[0])
-        u = self.n_utts
-        host = staging.get(3 * u + 1)  # pinned, reused: one upload of 12 bytes per utterance
-        host[:u] = torch.from_numpy(starts)
-        host[u:2 * u] = torch.from_numpy(n_pool)
-        host[2 * u:3 * u + 1] = torch.from_numpy(slot_start)
-        dev = torch.empty(3 * u + 1, dtype=torch.int32, device=device)
-        dev.copy_(host[: 3 * u + 1], non_blocking=True)
+        self.frames = int(np.sum(lengths))  # rows of the whole frame matrix
+        self.n_out = int(fin[0].shape[0]) if fin else self.n_utts
+        arrays = (starts, n_pool, slot_start) + fin
+        total = sum(int(a.shape[0]) for a in arrays)
+        host = staging.get(total)  # pinned, reused: one upload of 12 bytes per utterance (+ 12 per window)
+        dev = torch.empty(total, dtype=torch.int32, device=device)
+        views, off = [], 0
+        for a in arrays:
+            host[off:off + a.shape[0]] = torch.from_numpy(a)
+            views.append(dev[off:off + a.shape[0]])
+            off += a.shape[0]
+        dev.copy_(host[:total], non_blocking=True)
         staging.mark()
-        self.starts, self.n_pool, self.utt_slot_start = dev[:u], dev[u:2 * u], dev[2 * u:]
+        self.starts, self.n_pool, self.utt_slot_start = views[:3]
+        self.win_slot_lo, self.win_slot_hi, self.win_n_pool = views[3:] if fin else (None, None, None)
         self.row_utt = torch.empty(rows, dtype=torch.int32, device=device)
         self.blk_slot_base = torch.empty(((rows + 255) // 256) * (256 // _lib.POOL_BLOCK), dtype=torch.int32, device=device)
         ops.build_layout_device(self.starts, self.n_pool, self.utt_slot_start, rows, self.row_utt, self.blk_slot_base)
@@ -169,14 +184,17 @@ class XVectorModel(nn.Module):
         if self.training:
             raise RuntimeError("xvec_b200.XVectorModel implements the eval-mode extraction path only; call .eval() first")
 
-    def _layout_for(self, lengths) -> _Layout:
+    def _layout_for(self, lengths, windows=None) -> _Layout:
         lengths = np.asarray(lengths, dtype=np.int64)
         dev = self._device()
-        key = (lengths.tobytes(), dev.index, _lib.stream_ptr(dev.index))
+        if windows is not None:
+            windows = np.ascontiguousarray(windows)
+        key = (lengths.tobytes(), None if windows is None else (windows.shape, windows.dtype.str, windows.tobytes()), dev.index,
+               _lib.stream_ptr(dev.index))
         lay = self._layouts.get(key)
         if lay is None:
             st = self._scratch.setdefault(("pin", str(dev)), _PinnedStaging())  # one ring per device: its buffers are event-guarded
-            lay = _Layout(lengths, self.lost_frames, dev, st)
+            lay = _Layout(lengths, self.lost_frames, dev, st, windows)
             self._layouts[key] = lay
             while len(self._layouts) > 128:
                 self._layouts.popitem(last=False)
@@ -305,38 +323,45 @@ class XVectorModel(nn.Module):
         return x
 
     # ------------------------------------------------------------------ the hot path
-    def _extract_forward(self, flat_x: torch.Tensor, lengths, slot: int, head: bool, out: torch.Tensor | None = None):
-        """ONE C-ABI call (xvec_extract_forward) that enqueues the path on the current stream: the TDNN stack (the persistent
-        stack kernel, or one launch per layer for stacks it does not take) with the pooling partials, the pooling finalize into
-        the slot's scratch and, when `head`, the segment layer(s) into `out` (allocated when None).  Returns (layout, scratch, out)."""
+    def _extract_forward(self, flat_x: torch.Tensor, lengths, slot: int, head: bool, out: torch.Tensor | None = None, windows=None):
+        """ONE C-ABI call (xvec_extract_forward, or xvec_extract_windows with `windows`) that enqueues the path on the current
+        stream: the TDNN stack (the persistent stack kernel, or one launch per layer for stacks it does not take) with the pooling
+        partials, the pooling finalize into the slot's scratch and, when `head`, the segment layer(s) into `out` (allocated when
+        None).  Returns (layout, scratch, out)."""
         self._check_eval()
         if not flat_x.is_cuda:
             raise ValueError("xvec_b200 has no CPU path: move the input (and the model) to a CUDA device")
         if flat_x.dim() != 2 or flat_x.shape[1] != self.input_size:
             raise ValueError(f"expected a flat (rows, {self.input_size}) frame matrix")
-        lay = self._layout_for(lengths)
-        if lay.rows != flat_x.shape[0]:
+        lay = self._layout_for(lengths, windows)
+        if lay.frames != flat_x.shape[0]:
             raise ValueError("sum(lengths) does not match the number of rows")
         pipe = self._pipeline()
         sc = self._scratch_for(slot)
-        sc.ensure(lay.rows, lay.n_slots, lay.n_utts)
+        sc.ensure(lay.rows, lay.n_slots, lay.n_out)
         if flat_x.dtype != torch.float32:
             flat_x = flat_x.float()
+        if lay.rows != lay.frames:  # windows: the stack reads the rows from the first window's first frame to the last one's end
+            flat_x = flat_x[lay.row0: lay.row0 + lay.rows]
         x = self._frames_for(flat_x, pipe)  # layer 1 always reads the float32 frames (TF32 math): no cast pass over the input
         fc, n_fc, fc_tmp, ws = None, 0, None, None
         if head:
-            sc.ensure_head(lay.n_utts, pipe["fc_shapes"], pipe["hidden"])
+            sc.ensure_head(lay.n_out, pipe["fc_shapes"], pipe["hidden"])
             fc, n_fc, fc_tmp, ws = pipe["fc"], pipe["n_fc"], sc.fc_tmp, sc.ws
             if out is None:
-                out = torch.empty((lay.n_utts, pipe["out_dim"]), dtype=torch.float32, device=flat_x.device)
-            elif (out.dtype != torch.float32 or out.device != flat_x.device or out.shape != (lay.n_utts, pipe["out_dim"]) or out.stride(1) != 1):
-                raise ValueError(f"out must be a float32 ({lay.n_utts}, {pipe['out_dim']}) tensor on the input's device with unit column stride")
+                out = torch.empty((lay.n_out, pipe["out_dim"]), dtype=torch.float32, device=flat_x.device)
+            elif (out.dtype != torch.float32 or out.device != flat_x.device or out.shape != (lay.n_out, pipe["out_dim"]) or out.stride(1) != 1):
+                raise ValueError(f"out must be a float32 ({lay.n_out}, {pipe['out_dim']}) tensor on the input's device with unit column stride")
         lib = _lib.load()
         p = _lib.ptr
+        if windows is None:
+            call, fin = lib.xvec_extract_forward, (p(lay.utt_slot_start), p(lay.n_pool), lay.n_utts)
+        else:
+            call, fin = lib.xvec_extract_windows, (p(lay.win_slot_lo), p(lay.win_slot_hi), p(lay.win_n_pool), lay.n_out)
         with _lib.on_device(flat_x.device):
-            _lib.check(lib.xvec_extract_forward(
+            _lib.check(call(
                 pipe["tdnn"], pipe["n_tdnn"], p(x), lay.rows, x.stride(0), p(sc.act[0]), p(sc.act[1]), sc.ld, p(lay.row_utt),
-                p(lay.blk_slot_base), p(lay.utt_slot_start), p(lay.n_pool), lay.n_utts, p(sc.part), p(pipe["scale5"]), p(pipe["shift5"]),
+                p(lay.blk_slot_base), *fin, p(sc.part), p(pipe["scale5"]), p(pipe["shift5"]),
                 p(sc.pooled), p(sc.pooled_lp), fc, n_fc, p(fc_tmp), p(ws), 0 if ws is None else ws.numel(),
                 p(out), 0 if out is None else out.stride(0), p(sc.ctrl), sc.ctrl.numel(), _lib.stream_ptr()))
         return lay, sc, out
@@ -362,6 +387,18 @@ class XVectorModel(nn.Module):
         The whole path is ONE C-ABI call (xvec_extract_forward) that enqueues its kernels on the current stream: the
         persistent TDNN-stack kernel (all five layers + pooling partials), the pooling finalize and the segment layer(s)."""
         return self._extract_forward(flat_x, lengths, slot, head=True, out=out)[2]
+
+    def extract_x_vec_windows(self, flat_x: torch.Tensor, lengths, windows, slot: int = 0, out: torch.Tensor | None = None) -> torch.Tensor:
+        """x-vectors of windows of recordings: flat (sum(lengths), input_size) frames of the recordings -> float32
+        (W, x_vector_size).  windows: int (W, 3) array of (recording, first_frame, n_frames); row w is what extract_x_vec
+        (main.py:81-94) gives for frames [first_frame, first_frame + n_frames) of that recording alone, layer 6 / 7 / other
+        alike.  Windows may come in any order, repeat and nest; n_frames must exceed the model's lost_frames (a window of
+        lost_frames + 1 frames pools one frame: NaN, like torch.std).  layout.sliding_windows makes the usual fixed-length,
+        fixed-shift windows.
+        The frame-level stack runs ONCE over the recordings (from the first window's first frame to the last window's last
+        frame) instead of once per window; only the pooling finalize and the segment layer(s) are per window.  One C-ABI call
+        (xvec_extract_windows) on the current stream; `slot` and `out` as for extract_x_vec_flat."""
+        return self._extract_forward(flat_x, lengths, slot, head=True, out=out, windows=windows)[2]
 
     # ------------------------------------------------------------------ reference surface
     def extract_x_vec(self, x: torch.Tensor) -> torch.Tensor:
