@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define XVEC_ABI_VERSION 9
+#define XVEC_ABI_VERSION 10
 
 #if defined(__GNUC__)
 #define XVEC_API __attribute__((visibility("default")))
@@ -207,50 +207,45 @@ XVEC_API int xvec_linear_small(const void* x_dev, int dtype, int64_t rows, int k
                       const float* bias_dev, int relu, void* y_dev, int y_dtype, int64_t y_ld, void* stream);
 
 /* The whole extraction path for one flat batch in ONE call (3 kernel launches + one small memset enqueued on `stream`; the tensor
- * maps of recurring argument sets are cached): xvec_tdnn_stack, xvec_pool_finalize, then the n_fc segment layers (ReLU between
- * them, none after the last; xvec_linear_small when the layer carries w_plain_dev, else xvec_tdnn_layer with split-K).
- * Without ctrl_dev (NULL) or for a stack xvec_tdnn_stack does not take, the TDNN layers run as one launch each
- * (xvec_tdnn_layer / xvec_tdnn_pool_fused) — same results.
+ * maps of recurring argument sets are cached): xvec_tdnn_stack, the pooling finalize (xvec_pool_finalize over slot ranges), then
+ * the n_fc segment layers (ReLU between them, none after the last; xvec_linear_small when the layer carries w_plain_dev, else
+ * xvec_tdnn_layer with split-K).  Without ctrl_dev (NULL) or for a stack xvec_tdnn_stack does not take, the TDNN layers run as one
+ * launch each (xvec_tdnn_layer / xvec_tdnn_pool_fused) — same results.
  * replaces: XVectorModel.extract_x_vec (main.py:81-94) = time_context_layers (main.py:38-44) + stat_pool (:59-63) +
  * segment_layer6 [+ relu + segment_layer7]; eval-mode BatchNorm of layers 0..n-2 must already be folded into the next
- * layer's packed weights, the last TDNN layer's BatchNorm is passed as bn_last_scale/shift (or NULL).
+ * layer's packed weights, the last TDNN layer's BatchNorm is passed as bn_last_scale/shift (both or neither).
  *   x_dev (rows, tdnn[0].cin) of tdnn[0].dtype, row stride x_ld (window form: see xvec_tdnn_stack);  act0/act1: ping-pong activation buffers (rows, act_ld) of the
- *   dtype of tdnn[1];  layout arrays as for xvec_tdnn_pool_fused / xvec_pool_finalize;  part_dev (n_slots, 2, n_last);
- *   pooled_dev float32 (n_utts, 2 n_last);  pooled_lp_dev NULL or a 16-bit copy of it (n_utts, 2 n_last): in fc[0].dtype when that
+ *   dtype of tdnn[1];  row_utt_dev / blk_slot_base_dev as for xvec_tdnn_pool_fused;  part_dev (n_slots, 2, n_last);
+ *   out_slot_lo_dev, out_slot_hi_dev, out_n_pool_dev  int32 (n_out), n_out >= 1: output row u reduces the partial slots
+ *   [out_slot_lo_dev[u], out_slot_hi_dev[u]) of n = out_n_pool_dev[u] pooled frames (n == 1 gives a NaN std, like torch.std of
+ *   one frame); the ranges are independent and may overlap;
+ *   pooled_dev float32 (n_out, 2 n_last);  pooled_lp_dev NULL or a 16-bit copy of it (n_out, 2 n_last): in fc[0].dtype when that
  *   is XVEC_BF16 or XVEC_F16 (the first segment layer reads it; required then), else in float16 when the TDNN layers are
  *   XVEC_F16, else in bfloat16;  fc: n_fc segment layers (taps == 1);
- *   fc_tmp_dev (n_utts, fc[0].n) of fc[1].dtype when n_fc == 2;  out_dev float32 (n_utts, fc[n_fc-1].n), row stride out_ld;
+ *   fc_tmp_dev (n_out, fc[0].n) of fc[1].dtype when n_fc == 2;  out_dev float32 (n_out, fc[n_fc-1].n), row stride out_ld;
  *   splitk_ws_dev: scratch for the segment layers (see xvec_splitk_workspace_bytes) or NULL;
  *   ctrl_dev / ctrl_bytes: scratch of xvec_tdnn_stack or NULL / 0.
- *   n_fc == 0 ends the call after xvec_pool_finalize; fc_host, fc_tmp_dev, splitk_ws_dev and out_dev may then be NULL. */
+ *   n_fc == 0 ends the call after the finalize; fc_host, fc_tmp_dev, splitk_ws_dev and out_dev may then be NULL.
+ *   Every argument is checked before the first CUDA call.
+ * Utterances: the pooled runs are the utterances (xvec_build_layout of their first rows, pooled counts and slot prefix
+ *   slot_start, n_utts + 1 entries); out_slot_lo_dev = slot_start, out_slot_hi_dev = slot_start + 1 (the same device array, one
+ *   element on), out_n_pool_dev = the pooled counts, n_out = n_utts: one x-vector per utterance.
+ * Windows: x-vectors of windows of recordings (many overlapping windows of a long recording for diarization / segment-level
+ *   verification) from ONE pass of the frame-level stack over the recordings.  Window w of recording k, frames [a, a + n), gives
+ *   the x-vector this call gives for those n frames cut out as an utterance: its pooled rows are the TDNN-stack output rows
+ *   a .. a+n-1-lost (lost = sum of the layers' c_last - c_0), and output row r reads input rows r .. r+lost only, so one pass over
+ *   the recording computes them with the same bits; only the fp32 summation order of the pooling differs, through where the rows
+ *   sit in the 128-row blocks.  The pooled rows are cut at every window's first and one-past-last pooled row into disjoint
+ *   PIECES; pieces are the "utterances" of row_utt_dev / blk_slot_base_dev / part_dev (xvec_build_layout takes their first rows,
+ *   pooled counts and slot prefix; rows no window pools are -1), and window w owns the consecutive partial slots
+ *   [out_slot_lo_dev[w], out_slot_hi_dev[w]) of the pieces it covers, out_n_pool_dev[w] = n - lost, n_out = the number of
+ *   windows.  Windows may come in any order and may repeat or nest.  The finalize reads every slot of every window: with dense
+ *   overlap (a 300-frame window every 10 frames) that is ~30 slots per window.  The reference has no window API: this replaces
+ *   extract_x_vec applied to mfcc[k, a:a+n] for every window. */
 XVEC_API int xvec_extract_forward(const XvecLayerDesc* tdnn_host, int n_tdnn, const void* x_dev, int64_t rows, int64_t x_ld,
                          void* act0_dev, void* act1_dev, int64_t act_ld, const int32_t* row_utt_dev,
-                         const int32_t* blk_slot_base_dev, const int32_t* utt_slot_start_dev, const int32_t* n_pool_dev,
-                         int n_utts, float* part_dev, const float* bn_last_scale_dev, const float* bn_last_shift_dev,
-                         float* pooled_dev, void* pooled_lp_dev, const XvecLayerDesc* fc_host, int n_fc, void* fc_tmp_dev,
-                         void* splitk_ws_dev, int64_t splitk_ws_bytes, float* out_dev, int64_t out_ld, void* ctrl_dev,
-                         int64_t ctrl_bytes, void* stream);
-
-/* x-vectors of windows of recordings (many overlapping windows of a long recording for diarization / segment-level verification)
- * from ONE pass of the frame-level stack over the recordings, in one call: xvec_tdnn_stack (or one launch per layer, as for
- * xvec_extract_forward), a finalize over independent slot ranges, then the n_fc segment layers.  Window w of recording k,
- * frames [a, a + n), gives the x-vector xvec_extract_forward gives for those n frames cut out as an utterance: its pooled rows
- * are the TDNN-stack output rows a .. a+n-1-lost (lost = sum of the layers' c_last - c_0), and output row r reads input rows
- * r .. r+lost only, so one pass over the recording computes them with the same bits; only the fp32 summation order of the
- * pooling differs, through where the rows sit in the 128-row blocks.
- * replaces: XVectorModel.extract_x_vec (main.py:81-94) applied to mfcc[k, a:a+n] for every window; the reference has no window API.
- *   Arguments as for xvec_extract_forward, except the finalize layout: the pooled rows are cut at every window's first and
- *   one-past-last pooled row into disjoint PIECES; pieces are the "utterances" of row_utt_dev / blk_slot_base_dev / part_dev
- *   (xvec_build_layout takes their first rows, pooled counts and slot prefix; rows no window pools are -1), and window w owns the
- *   consecutive partial slots [win_slot_lo_dev[w], win_slot_hi_dev[w]) of the pieces it covers.
- *   win_slot_lo_dev, win_slot_hi_dev, win_n_pool_dev  int32 (n_windows): slot range and pooled-frame count n - lost of each
- *   window (n - lost == 1 gives a NaN std, like torch.std of one frame);  n_windows >= 1;  pooled_dev / pooled_lp_dev /
- *   fc_tmp_dev / out_dev hold n_windows rows.  Windows may come in any order and may repeat or nest.  The finalize reads every
- *   slot of every window: with dense overlap (a 300-frame window every 10 frames) that is ~30 slots per window. */
-XVEC_API int xvec_extract_windows(const XvecLayerDesc* tdnn_host, int n_tdnn, const void* x_dev, int64_t rows, int64_t x_ld,
-                         void* act0_dev, void* act1_dev, int64_t act_ld, const int32_t* row_utt_dev,
-                         const int32_t* blk_slot_base_dev, const int32_t* win_slot_lo_dev, const int32_t* win_slot_hi_dev,
-                         const int32_t* win_n_pool_dev, int n_windows, float* part_dev, const float* bn_last_scale_dev,
+                         const int32_t* blk_slot_base_dev, const int32_t* out_slot_lo_dev, const int32_t* out_slot_hi_dev,
+                         const int32_t* out_n_pool_dev, int n_out, float* part_dev, const float* bn_last_scale_dev,
                          const float* bn_last_shift_dev, float* pooled_dev, void* pooled_lp_dev, const XvecLayerDesc* fc_host,
                          int n_fc, void* fc_tmp_dev, void* splitk_ws_dev, int64_t splitk_ws_bytes, float* out_dev, int64_t out_ld,
                          void* ctrl_dev, int64_t ctrl_bytes, void* stream);

@@ -16,7 +16,7 @@ LIB_PATH = os.environ.get("XVEC_LIB") or os.path.join(HERE, "libxvec_b200.so")  
 F32, BF16, F16 = 0, 1, 2
 E_ARG, E_CUDA, E_DEVICE = -1, -2, -3
 TILE_N, POOL_BLOCK, POOL_CHUNK, MAX_TAPS = 256, 128, 128, 8
-ABI_VERSION = 9
+ABI_VERSION = 10
 MAX_STACK = 6
 STACK_MAX_TAP_OFFSET = 8  # XVEC_STACK_MAX_TAP_OFFSET
 
@@ -47,9 +47,6 @@ _SIGNATURES = {
     "xvec_pool_finalize": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                    c_int, c_int64, c_void_p]),
     "xvec_extract_forward": (c_int, [POINTER(LayerDesc), c_int, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_void_p, c_void_p,
-                                     c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, POINTER(LayerDesc), c_int,
-                                     c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p]),
-    "xvec_extract_windows": (c_int, [POINTER(LayerDesc), c_int, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_void_p, c_void_p,
                                      c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, POINTER(LayerDesc),
                                      c_int, c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p]),
     "xvec_stack_ctrl_bytes": (c_int64, [c_int64, c_int]),

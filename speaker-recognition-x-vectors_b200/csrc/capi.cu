@@ -165,8 +165,8 @@ int xvec_tdnn_stack(const XvecLayerDesc* tdnn, int n_tdnn, const void* x_dev, in
                         ctrl_bytes, band, stream);
 }
 
-// Frame-level stack of xvec_extract_forward / xvec_extract_windows: the persistent stack kernel when given its scratch and the
-// stack fits it, else one launch per layer.
+// Frame-level stack of xvec_extract_forward: the persistent stack kernel when given its scratch and the stack fits it, else one
+// launch per layer.
 static int frame_stack(const XvecLayerDesc* tdnn, int n_tdnn, const void* x, int64_t rows, int64_t x_ld, void* act0, void* act1,
                        int64_t act_ld, const int32_t* row_utt, const int32_t* blk_slot_base, float* part, void* ctrl, int64_t ctrl_bytes,
                        void* stream) {
@@ -184,8 +184,7 @@ static int frame_stack(const XvecLayerDesc* tdnn, int n_tdnn, const void* x, int
   return gemm_pool(tdnn[n_tdnn - 1], h, rows, h_ld, rows, row_utt, blk_slot_base, part, stream);
 }
 
-// Segment head of xvec_extract_forward / xvec_extract_windows: n_fc layers on the pooled statistics `a`, ReLU between them, none
-// after the last.
+// Segment head of xvec_extract_forward: n_fc layers on the pooled statistics `a`, ReLU between them, none after the last.
 static int segment_head(const XvecLayerDesc* fc, int n_fc, const void* a, int64_t a_ld, int n_utts, void* fc_tmp, void* splitk_ws,
                         int64_t splitk_ws_bytes, float* out, int64_t out_ld, void* stream) {
   for (int i = 0; i < n_fc; ++i) {
@@ -208,69 +207,37 @@ static int segment_head(const XvecLayerDesc* fc, int n_fc, const void* a, int64_
   return XVEC_OK;
 }
 
-// Argument checks of xvec_extract_forward / xvec_extract_windows (made before any CUDA call).  On success *lp_head tells whether
-// the first segment layer is 16-bit and reads the pooled statistics in its own dtype, and *lp_dtype is the dtype of the 16-bit copy.
-static int check_extract_args(const XvecLayerDesc* tdnn, int n_tdnn, const void* x_dev, const void* act0_dev, const void* act1_dev,
-                              const float* pooled_dev, const void* pooled_lp_dev, const XvecLayerDesc* fc, int n_fc,
-                              const void* fc_tmp_dev, const float* out_dev, bool* lp_head, int* lp_dtype) {
-  if (!tdnn || n_tdnn < 2 || n_fc < 0 || n_fc > 2 || (n_fc > 0 && !fc))
-    return set_error(XVEC_E_ARG, "need >= 2 TDNN layers and 0 to 2 segment layers");
-  if (!x_dev || !act0_dev || !act1_dev || !pooled_dev || (n_fc > 0 && !out_dev)) return set_error(XVEC_E_ARG, "null pointer argument");
-  if (n_fc == 2 && !fc_tmp_dev) return set_error(XVEC_E_ARG, "fc_tmp_dev is NULL");
-  *lp_head = n_fc > 0 && (fc[0].dtype == XVEC_BF16 || fc[0].dtype == XVEC_F16);
-  if (*lp_head && !pooled_lp_dev) return set_error(XVEC_E_ARG, "pooled_lp_dev is required for 16-bit segment layers");
-  // the 16-bit copy: in the first segment layer's dtype when that reads it, else (n_fc == 0: the caller runs the head itself) in
-  // float16 for a float16 frame stack, else in bfloat16
-  *lp_dtype = *lp_head ? fc[0].dtype : tdnn[n_tdnn - 1].dtype == XVEC_F16 ? XVEC_F16 : XVEC_BF16;
-  return XVEC_OK;
-}
-
 int xvec_extract_forward(const XvecLayerDesc* tdnn, int n_tdnn, const void* x_dev, int64_t rows, int64_t x_ld, void* act0_dev,
                          void* act1_dev, int64_t act_ld, const int32_t* row_utt_dev, const int32_t* blk_slot_base_dev,
-                         const int32_t* utt_slot_start_dev, const int32_t* n_pool_dev, int n_utts, float* part_dev,
-                         const float* bn_last_scale_dev, const float* bn_last_shift_dev, float* pooled_dev, void* pooled_lp_dev,
-                         const XvecLayerDesc* fc, int n_fc, void* fc_tmp_dev, void* splitk_ws_dev, int64_t splitk_ws_bytes,
-                         float* out_dev, int64_t out_ld, void* ctrl_dev, int64_t ctrl_bytes, void* stream) {
-  bool lp_head;
-  int lp_dtype;
-  int rc = check_extract_args(tdnn, n_tdnn, x_dev, act0_dev, act1_dev, pooled_dev, pooled_lp_dev, fc, n_fc, fc_tmp_dev, out_dev, &lp_head,
-                              &lp_dtype);
-  if (rc) return rc;
-  rc = frame_stack(tdnn, n_tdnn, x_dev, rows, x_ld, act0_dev, act1_dev, act_ld, row_utt_dev, blk_slot_base_dev, part_dev, ctrl_dev,
-                   ctrl_bytes, stream);
-  if (rc) return rc;
-  const int64_t pooled_ld = 2 * static_cast<int64_t>(tdnn[n_tdnn - 1].n);
-  rc = xvec_pool_finalize(part_dev, utt_slot_start_dev, n_pool_dev, n_utts, tdnn[n_tdnn - 1].n, bn_last_scale_dev, bn_last_shift_dev, nullptr,
-                          pooled_dev, pooled_lp_dev, lp_dtype, pooled_ld, stream);
-  if (rc) return rc;
-  return segment_head(fc, n_fc, lp_head ? pooled_lp_dev : static_cast<const void*>(pooled_dev), pooled_ld, n_utts, fc_tmp_dev, splitk_ws_dev,
-                      splitk_ws_bytes, out_dev, out_ld, stream);
-}
-
-int xvec_extract_windows(const XvecLayerDesc* tdnn, int n_tdnn, const void* x_dev, int64_t rows, int64_t x_ld, void* act0_dev,
-                         void* act1_dev, int64_t act_ld, const int32_t* row_utt_dev, const int32_t* blk_slot_base_dev,
-                         const int32_t* win_slot_lo_dev, const int32_t* win_slot_hi_dev, const int32_t* win_n_pool_dev, int n_windows,
+                         const int32_t* out_slot_lo_dev, const int32_t* out_slot_hi_dev, const int32_t* out_n_pool_dev, int n_out,
                          float* part_dev, const float* bn_last_scale_dev, const float* bn_last_shift_dev, float* pooled_dev,
                          void* pooled_lp_dev, const XvecLayerDesc* fc, int n_fc, void* fc_tmp_dev, void* splitk_ws_dev,
                          int64_t splitk_ws_bytes, float* out_dev, int64_t out_ld, void* ctrl_dev, int64_t ctrl_bytes, void* stream) {
-  bool lp_head;
-  int lp_dtype;
-  int rc = check_extract_args(tdnn, n_tdnn, x_dev, act0_dev, act1_dev, pooled_dev, pooled_lp_dev, fc, n_fc, fc_tmp_dev, out_dev, &lp_head,
-                              &lp_dtype);
-  if (rc) return rc;
-  if (!win_slot_lo_dev || !win_slot_hi_dev || !win_n_pool_dev) return set_error(XVEC_E_ARG, "null window layout argument");
-  if (n_windows < 1) return set_error(XVEC_E_ARG, "n_windows must be >= 1");
+  // every argument check comes before the first CUDA call
+  if (!tdnn || n_tdnn < 2 || n_fc < 0 || n_fc > 2 || (n_fc > 0 && !fc))
+    return set_error(XVEC_E_ARG, "need >= 2 TDNN layers and 0 to 2 segment layers");
+  if (!x_dev || !act0_dev || !act1_dev || !part_dev || !pooled_dev || (n_fc > 0 && !out_dev))
+    return set_error(XVEC_E_ARG, "null pointer argument");
+  if (n_fc == 2 && !fc_tmp_dev) return set_error(XVEC_E_ARG, "fc_tmp_dev is NULL");
+  if (!out_slot_lo_dev || !out_slot_hi_dev || !out_n_pool_dev) return set_error(XVEC_E_ARG, "null finalize layout argument");
+  if (n_out < 1) return set_error(XVEC_E_ARG, "n_out must be >= 1");
   if ((bn_last_scale_dev == nullptr) != (bn_last_shift_dev == nullptr))
     return set_error(XVEC_E_ARG, "bn_last_scale and bn_last_shift must be given together");
-  rc = frame_stack(tdnn, n_tdnn, x_dev, rows, x_ld, act0_dev, act1_dev, act_ld, row_utt_dev, blk_slot_base_dev, part_dev, ctrl_dev,
-                   ctrl_bytes, stream);
+  const bool lp_head = n_fc > 0 && (fc[0].dtype == XVEC_BF16 || fc[0].dtype == XVEC_F16);
+  if (lp_head && !pooled_lp_dev) return set_error(XVEC_E_ARG, "pooled_lp_dev is required for 16-bit segment layers");
+  // the 16-bit copy: in the first segment layer's dtype when that reads it, else (n_fc == 0: the caller runs the head itself) in
+  // float16 for a float16 frame stack, else in bfloat16
+  const int lp_dtype = lp_head ? fc[0].dtype : tdnn[n_tdnn - 1].dtype == XVEC_F16 ? XVEC_F16 : XVEC_BF16;
+
+  int rc = frame_stack(tdnn, n_tdnn, x_dev, rows, x_ld, act0_dev, act1_dev, act_ld, row_utt_dev, blk_slot_base_dev, part_dev, ctrl_dev,
+                       ctrl_bytes, stream);
   if (rc) return rc;
   const int64_t pooled_ld = 2 * static_cast<int64_t>(tdnn[n_tdnn - 1].n);
-  rc = pool_finalize_ranges(part_dev, win_slot_lo_dev, win_slot_hi_dev, win_n_pool_dev, n_windows, tdnn[n_tdnn - 1].n, bn_last_scale_dev,
-                            bn_last_shift_dev, pooled_dev, pooled_lp_dev, lp_dtype, pooled_ld, stream);
+  rc = pool_finalize(part_dev, out_slot_lo_dev, out_slot_hi_dev, out_n_pool_dev, n_out, tdnn[n_tdnn - 1].n, bn_last_scale_dev,
+                     bn_last_shift_dev, nullptr, pooled_dev, pooled_lp_dev, lp_dtype, pooled_ld, stream);
   if (rc) return rc;
-  return segment_head(fc, n_fc, lp_head ? pooled_lp_dev : static_cast<const void*>(pooled_dev), pooled_ld, n_windows, fc_tmp_dev,
-                      splitk_ws_dev, splitk_ws_bytes, out_dev, out_ld, stream);
+  return segment_head(fc, n_fc, lp_head ? pooled_lp_dev : static_cast<const void*>(pooled_dev), pooled_ld, n_out, fc_tmp_dev, splitk_ws_dev,
+                      splitk_ws_bytes, out_dev, out_ld, stream);
 }
 
 }  // extern "C"

@@ -84,12 +84,10 @@ stats_pool_partial_kernel(const void* __restrict__ x, long long ld, int p, const
   *reinterpret_cast<float4*>(dst + p) = make_float4(q0, q1, q2, q3);
 }
 
-// grid = (n_utts, ceil(p/128)), block = 128: fixed-order float64 reduction of an utterance's partial slots
-// [slot_start[u], slot_start[u+1]).  kRanges: output row u reduces [slot_start[u], slot_hi[u]) instead — independent, possibly
-// overlapping ranges (the windows of xvec_extract_windows), summed in the same order.
-template <bool kRanges>
+// grid = (n_out, ceil(p/128)), block = 128: fixed-order float64 reduction of output row u's partial slots [slot_lo[u], slot_hi[u]).
+// The ranges are independent and may overlap (windows); an utterance's range is [slot_start[u], slot_start[u+1]).
 __global__ void __launch_bounds__(128)
-pool_finalize_kernel(const float* __restrict__ part, const int* __restrict__ slot_start, const int* __restrict__ n_rows, int p,
+pool_finalize_kernel(const float* __restrict__ part, const int* __restrict__ slot_lo, const int* __restrict__ n_rows, int p,
                      const float* __restrict__ scale, const float* __restrict__ shift, const float* __restrict__ pivot,
                      float* __restrict__ out, void* __restrict__ out_lp, int lp_dtype, long long lp_ld, const int* __restrict__ slot_hi) {
   const int u = blockIdx.x;
@@ -102,7 +100,7 @@ pool_finalize_kernel(const float* __restrict__ part, const int* __restrict__ slo
   }
   __syncthreads();
   if (col >= p) return;
-  const int sl0 = slot_start[u], sl1 = kRanges ? slot_hi[u] : slot_start[u + 1];
+  const int sl0 = slot_lo[u], sl1 = slot_hi[u];
   double S = 0.0, Q = 0.0;
   int sl = sl0;
   for (; sl + 4 <= sl1; sl += 4) {  // 8 independent loads in flight, summed in slot order
@@ -315,15 +313,13 @@ static int check_launch(const char* what) {
   return XVEC_OK;
 }
 
-int pool_finalize_ranges(const float* part, const int32_t* slot_lo, const int32_t* slot_hi, const int32_t* n_rows, int n_out, int p,
-                         const float* bn_scale, const float* bn_shift, float* out, void* out_lp, int lp_dtype, int64_t lp_ld,
-                         void* stream) {
-  int rc = device_check();
-  if (rc) return rc;
+int pool_finalize(const float* part, const int32_t* slot_lo, const int32_t* slot_hi, const int32_t* n_rows, int n_out, int p,
+                  const float* bn_scale, const float* bn_shift, const float* pivot, float* out, void* out_lp, int lp_dtype, int64_t lp_ld,
+                  void* stream) {
   dim3 grid(n_out, (p + 127) / 128);
-  pool_finalize_kernel<true><<<grid, 128, 0, static_cast<cudaStream_t>(stream)>>>(part, slot_lo, n_rows, p, bn_scale, bn_shift, nullptr,
-                                                                                  out, out_lp, lp_dtype, lp_ld, slot_hi);
-  return check_launch("pool_finalize_kernel<ranges>");
+  pool_finalize_kernel<<<grid, 128, 0, static_cast<cudaStream_t>(stream)>>>(part, slot_lo, n_rows, p, bn_scale, bn_shift, pivot, out,
+                                                                            out_lp, lp_dtype, lp_ld, slot_hi);
+  return check_launch("pool_finalize_kernel");
 }
 
 }  // namespace xvec
@@ -379,11 +375,8 @@ int xvec_pool_finalize(const float* part_dev, const int32_t* slot_start_dev, con
   if ((bn_scale_dev == nullptr) != (bn_shift_dev == nullptr)) return set_error(XVEC_E_ARG, "bn_scale and bn_shift must be given together");
   if (out_lp_dev && !valid_dtype(out_lp_dtype)) return set_error(XVEC_E_ARG, "bad out_lp_dtype");
   if (out_lp_dev && out_lp_ld < 2 * p) return set_error(XVEC_E_ARG, "out_lp_ld < 2p");
-  dim3 grid(n_utts, (p + 127) / 128);
-  pool_finalize_kernel<false><<<grid, 128, 0, static_cast<cudaStream_t>(stream)>>>(part_dev, slot_start_dev, n_rows_dev, p, bn_scale_dev,
-                                                                                   bn_shift_dev, pivot_dev, out_f32_dev, out_lp_dev,
-                                                                                   out_lp_dtype, out_lp_ld, nullptr);
-  return check_launch("pool_finalize_kernel");
+  return pool_finalize(part_dev, slot_start_dev, slot_start_dev + 1, n_rows_dev, n_utts, p, bn_scale_dev, bn_shift_dev, pivot_dev,
+                       out_f32_dev, out_lp_dev, out_lp_dtype, out_lp_ld, stream);
 }
 
 int xvec_cast(const float* src_dev, int64_t src_ld, void* dst_dev, int dst_dtype, int64_t dst_ld, int64_t rows, int cols, void* stream) {

@@ -50,9 +50,11 @@ bool fc_small_supported(int64_t rows, int k, int n, int64_t x_ld, int64_t w_ld, 
 int fc_small_dispatch(const void* x, int dtype, int64_t rows, int k, int64_t x_ld, const void* w, int n, int64_t w_ld, const float* bias,
                       int relu, void* y, int y_dtype, int64_t y_ld, void* stream);
 int64_t splitk_workspace_bytes(int64_t rows, int cin, int taps, int n, int dtype);
-// pool.cu: the finalize of xvec_pool_finalize over independent slot ranges [slot_lo[w], slot_hi[w]) (xvec_extract_windows), no pivot.
-int pool_finalize_ranges(const float* part, const int32_t* slot_lo, const int32_t* slot_hi, const int32_t* n_rows, int n_out, int p,
-                         const float* bn_scale, const float* bn_shift, float* out, void* out_lp, int lp_dtype, int64_t lp_ld, void* stream);
+// pool.cu: launches the pooling finalize of output rows [0, n_out), row u reducing the partial slots [slot_lo[u], slot_hi[u]); no
+// argument checks (xvec_pool_finalize, xvec_extract_forward make them).
+int pool_finalize(const float* part, const int32_t* slot_lo, const int32_t* slot_hi, const int32_t* n_rows, int n_out, int p,
+                  const float* bn_scale, const float* bn_shift, const float* pivot, float* out, void* out_lp, int lp_dtype, int64_t lp_ld,
+                  void* stream);
 
 // Per-device one-time initialisation (cudaFuncSetAttribute, binding the watchdog word) that is safe when several host threads
 // — one per device or several per device — make their first call at the same time.

@@ -42,11 +42,16 @@ class HostExtractor:
         self.h2d_bytes = 0
         self.d2h_bytes = 0
 
+    @property
+    def _dim(self) -> int:
+        """Width of an x-vector: the output of segment_layer7 (x_vec_extract_layer 7) or segment_layer6."""
+        return (self.model.segment_layer7 if self.model.x_vec_extract_layer == 7 else self.model.segment_layer6).out_features
+
     def reserve(self, max_rows: int, max_utts: int, channels: int, max_slots: int | None = None) -> None:
         """Size the staging buffer, the pinned result buffer and the model scratch of every slot for batches of up to
         max_rows frames / max_utts utterances (or windows) / max_slots pooling partial slots (default: the most max_utts
         utterances in max_rows frames can have); allocation synchronises the device, so do it before the pipeline runs."""
-        dim = (self.model.segment_layer7 if self.model.x_vec_extract_layer == 7 else self.model.segment_layer6).out_features
+        dim = self._dim
         # partial slots: an utterance of n pooled frames touches <= n/128 + 2 groups
         pooled_slots = max_rows // 128 + 2 * max_utts + 2 if max_slots is None else max_slots
         with torch.cuda.device(self.device):
@@ -76,7 +81,7 @@ class HostExtractor:
             sl.done.synchronize()
         rows, c = x_host.shape
         n_utts = len(lengths) if windows is None else len(windows)
-        dim = (self.model.segment_layer7 if self.model.x_vec_extract_layer == 7 else self.model.segment_layer6).out_features
+        dim = self._dim
         with _lib.on_device(self.device), torch.cuda.stream(sl.stream):
             if sl.x_dev is None or sl.x_dev.shape[0] < rows or sl.x_dev.shape[1] != c:
                 sl.x_dev = torch.empty((rows, c), dtype=torch.float32, device=self.device)
@@ -116,54 +121,21 @@ class HostExtractor:
         (sharding.shard_batches: batch boundaries that do not depend on the number of GPUs) instead of the greedy cut;
         out_dev: with to_host=False, the (N, dim) float32 CUDA tensor to fill (e.g. the send buffer of the NCCL gather)."""
         lengths = np.asarray(lengths, dtype=np.int64)
-        if flat_host.dim() != 2 or flat_host.shape[0] != int(lengths.sum()):
-            raise ValueError("flat_host must be (sum(lengths), C)")
-        ends = np.cumsum(lengths)
-        out = None
-        pending = []
-        dim = (self.model.segment_layer7 if self.model.x_vec_extract_layer == 7 else self.model.segment_layer6).out_features
+        n = len(lengths)
         if to_host:
             out_dev = None
-        elif out_dev is None:
-            out_dev = torch.empty((len(lengths), dim), dtype=torch.float32, device=self.device)
-        elif out_dev.shape != (len(lengths), dim) or out_dev.dtype != torch.float32 or out_dev.device != self.device:
-            raise ValueError(f"out_dev must be a float32 ({len(lengths)}, {dim}) tensor on {self.device}")
-
-        def drain(k):
-            nonlocal out
-            while len(pending) > k:
-                ticket, lo, hi = pending.pop(0)
-                r = self.result(ticket)
-                if not to_host:
-                    continue
-                if out is None:
-                    out = np.empty((len(lengths), r.shape[1]), dtype=np.float64)
-                out[lo:hi] = r.numpy()
-
-        # plan the batches first, so that every slot's buffers can be sized once for the largest batch: growing a slot's
-        # scratch in the middle of the run costs a cudaFree + cudaMalloc (device-wide synchronisation) per growth
-        plan = []
-        lo = 0
-        n = len(lengths)
+        elif out_dev is not None and (out_dev.shape != (n, self._dim) or out_dev.dtype != torch.float32 or out_dev.device != self.device):
+            raise ValueError(f"out_dev must be a float32 ({n}, {self._dim}) tensor on {self.device}")
         if batch_sizes is not None:
             if int(np.sum(batch_sizes)) != n or min(int(b) for b in batch_sizes) < 1:
                 raise ValueError("batch_sizes must be positive and sum to the number of utterances")
-            for b in batch_sizes:
-                hi = lo + int(b)
-                plan.append((lo, hi, int(ends[lo - 1]) if lo else 0, int(ends[hi - 1])))
-                lo = hi
-        while lo < n:
-            row0 = int(ends[lo - 1]) if lo else 0
-            hi = int(np.searchsorted(ends, row0 + max_frames, side="right"))
-            hi = max(lo + 1, min(hi, lo + max_utts, n))
-            plan.append((lo, hi, row0, int(ends[hi - 1])))
-            lo = hi
-        self.reserve(max(r1 - r0 for _, _, r0, r1 in plan), max(hi - lo for lo, hi, _, _ in plan), flat_host.shape[1])
-        for lo, hi, row0, row1 in plan:
-            drain(len(self.slots) - 1)
-            pending.append((self.submit(flat_host[row0:row1], lengths[lo:hi], None if to_host else out_dev[lo:hi]), lo, hi))
-        drain(0)
-        return out if to_host else out_dev
+            cuts = np.concatenate(([0], np.cumsum(batch_sizes))).tolist()
+            runs = list(zip(cuts[:-1], cuts[1:]))
+        else:
+            runs = _runs(lengths, max_frames, max_utts)
+        # an utterance of n pooled frames touches <= n/128 + 2 partial slots
+        batches = [(lo, hi, None, lo, hi, int(lengths[lo:hi].sum()) // 128 + 2 * (hi - lo) + 2) for lo, hi in runs]
+        return self._extract(flat_host, lengths, batches, n, to_host, out_dev)
 
     def extract_windows(self, flat_host: torch.Tensor, lengths, windows, max_frames: int = 1 << 17, to_host: bool = True):
         """x-vectors of windows (recording, first_frame, n_frames) of recordings given as ONE flat host tensor (sum(lengths), C)
@@ -171,46 +143,51 @@ class HostExtractor:
         Batches are runs of consecutive WHOLE recordings of at most max_frames frames; a longer recording is a batch of its own.
         Returns float64 numpy (W, dim) in the order of `windows` — or, with to_host=False, a float32 CUDA tensor (W, dim)."""
         lengths, windows = check_windows(lengths, windows, self.model.lost_frames)
-        if flat_host.dim() != 2 or flat_host.shape[0] != int(lengths.sum()):
-            raise ValueError("flat_host must be (sum(lengths), C)")
-        dim = (self.model.segment_layer7 if self.model.x_vec_extract_layer == 7 else self.model.segment_layer6).out_features
         order = np.argsort(windows[:, 0], kind="stable")  # the windows of a batch are then one run of `order`
         sorted_w = windows[order]
-        ends = np.cumsum(lengths)
-        # plan the batches first and size every slot's scratch once for the largest (see extract_flat)
-        plan = []
-        lo, n = 0, len(lengths)
-        while lo < n:
-            row0 = int(ends[lo - 1]) if lo else 0
-            hi = max(lo + 1, min(int(np.searchsorted(ends, row0 + max_frames, side="right")), n))
-            w0, w1 = np.searchsorted(sorted_w[:, 0], [lo, hi], side="left")
+        batches = []
+        for lo, hi in _runs(lengths, max_frames):
+            w0, w1 = (int(i) for i in np.searchsorted(sorted_w[:, 0], [lo, hi], side="left"))
             if w1 > w0:  # recordings without a window are not read at all
                 wins = sorted_w[w0:w1] - np.asarray([lo, 0, 0])
-                wl = window_layout(lengths[lo:hi], wins, self.model.lost_frames)
-                plan.append((lo, hi, row0, int(ends[hi - 1]), int(w0), int(w1), wins, wl.n_slots))
-            lo = hi
-        self.reserve(max(p[3] - p[2] for p in plan), max(p[5] - p[4] for p in plan), flat_host.shape[1],
-                     max_slots=max(p[7] for p in plan))
-        out_sorted = None if to_host else torch.empty((len(windows), dim), dtype=torch.float32, device=self.device)
-        out = np.empty((len(windows), dim), dtype=np.float64) if to_host else None
+                batches.append((lo, hi, wins, w0, w1, window_layout(lengths[lo:hi], wins, self.model.lost_frames).n_slots))
+        return self._extract(flat_host, lengths, batches, len(windows), to_host, None, order)
+
+    def _extract(self, flat_host, lengths, batches, n_out, to_host, out_dev, order=None):
+        """Run `batches` (first and one-past-last recording, windows relative to the batch or None, first and one-past-last output
+        row, partial slots) through the slots and gather the (n_out, dim) result: float64 numpy, or with to_host=False a float32
+        CUDA tensor (out_dev when given).  order: the output row of each batch output row (windows, batched by recording), None
+        for the identity."""
+        if flat_host.dim() != 2 or flat_host.shape[0] != int(lengths.sum()):
+            raise ValueError("flat_host must be (sum(lengths), C)")
+        ends = np.concatenate(([0], np.cumsum(lengths))).tolist()
+        # size every slot's buffers once for the largest batch: growing a slot's scratch in the middle of the run costs a
+        # cudaFree + cudaMalloc (device-wide synchronisation) per growth
+        self.reserve(max(ends[hi] - ends[lo] for lo, hi, *_ in batches), max(o1 - o0 for _, _, _, o0, o1, _ in batches),
+                     flat_host.shape[1], max_slots=max(b[5] for b in batches))
+        out = np.empty((n_out, self._dim), dtype=np.float64) if to_host else None
+        if not to_host and out_dev is None:
+            out_dev = torch.empty((n_out, self._dim), dtype=torch.float32, device=self.device)
         pending = []
 
         def drain(k):
             while len(pending) > k:
-                ticket, w0, w1 = pending.pop(0)
+                ticket, o0, o1 = pending.pop(0)
                 r = self.result(ticket)
                 if to_host:
-                    out[order[w0:w1]] = r.numpy()
+                    out[slice(o0, o1) if order is None else order[o0:o1]] = r.numpy()
 
-        for lo, hi, row0, row1, w0, w1, wins, _ in plan:
+        for lo, hi, wins, o0, o1, _ in batches:
             drain(len(self.slots) - 1)
-            dst = None if to_host else out_sorted[w0:w1]
-            pending.append((self.submit(flat_host[row0:row1], lengths[lo:hi], dst, windows=wins), w0, w1))
+            dst = None if to_host else out_dev[o0:o1]
+            pending.append((self.submit(flat_host[ends[lo]:ends[hi]], lengths[lo:hi], dst, windows=wins), o0, o1))
         drain(0)
         if to_host:
             return out
-        res = torch.empty_like(out_sorted)
-        res[torch.from_numpy(order).to(self.device)] = out_sorted
+        if order is None:
+            return out_dev
+        res = torch.empty_like(out_dev)
+        res[torch.from_numpy(order).to(self.device)] = out_dev
         return res
 
     def extract_all(self, utts, max_frames: int = 1 << 17, max_utts: int = 1 << 30) -> np.ndarray:
@@ -220,3 +197,16 @@ class HostExtractor:
             self._flat = torch.empty((rows, utts[0].shape[1]), dtype=torch.float32, pin_memory=True)
         torch.cat([u.float() if u.dtype != torch.float32 else u for u in utts], out=self._flat[:rows])
         return self.extract_flat(self._flat[:rows], [int(u.shape[0]) for u in utts], max_frames, max_utts)
+
+
+def _runs(lengths, max_frames: int, max_utts: int = 1 << 30):
+    """Batches of consecutive whole recordings (or utterances): [(first, one past last)], each of at most max_frames frames (a
+    longer recording alone) and max_utts recordings."""
+    ends = np.cumsum(lengths)
+    runs, lo, n = [], 0, len(lengths)
+    while lo < n:
+        row0 = int(ends[lo - 1]) if lo else 0
+        hi = max(lo + 1, min(int(np.searchsorted(ends, row0 + max_frames, side="right")), lo + max_utts, n))
+        runs.append((lo, hi))
+        lo = hi
+    return runs

@@ -61,9 +61,10 @@ def build_layout(lengths, lost_frames: int = TOTAL_CONTEXT) -> FrameLayout:
     return FrameLayout(lengths, starts, n_pool.astype(np.int32), rows, row_utt, blk_slot_base, utt_slot_start.astype(np.int32), n_slots)
 
 
-def utterance_layout(lengths, lost_frames: int = TOTAL_CONTEXT):
-    """Per-utterance part of build_layout only (O(#utterances) host work): int32 arrays (starts, n_pool, utt_slot_start),
-    total rows and slots.  The per-row / per-block arrays are expanded from these on the device (xvec_build_layout)."""
+def utterance_layout(lengths, lost_frames: int = TOTAL_CONTEXT) -> WindowLayout:
+    """window_layout of the windows that are the whole utterances, in order, in O(#utterances) host work: the pieces are the
+    utterances and output row u reduces the slots [slot_start[u], slot_start[u+1]), so slot_lo / slot_hi are views of slot_start
+    and win_n_pool is n_pool.  The per-row / per-block arrays are expanded from it on the device (xvec_build_layout)."""
     lengths = np.asarray(lengths, dtype=np.int64).reshape(-1)
     if lengths.size == 0:
         raise ValueError("empty batch")
@@ -73,9 +74,10 @@ def utterance_layout(lengths, lost_frames: int = TOTAL_CONTEXT):
     rows = int(lengths.sum())
     if rows >= 2**31 - 256:
         raise ValueError("batch too large for 32-bit row indices; split it")
-    n_pool = lengths - lost_frames
-    slot_start = _slot_prefix(starts, n_pool)
-    return starts.astype(np.int32), n_pool.astype(np.int32), slot_start.astype(np.int32), rows, int(slot_start[-1])
+    n_pool = (lengths - lost_frames).astype(np.int32)
+    slot_start = _slot_prefix(starts, n_pool).astype(np.int32)
+    return WindowLayout(0, rows, starts.astype(np.int32), n_pool, slot_start, slot_start[:-1], slot_start[1:], n_pool,
+                        int(slot_start[-1]))
 
 
 def _slot_prefix(starts, n_pool):
@@ -88,8 +90,9 @@ def _slot_prefix(starts, n_pool):
 
 @dataclass
 class WindowLayout:
-    """Pooling bookkeeping of windows of recordings (window_layout).  Rows are relative to `row0`, the first input row the
-    frame-level stack has to read: rows before the first window's first frame are not passed to it at all."""
+    """Pooling bookkeeping of windows of recordings (window_layout), utterances being the windows that cover whole recordings
+    (utterance_layout).  Rows are relative to `row0`, the first input row the frame-level stack has to read: rows before the
+    first window's first frame are not passed to it at all."""
     row0: int                    # first row of the flat recordings matrix that the stack reads
     rows: int                    # rows the stack reads: [row0, row0 + rows)
     starts: np.ndarray           # int32 (P) first row (relative to row0) of each piece
@@ -131,7 +134,7 @@ def window_layout(lengths, windows, lost_frames: int = TOTAL_CONTEXT) -> WindowL
     one-past-last pooled row; the intervals between consecutive cuts that some window covers are the PIECES: disjoint, sorted by
     row, so the fused pooling epilogue sums each into its own slots exactly as it does utterances (xvec_build_layout takes them as
     they are).  A window then covers a run of consecutive pieces and with it the contiguous slot range [slot_lo, slot_hi).
-    With windows = the whole recordings in order, starts / n_pool / slot_start equal utterance_layout's."""
+    With windows = the whole recordings in order, the layout is utterance_layout's."""
     lengths, w = check_windows(lengths, windows, lost_frames)
     rec_start = np.concatenate(([0], np.cumsum(lengths)[:-1]))
     lo = rec_start[w[:, 0]] + w[:, 1]              # first pooled row of each window (absolute)

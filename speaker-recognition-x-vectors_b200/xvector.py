@@ -33,38 +33,41 @@ PRECISIONS = {"tf32": torch.float32, "fp32": torch.float32, "bf16": torch.bfloat
 
 
 class _Layout:
-    """Device-side pooling bookkeeping of one batch layout (cached by lengths, and windows, for repeated shapes).
-    Without windows the pooled runs are the utterances and the finalize writes one row per utterance (n_out == n_utts); with
-    windows (layout.window_layout) they are the windows' pieces, the finalize writes one row per window and the stack reads the
-    rows [row0, row0 + rows) of the frame matrix."""
+    """Device copy of a batch's pooling layout (layout.utterance_layout, or layout.window_layout with windows; cached by lengths
+    and windows for repeated shapes).  The stack reads the rows [row0, row0 + rows) of the frame matrix, its pooling epilogue sums
+    the pooled runs (`starts`, `n_pool`: the utterances, or the windows' pieces) into partial slots, and the finalize writes output
+    row u (an utterance, or a window) from the slots [slot_lo[u], slot_hi[u])."""
 
-    def __init__(self, lengths, lost_frames, device, staging, windows=None):
-        if windows is None:
-            starts, n_pool, slot_start, rows, n_slots = utterance_layout(lengths, lost_frames)
-            self.row0, fin = 0, ()
+    def __init__(self, wl, frames, device, staging):
+        self.row0, self.rows, self.n_slots, self.n_utts = wl.row0, wl.rows, wl.n_slots, int(wl.starts.shape[0])
+        self.frames = frames  # rows of the whole frame matrix
+        self.n_out = int(wl.slot_lo.shape[0])
+        (self.starts, self.n_pool, self.utt_slot_start, self.slot_lo, self.slot_hi, self.out_n_pool) = _upload(
+            (wl.starts, wl.n_pool, wl.slot_start, wl.slot_lo, wl.slot_hi, wl.win_n_pool), device, staging)
+        self.row_utt = torch.empty(self.rows, dtype=torch.int32, device=device)
+        self.blk_slot_base = torch.empty(((self.rows + 255) // 256) * (256 // _lib.POOL_BLOCK), dtype=torch.int32, device=device)
+        ops.build_layout_device(self.starts, self.n_pool, self.utt_slot_start, self.rows, self.row_utt, self.blk_slot_base)
+
+
+def _upload(arrays, device, staging):
+    """Device copies of 1-D int32 host arrays from ONE pinned upload.  An array that is a view of an earlier one (utterance_layout's
+    slot_lo / slot_hi are slot_start[:-1] / slot_start[1:], its win_n_pool is n_pool) becomes the same view of that array's device
+    copy and adds no bytes."""
+    host = staging.get(sum(int(a.shape[0]) for a in arrays))
+    addr = lambda a: a.__array_interface__["data"][0]
+    place, total = [], 0  # element offset of each array in the upload
+    for i, a in enumerate(arrays):
+        j = next((j for j in range(i) if a is arrays[j] or a.base is arrays[j]), None)
+        if j is None:
+            host[total:total + a.shape[0]] = torch.from_numpy(a)
+            place.append(total)
+            total += a.shape[0]
         else:
-            wl = window_layout(lengths, windows, lost_frames)
-            starts, n_pool, slot_start, rows, n_slots = wl.starts, wl.n_pool, wl.slot_start, wl.rows, wl.n_slots
-            self.row0, fin = wl.row0, (wl.slot_lo, wl.slot_hi, wl.win_n_pool)
-        self.rows, self.n_slots, self.n_utts = rows, n_slots, int(starts.shape[0])
-        self.frames = int(np.sum(lengths))  # rows of the whole frame matrix
-        self.n_out = int(fin[0].shape[0]) if fin else self.n_utts
-        arrays = (starts, n_pool, slot_start) + fin
-        total = sum(int(a.shape[0]) for a in arrays)
-        host = staging.get(total)  # pinned, reused: one upload of 12 bytes per utterance (+ 12 per window)
-        dev = torch.empty(total, dtype=torch.int32, device=device)
-        views, off = [], 0
-        for a in arrays:
-            host[off:off + a.shape[0]] = torch.from_numpy(a)
-            views.append(dev[off:off + a.shape[0]])
-            off += a.shape[0]
-        dev.copy_(host[:total], non_blocking=True)
-        staging.mark()
-        self.starts, self.n_pool, self.utt_slot_start = views[:3]
-        self.win_slot_lo, self.win_slot_hi, self.win_n_pool = views[3:] if fin else (None, None, None)
-        self.row_utt = torch.empty(rows, dtype=torch.int32, device=device)
-        self.blk_slot_base = torch.empty(((rows + 255) // 256) * (256 // _lib.POOL_BLOCK), dtype=torch.int32, device=device)
-        ops.build_layout_device(self.starts, self.n_pool, self.utt_slot_start, rows, self.row_utt, self.blk_slot_base)
+            place.append(place[j] + (addr(a) - addr(arrays[j])) // a.itemsize)
+    dev = torch.empty(total, dtype=torch.int32, device=device)
+    dev.copy_(host[:total], non_blocking=True)
+    staging.mark()
+    return [dev[o:o + a.shape[0]] for a, o in zip(arrays, place)]
 
 
 class _PinnedStaging:
@@ -194,7 +197,9 @@ class XVectorModel(nn.Module):
         lay = self._layouts.get(key)
         if lay is None:
             st = self._scratch.setdefault(("pin", str(dev)), _PinnedStaging())  # one ring per device: its buffers are event-guarded
-            lay = _Layout(lengths, self.lost_frames, dev, st, windows)
+            wl = (utterance_layout(lengths, self.lost_frames) if windows is None
+                  else window_layout(lengths, windows, self.lost_frames))
+            lay = _Layout(wl, int(lengths.sum()), dev, st)
             self._layouts[key] = lay
             while len(self._layouts) > 128:
                 self._layouts.popitem(last=False)
@@ -324,7 +329,7 @@ class XVectorModel(nn.Module):
 
     # ------------------------------------------------------------------ the hot path
     def _extract_forward(self, flat_x: torch.Tensor, lengths, slot: int, head: bool, out: torch.Tensor | None = None, windows=None):
-        """ONE C-ABI call (xvec_extract_forward, or xvec_extract_windows with `windows`) that enqueues the path on the current
+        """ONE C-ABI call (xvec_extract_forward) that enqueues the path on the current
         stream: the TDNN stack (the persistent stack kernel, or one launch per layer for stacks it does not take) with the pooling
         partials, the pooling finalize into the slot's scratch and, when `head`, the segment layer(s) into `out` (allocated when
         None).  Returns (layout, scratch, out)."""
@@ -352,16 +357,11 @@ class XVectorModel(nn.Module):
                 out = torch.empty((lay.n_out, pipe["out_dim"]), dtype=torch.float32, device=flat_x.device)
             elif (out.dtype != torch.float32 or out.device != flat_x.device or out.shape != (lay.n_out, pipe["out_dim"]) or out.stride(1) != 1):
                 raise ValueError(f"out must be a float32 ({lay.n_out}, {pipe['out_dim']}) tensor on the input's device with unit column stride")
-        lib = _lib.load()
         p = _lib.ptr
-        if windows is None:
-            call, fin = lib.xvec_extract_forward, (p(lay.utt_slot_start), p(lay.n_pool), lay.n_utts)
-        else:
-            call, fin = lib.xvec_extract_windows, (p(lay.win_slot_lo), p(lay.win_slot_hi), p(lay.win_n_pool), lay.n_out)
         with _lib.on_device(flat_x.device):
-            _lib.check(call(
+            _lib.check(_lib.load().xvec_extract_forward(
                 pipe["tdnn"], pipe["n_tdnn"], p(x), lay.rows, x.stride(0), p(sc.act[0]), p(sc.act[1]), sc.ld, p(lay.row_utt),
-                p(lay.blk_slot_base), *fin, p(sc.part), p(pipe["scale5"]), p(pipe["shift5"]),
+                p(lay.blk_slot_base), p(lay.slot_lo), p(lay.slot_hi), p(lay.out_n_pool), lay.n_out, p(sc.part), p(pipe["scale5"]), p(pipe["shift5"]),
                 p(sc.pooled), p(sc.pooled_lp), fc, n_fc, p(fc_tmp), p(ws), 0 if ws is None else ws.numel(),
                 p(out), 0 if out is None else out.stride(0), p(sc.ctrl), sc.ctrl.numel(), _lib.stream_ptr()))
         return lay, sc, out
@@ -371,7 +371,7 @@ class XVectorModel(nn.Module):
         Returns (pooled float32 (U, 3000), same in the activation dtype or None).  The returned tensors are scratch of
         the (lengths, slot) plan: they are overwritten by the next call with the same lengths and slot."""
         lay, sc, _ = self._extract_forward(flat_x, lengths, slot, head=False)
-        return sc.pooled[: lay.n_utts], None if sc.pooled_lp is None else sc.pooled_lp[: lay.n_utts]
+        return sc.pooled[: lay.n_out], None if sc.pooled_lp is None else sc.pooled_lp[: lay.n_out]
 
     def _head(self, pooled, pooled_lp, layer) -> torch.Tensor:
         a = pooled if pooled_lp is None else pooled_lp
@@ -397,7 +397,7 @@ class XVectorModel(nn.Module):
         fixed-shift windows.
         The frame-level stack runs ONCE over the recordings (from the first window's first frame to the last window's last
         frame) instead of once per window; only the pooling finalize and the segment layer(s) are per window.  One C-ABI call
-        (xvec_extract_windows) on the current stream; `slot` and `out` as for extract_x_vec_flat."""
+        (xvec_extract_forward) on the current stream; `slot` and `out` as for extract_x_vec_flat."""
         return self._extract_forward(flat_x, lengths, slot, head=True, out=out, windows=windows)[2]
 
     # ------------------------------------------------------------------ reference surface

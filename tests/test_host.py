@@ -55,9 +55,10 @@ def test_fails_loudly_without_gpu():
         m.stat_pool(torch.randn(2, 40, 1500))
 
 
-def test_extract_forward_segment_layer_count():
-    """xvec_extract_forward takes 0 to 2 segment layers.  Its arguments are checked before any CUDA call, so this needs no
-    device: 3 layers are rejected; 0 layers with NULL fc_host / out_dev pass the checks and fail only at the missing device."""
+def test_extract_forward_rejects_bad_arguments_without_a_device():
+    """xvec_extract_forward takes 0 to 2 segment layers and a finalize layout in ranges form.  Its arguments are checked before any
+    CUDA call, so this needs no device; well-formed arguments (0 segment layers with NULL fc_host / out_dev among them) pass the
+    checks and fail only at the missing device."""
     lib = xvec_b200._lib.load()
     tdnn = (xvec_b200._lib.LayerDesc * 2)()
     for d in tdnn:
@@ -65,13 +66,18 @@ def test_extract_forward_segment_layer_count():
     fc = (xvec_b200._lib.LayerDesc * 3)()
     buf = 256  # stands for device pointers; nothing is dereferenced on these paths
 
-    def call(fc_host, n_fc, out):
-        return lib.xvec_extract_forward(tdnn, 2, buf, 300, 256, buf, buf, 256, buf, buf, buf, buf, 1, buf, None, None, buf, None,
-                                        fc_host, n_fc, buf, None, 0, out, 256, None, 0, None)
+    def call(lo=buf, hi=buf, npool=buf, n_out=4, fc_host=fc, n_fc=1, out=buf, shift=None):
+        return lib.xvec_extract_forward(tdnn, 2, buf, 300, 256, buf, buf, 256, buf, buf, lo, hi, npool, n_out, buf, None, shift,
+                                        buf, None, fc_host, n_fc, buf, None, 0, out, 256, None, 0, None)
 
-    assert call(fc, 3, buf) == xvec_b200._lib.E_ARG
+    E = xvec_b200._lib.E_ARG
+    assert call(n_fc=3) == E
+    assert call(lo=None) == E and call(hi=None) == E and call(npool=None) == E
+    assert call(n_out=0) == E and call(n_out=-1) == E
+    assert call(out=None) == E
+    assert call(shift=buf) == E  # BN shift without scale
     if lib.xvec_device_check() != 0:  # no usable device: the call gets as far as the first CUDA call and reports its error
-        assert call(None, 0, None) == lib.xvec_device_check() != xvec_b200._lib.E_ARG
+        assert call(fc_host=None, n_fc=0, out=None) == lib.xvec_device_check() != E
 
 
 def _emulate_fused_pool(lay, r):

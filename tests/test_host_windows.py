@@ -1,6 +1,8 @@
 """CPU tests of windowed extraction (x-vectors of windows of recordings from one pass of the frame-level stack): the piece layout
-of layout.window_layout, a numpy restatement of the fused pooling epilogue + the ranges finalize on it, sliding_windows, the
-validation, and the argument checks of xvec_extract_windows (made before any CUDA call)."""
+of layout.window_layout, a numpy restatement of the fused pooling epilogue + the ranges finalize on it, sliding_windows and the
+validation."""
+import dataclasses
+
 import numpy as np
 import pytest
 
@@ -125,15 +127,23 @@ def test_epilogue_and_ranges_finalize_equal_direct_window_statistics(seed, late)
             assert np.isnan(got[i, 6:]).all()  # one pooled frame: NaN, like torch.std
 
 
-@pytest.mark.parametrize("lengths", [[300, 45, 1000, 15], [15], [128, 129, 256, 257]])
+@pytest.mark.parametrize("lengths", [[300, 45, 1000, 15], [15], [128, 129, 256, 257],
+                                     [142, 142, 142],    # 128 pooled rows each, starting off block boundaries
+                                     [16] * 20,          # two pooled rows each, many utterances per 128-row block
+                                     [141, 15, 142],     # 127, 1 and 128 pooled rows: a one-frame utterance between block edges
+                                     [5000, 15, 300]])   # one utterance spanning 39 blocks
 def test_whole_recording_windows_equal_the_utterance_layout(lengths):
     w = np.stack([np.arange(len(lengths)), np.zeros(len(lengths), dtype=np.int64), lengths], 1)
     wl = xvec_b200.window_layout(lengths, w)
-    starts, n_pool, slot_start, rows, n_slots = L.utterance_layout(lengths)
-    assert wl.row0 == 0 and wl.rows == rows and wl.n_slots == n_slots
-    for a, b in ((wl.starts, starts), (wl.n_pool, n_pool), (wl.slot_start, slot_start), (wl.slot_lo, slot_start[:-1]),
-                 (wl.slot_hi, slot_start[1:]), (wl.win_n_pool, n_pool)):
-        assert a.dtype == b.dtype == np.int32 and np.array_equal(a, b)
+    ul = L.utterance_layout(lengths)
+    assert type(ul) is type(wl) and wl.row0 == 0
+    for f in dataclasses.fields(wl):
+        a, b = getattr(wl, f.name), getattr(ul, f.name)
+        if isinstance(a, np.ndarray):
+            assert a.dtype == b.dtype == np.int32 and np.array_equal(a, b), f.name
+        else:
+            assert type(a) is type(b) is int and a == b, f.name
+    assert np.array_equal(ul.slot_lo, ul.slot_start[:-1]) and np.array_equal(ul.slot_hi, ul.slot_start[1:])
     lay = xvec_b200.build_layout(lengths)
     row_utt, blk_slot_base = _expand(wl)
     assert np.array_equal(row_utt, lay.row_utt)
@@ -176,27 +186,3 @@ def test_window_validation_uses_the_models_lost_frames():
     assert xvec_b200.window_layout([100], [[0, 0, 15]]).win_n_pool.tolist() == [1]
     with pytest.raises(ValueError, match="more than 20"):
         xvec_b200.window_layout([100], [[0, 0, 20]], lost_frames=20)
-
-
-def test_extract_windows_rejects_bad_arguments_without_a_device():
-    """xvec_extract_windows checks its arguments before any CUDA call, like xvec_extract_forward; well-formed arguments get as far
-    as the first CUDA call and report the missing device there."""
-    lib = xvec_b200._lib.load()
-    tdnn = (xvec_b200._lib.LayerDesc * 2)()
-    for d in tdnn:
-        d.w_packed_dev, d.bias_dev, d.n, d.cin, d.taps, d.dtype = 256, 256, 256, 256, 1, xvec_b200._lib.F32
-    fc = (xvec_b200._lib.LayerDesc * 3)()
-    buf = 256  # stands for device pointers; nothing is dereferenced on these paths
-
-    def call(lo=buf, hi=buf, npool=buf, n_windows=4, fc_host=fc, n_fc=1, out=buf, shift=None):
-        return lib.xvec_extract_windows(tdnn, 2, buf, 300, 256, buf, buf, 256, buf, buf, lo, hi, npool, n_windows, buf, None, shift,
-                                        buf, None, fc_host, n_fc, buf, None, 0, out, 256, None, 0, None)
-
-    E = xvec_b200._lib.E_ARG
-    assert call(n_fc=3) == E
-    assert call(lo=None) == E and call(hi=None) == E and call(npool=None) == E
-    assert call(n_windows=0) == E and call(n_windows=-1) == E
-    assert call(out=None) == E
-    assert call(shift=buf) == E  # BN shift without scale
-    if lib.xvec_device_check() != 0:
-        assert call(fc_host=None, n_fc=0, out=None) == lib.xvec_device_check() != E

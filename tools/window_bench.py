@@ -9,7 +9,7 @@ the 126 MB of L2), device-resident.  For each window case (150/75, 300/150 and t
    extract_x_vec_flat in batches of <= 131 072 frames.  Two streams, two scratch slots, the two paths alternated over `reps`
    repetitions (rotating which goes first); device time per leg from CUDA events -> windows/s.
 2. Frame-level FLOPs of each path from shapes (bench.FLOPS_L / LOST per layer and output row) and their ratio.
-3. The ranges finalize (pool_finalize_kernel<true>) and the stack kernel alone: summed kernel time of one windowed leg per case
+3. The finalize (pool_finalize_kernel) and the stack kernel alone: summed kernel time of one windowed leg per case
    under torch.profiler (a separate, untimed run).
 4. Agreement of the two paths: max-abs difference over max |re-extraction|.
 5. The device name, power limit and max SM clock (nvidia-smi, read-only query) in the same run.
@@ -121,7 +121,7 @@ def main():
                     ms[k].append(timed(legs[k])[0])
             with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
                 timed(win_calls)
-            fin_us, fin_n = kernel_us(prof, "pool_finalize_kernel<true>")
+            fin_us, fin_n = kernel_us(prof, "pool_finalize_kernel")
             stack_us, stack_n = kernel_us(prof, "tdnn_stack_kernel")
             del xs, re_calls, legs
             torch.cuda.empty_cache()
